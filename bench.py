@@ -15,6 +15,10 @@ moment assembly and the closed-form estimator.
 
 `--impl reference` times the reference's own CPU implementation (oracle/_ref/kgl_ref_harness, the reference TUs
 compiled where they lie; else the oracle port) on a bounded sample of the same workload, on the host cores.
+
+`--dump-outputs DIR` writes, after the timed steps, the per-locus counts and per-genome results of the step as
+DIR/<name>.npy (see dump_outputs and run_ours). The inputs depend on the arguments only, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -57,12 +61,12 @@ SEED = 20261018
 METRIC = "inbreeding genotype-loci/s"
 UNIT = "genotype-loci/s"
 # Bounded samples of the reference CPU path (BASELINE.md section 4 / SURVEY 8d: 2,504 genomes x 50,000 loci; the reference
-# cannot materialise config 2 as a PopulationDB). --impl reference times the BASELINE sample (~25 s per repeat on 15 threads,
-# so at most REFERENCE_MAX_REPEATS repeats: the run stays within a few minutes); the cpu_baseline object of the GPU arm
-# uses a 20,000-locus prefix of the same population (~10 s per repeat).
+# cannot materialise config 2 as a PopulationDB). --impl reference times the BASELINE sample (~25 s per repeat on 15 threads);
+# the cpu_baseline object of the GPU arm uses a 20,000-locus prefix of the same population (~10 s per repeat).
 REFERENCE_SAMPLE = (2504, 50_000)
 CPU_SAMPLE = (2504, 20_000)
-REFERENCE_MAX_REPEATS = 6
+DUMP_BYTES = 64_000_000     # --dump-outputs: at most this much in all, .npy headers included
+DUMP_HEADER_BYTES = 4096    # what the headers of its (at most 14) files may take
 
 
 def parse_args():
@@ -84,7 +88,47 @@ def parse_args():
                     help="loci of the pairwise run (default: BASELINE config 4, 20 M SNPs; 0 = the resident chr22-shape matrix)")
     ap.add_argument("--kinship-steps", type=int, default=3)
     ap.add_argument("--reference-sample", default="", help="--impl reference: GENOMESxLOCI of the CPU sample (default 2504x50000, BASELINE.md section 4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the per-locus counts and per-genome results of the step as DIR/<name>.npy "
+                         "(one GPU: of one more run of the step; N > 1: of the last timed step, locus counts of rank 0's shard)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
+    return args
+
+
+def sample_rows(n_rows: int, row_bytes: int, room: int, seed: int):
+    """None if n_rows rows of row_bytes fit in room bytes; else the sorted row numbers of a fixed sample, drawn with `seed`,
+    that fits there together with the row numbers themselves (8 B per row)."""
+    if n_rows * row_bytes <= room:
+        return None
+    return np.sort(np.random.default_rng(seed).choice(n_rows, size=max(1, room // (row_bytes + 8)), replace=False))
+
+
+def dump_outputs(path, locus_counts, results):
+    """Writes what one step of the timed path hands its caller: the per-locus allele counts uint32 [L, 4] as locus_counts.npy
+    (float32, exact below 2^24 genomes) and every LocusResults field of every genome as genome_<field>.npy (float64), at most
+    DUMP_BYTES in all. The per-genome arrays get at most half of that, the per-locus counts the rest; an array that does not
+    fit its share holds a fixed sample of rows, drawn with the bench seed, and genome_rows.npy / locus_rows.npy their row
+    numbers."""
+    os.makedirs(path, exist_ok=True)
+    out = {}
+    room = DUMP_BYTES - DUMP_HEADER_BYTES
+    rows = sample_rows(results.shape[0], 8 * len(results.dtype.names), room // 2, SEED)
+    if rows is not None:
+        out["genome_rows"] = rows.astype(np.float64)
+        results = results[rows]
+    out.update({"genome_" + f: results[f].astype(np.float64) for f in results.dtype.names})
+    room -= sum(a.nbytes for a in out.values())
+    rows = sample_rows(locus_counts.shape[0], 16, room, SEED + 1)
+    if rows is not None:
+        out["locus_rows"] = rows.astype(np.float64)
+        locus_counts = locus_counts[rows]
+    out["locus_counts"] = locus_counts.astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def stream_kernel_name(n_genomes: int) -> str:
@@ -165,8 +209,8 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    repeats = max(1, min(args.steps + args.warmup, REFERENCE_MAX_REPEATS))
-    warm = min(args.warmup, repeats - 1, 1)               # at most one untimed repeat: the reference has no caches to warm
+    warm = min(args.warmup, 1)                            # at most one untimed repeat: the reference has no caches to warm
+    repeats = warm + args.steps
     sample = REFERENCE_SAMPLE
     if args.reference_sample:
         sample = tuple(int(x) for x in args.reference_sample.lower().split("x"))
@@ -180,7 +224,7 @@ def run_reference_arm(args):
         "dtype": "f64", "data": "synthetic",
         "config": {"workload": workload_name(args.genomes, args.loci, 1),
                    "note": "reference CPU path timed on a bounded sample of this workload (BASELINE.md section 4: 2,504 genomes x 50,000 loci); "
-                           "value is per-unit throughput; repeats capped so that the run ends within a few minutes"},
+                           "value is per-unit throughput"},
         "cpu_baseline": {"value": value, "unit": UNIT, "cores": r["cores"], "kind": r["kind"], "sample": r["sample"]},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
@@ -367,6 +411,15 @@ def run_ours(args):
     res = ctx.inbreed_fetch() if world > 1 else None
     lc = ctx.fetch_locus_counts()
     assert int(lc.sum()) == n * l and np.all(lc.sum(axis=1) == n), "per-locus counts do not add up to the genome count"
+    if args.dump_outputs:
+        if world == 1:
+            # The C ABI hands the per-genome results of a single-GPU pass to the host only through the one-call form of the
+            # same pass (kgl_b200_run_count_and_inbreed): what is written comes from one more run of the step, whose per-locus
+            # counts must equal those of the last timed step.
+            lc_again, res = ctx.count_and_inbreed()
+            assert np.array_equal(lc_again, lc), "a repeated pass gives other per-locus counts"
+        if rank == 0:
+            dump_outputs(args.dump_outputs, lc, res)
 
     # ---- end to end through the C ABI with host buffers ----
     e2e = None

@@ -790,6 +790,46 @@ def test_peer_exchange_two_gpus():
         pytest.skip("CUDA IPC peer mapping unavailable on this box: " + line["config"]["exchange"])
 
 
+def test_bench_dump_outputs_two_gpus(tmp_path):
+    """bench.py --dump-outputs with two locus-sharded ranks: rank 0's per-locus counts and the exchanged per-genome Simple results
+    of the last timed step, against the oracle on rank 0's shard and on both shards together. Needs two GPUs."""
+    import json
+    import subprocess
+    import sys
+    import torch
+    from bench import SEED
+    from kgl_gene_b200.flatfile import FlatPopulation
+    from kgl_gene_b200.synth import make_genomes, make_loci
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two GPUs")
+    n, l = 300, 50_000
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2", "--master-addr", "127.0.0.1",
+           "--master-port", "29537", os.path.join(root, "bench.py"), "--gpus", "2", "--steps", "3", "--warmup", "1",
+           "--genomes", str(n), "--loci", str(l), "--no-kinship", "--no-estimators", "--no-e2e", "--no-cpu-baseline",
+           "--dump-outputs", str(tmp_path)]
+    proc = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=root)
+    assert proc.returncode == 0, proc.stderr[-2000:]
+    assert json.loads(proc.stdout.strip().splitlines()[-1])["n_gpus"] == 2
+    superpop, inbreeding = make_genomes(n, SEED)
+    shards = []
+    for rank in range(2):           # bench.py's shard of each rank
+        offsets, af = make_loci(l, SEED + 1000 * rank)
+        shards.append((offsets, af, O.synth_genotypes(SEED, n, l, af, superpop, inbreeding, locus_base=rank * l)))
+    rank0 = FlatPopulation(shards[0][0], shards[0][1], superpop, shards[0][2], n, False)
+    assert np.array_equal(np.load(tmp_path / "locus_counts.npy"), O.allele_count(rank0)[0])
+    offsets = np.concatenate([shards[0][0], shards[1][0] + shards[0][0][-1] + 10])       # the two shards as one locus table
+    both = FlatPopulation(offsets, np.concatenate([shards[0][1], shards[1][1]], axis=1), superpop,
+                          np.concatenate([shards[0][2], shards[1][2]]), n, False)
+    want = O.inbreed(both, O.select_all_pops(both), "Simple")
+    for f in want.dtype.names:
+        got = np.load(tmp_path / f"genome_{f}.npy")
+        if f.endswith("_count"):
+            assert np.array_equal(got, want[f]), f
+        else:
+            assert np.max(np.abs(got - want[f]) / np.maximum(np.abs(want[f]), 1e-3)) < 1e-6, f
+
+
 @pytest.mark.parametrize("multi", [False, True], ids=["biallelic", "multi-allelic"])
 def test_count_limited_selection_and_locus_filter(gpu, multi):
     """N3: RetrieveLociiVector::getLociiCount on the device (kgl_b200_count_loci: how the window loop of populationInbreeding finds
