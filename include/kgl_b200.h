@@ -194,6 +194,31 @@ int kgl_b200_set_ibs_tensor_cores(kgl_b200_ctx* ctx, int enable);
 int kgl_b200_ibs_used_tensor_cores(const kgl_b200_ctx* ctx);     /* the last IBS call: 1 tensor cores, 0 popcount kernel */
 int kgl_b200_run_ibs_tiles(kgl_b200_ctx* ctx, uint64_t first, uint64_t stride, uint64_t count, uint32_t* out);
 
+/* KING-robust kinship (Manichaikul et al., Bioinformatics 2010; the between-family estimator of PLINK 2's --make-king), for
+ * structured populations: it needs no allele frequencies. For genomes a, b over the loci where neither is coded 3 (multi-allelic
+ * rows count as missing for their non-reference cells, as in kgl_b200_run_ibs):
+ *     kinship = 0.5 - (4 IBS0 + IBS1) / (4 min(het_a, het_b))        NaN when min(het_a, het_b) == 0
+ * het_a / het_b = heterozygous loci of a / of b among the loci valid in both; het_het = loci where both are heterozygous
+ * (het_a + het_b = IBS1 + 2 het_het). Counts are exact integers and the kinship is one IEEE division and one subtraction in
+ * double. IBS0 / IBS1 come from the IBS path (tensor cores or popcount kernel, kgl_b200_set_ibs_tensor_cores), het_het and the
+ * per-pair het counts from int8 Gram runs on the tensor cores (king.cuh). n_loci < 2^29. Both entry points need a genotype upload
+ * (KGL_B200_ERR_STATE before it). */
+typedef struct kgl_b200_king_pair {          /* 40 bytes */
+  uint32_t a, b;                             /* genome indices, a < b */
+  uint32_t n_valid, ibs0, ibs1, het_het, het_a, het_b;
+  double kinship;
+} kgl_b200_king_pair;
+/* kinship double[row_end-row_begin][n_genomes]: genomes [row_begin,row_end) against all genomes (the band / whole-matrix logic of
+ * kgl_b200_run_ibs). The diagonal is 0.5 for a genome with a heterozygous locus. */
+int kgl_b200_run_king(kgl_b200_ctx* ctx, uint64_t row_begin, uint64_t row_end, double* kinship);
+/* Every pair a < b with kinship >= min_kinship (NaN never qualifies) inside the given 64 x 64 tiles (coords uint32[n_coords][2] =
+ * (tile row, tile column) with tile row <= tile column, e.g. a rank's shards.block_tile_coords; NULL or n_coords == 0 = the whole
+ * upper triangle), in ascending (a, b) order. *n_pairs = the true total; if it exceeds capacity nothing is copied and the call
+ * returns KGL_B200_ERR_NOMEM: retry with capacity = *n_pairs (the retry computes every tile again). A tile outside the grid or below the diagonal: KGL_B200_ERR_INVALID.
+ * 0.0442 (~2^-4.5) keeps third-degree relatives and closer. */
+int kgl_b200_run_king_pairs(kgl_b200_ctx* ctx, uint64_t n_coords, const uint32_t* coords, double min_kinship, uint64_t capacity,
+                            kgl_b200_king_pair* pairs, uint64_t* n_pairs);
+
 /* CalcFWS::updateGenomeFWSMap (kga_PfEMP/kga_analysis_PfEMP_FWS.cpp:15-101): for each of n_bins allele-frequency bins
  * [lower[b], upper[b]) of AF column `pop` (the P7FrequencyFilter pair AF >= lower and not AF >= upper,
  * kgl_variant_filter_Pf7.cpp:20-66; a locus without AF is in no bin) the AlleleSummmary of every genome over the bin's loci:

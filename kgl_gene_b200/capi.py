@@ -22,12 +22,22 @@ RESULT_DTYPE = np.dtype([  # kgl_b200_locus_results == kga::LocusResults field o
     ("total_allele_count", "<u8"), ("inbred_allele_sum", "<f8"),
 ])
 
+class KingPair(C.Structure):
+    """kgl_b200_king_pair (include/kgl_b200.h), 40 bytes."""
+    _fields_ = [("a", C.c_uint32), ("b", C.c_uint32), ("n_valid", C.c_uint32), ("ibs0", C.c_uint32), ("ibs1", C.c_uint32),
+                ("het_het", C.c_uint32), ("het_a", C.c_uint32), ("het_b", C.c_uint32), ("kinship", C.c_double)]
+
+
+KING_PAIR_DTYPE = np.dtype([(name, "<f8" if ctype is C.c_double else "<u4") for name, ctype in KingPair._fields_])
+
+KGL_B200_ERR_NOMEM = 5
+
 EXPORTS = [
     "kgl_b200_version", "kgl_b200_device_count", "kgl_b200_create", "kgl_b200_destroy", "kgl_b200_last_error",
     "kgl_b200_set_stream", "kgl_b200_synchronize", "kgl_b200_upload_genotypes", "kgl_b200_upload_loci",
     "kgl_b200_set_genome_superpop", "kgl_b200_upload_multi_allelic", "kgl_b200_run_multi_allele_count", "kgl_b200_set_unphased", "kgl_b200_select_loci", "kgl_b200_set_locus_selection",
     "kgl_b200_get_locus_selection", "kgl_b200_count_loci", "kgl_b200_set_locus_filter", "kgl_b200_synth_genotypes", "kgl_b200_download_genotypes", "kgl_b200_run_allele_count",
-    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
+    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
     "kgl_b200_run_binned_genome_counts", "kgl_b200_run_hetero_homo", "kgl_b200_location_fis", "kgl_b200_run_gram", "kgl_b200_run_grm", "kgl_b200_enqueue_gram", "kgl_b200_last_gram_kernel_ms", "kgl_b200_enqueue_gram_tiles", "kgl_b200_gram_buffer", "kgl_b200_fetch_gram",
     "kgl_b200_enqueue_ibs_tiles", "kgl_b200_ibs_tiles_buffer", "kgl_b200_ibs_timer_reset", "kgl_b200_ibs_timer_read",
     "kgl_b200_enqueue_count_and_inbreed", "kgl_b200_flush", "kgl_b200_launch_count", "kgl_b200_last_stream_kernel_ms",
@@ -279,6 +289,35 @@ class KglB200:
         out = np.zeros((row_end - row_begin, self.n_genomes, 4), dtype=np.uint32)
         self._check(self.lib.kgl_b200_run_ibs(self.h, C.c_uint64(row_begin), C.c_uint64(row_end), _ptr(out)), "run_ibs")
         return out
+
+    def king(self, row_begin=0, row_end=None) -> np.ndarray:
+        """KING-robust kinship float64[row_end - row_begin][N] of genomes [row_begin, row_end) against all genomes."""
+        row_end = self.n_genomes if row_end is None else row_end
+        out = np.zeros((row_end - row_begin, self.n_genomes), dtype=np.float64)
+        self._check(self.lib.kgl_b200_run_king(self.h, C.c_uint64(row_begin), C.c_uint64(row_end), _ptr(out)), "run_king")
+        return out
+
+    def king_pairs(self, min_kinship: float, coords=None, capacity: int = 1 << 22) -> np.ndarray:
+        """Pairs a < b with KING kinship >= min_kinship inside the 64 x 64 tiles `coords` (uint32[n][2], tile row <= tile column;
+        None = the whole upper triangle), sorted by (a, b): a KING_PAIR_DTYPE array. Retries once with the exact capacity; a retry
+        computes every tile again, so the default (4 M pairs, 168 MB of host buffer that is only touched as far as it is filled,
+        52 B per pair on the device, never more than the tiles hold) is sized for related-pair lists of biobank populations."""
+        if coords is not None:
+            coords = np.ascontiguousarray(coords, dtype=np.uint32).reshape(-1, 2)
+            if coords.shape[0] == 0:
+                return np.zeros(0, dtype=KING_PAIR_DTYPE)
+        n_coords = 0 if coords is None else coords.shape[0]
+        n = C.c_uint64(0)
+        for attempt in range(2):
+            out = np.zeros(max(int(capacity), 1), dtype=KING_PAIR_DTYPE)
+            rc = self.lib.kgl_b200_run_king_pairs(self.h, C.c_uint64(n_coords), _ptr(coords), C.c_double(min_kinship),
+                                                  C.c_uint64(capacity), _ptr(out), C.byref(n))
+            if rc == KGL_B200_ERR_NOMEM and attempt == 0:
+                capacity = int(n.value)
+                continue
+            self._check(rc, "run_king_pairs")
+            break
+        return out[: n.value].copy()
 
     def binned_genome_counts(self, lower, upper, pop: int = 0, present_only: bool = True):
         """(counts uint64[n_bins][N][4], rows uint64[n_bins]) -- CalcFWS' per-genome AlleleSummmary per AF bin."""

@@ -239,7 +239,9 @@ k_gram_i8(const GramParams P) {
 }
 
 // Genome-major 2-bit codes from the sample-major planes: codes[g][w16] holds loci 16 w16 .. 16 w16 + 15 of genome g,
-// code 3 -> 0. One thread per (genome, 32-locus word) -> two output words.
+// code 3 -> 0 (KEEP3: code 3 stays 3, for the code-3 indicator of the KING Gram run, king.cuh). One thread per
+// (genome, 32-locus word) -> two output words.
+template <bool KEEP3 = false>
 __global__ void __launch_bounds__(256)
 k_codes16(const uint32_t* __restrict__ sm_lo, const uint32_t* __restrict__ sm_hi, uint64_t n_gblocks, uint64_t n_words,
           uint64_t k_stages, uint64_t n_rows, uint32_t* __restrict__ codes /* zeroed */) {
@@ -247,8 +249,10 @@ k_codes16(const uint32_t* __restrict__ sm_lo, const uint32_t* __restrict__ sm_hi
   if (idx >= n_gblocks * n_words * 32) return;
   const uint64_t lane = idx & 31, w = (idx >> 5) % n_words, gb = (idx >> 5) / n_words;
   uint32_t lo = sm_lo[idx], hi = sm_hi[idx];
-  const uint32_t both = lo & hi;
-  lo &= ~both; hi &= ~both;
+  if (!KEEP3) {
+    const uint32_t both = lo & hi;
+    lo &= ~both; hi &= ~both;
+  }
   uint32_t out[2];
 #pragma unroll
   for (int h = 0; h < 2; ++h) {

@@ -15,6 +15,7 @@
 #include "multi_allelic.cuh"
 #include "gram_launch.cuh"
 #include "ibs_gram.cuh"
+#include "king.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -237,6 +238,15 @@ struct kgl_b200_ctx {
   uint64_t gram_ld = 0, gram_tiles_ld = 0, gram_n_tiles = 0, gram_first = 0, gram_stride = 1;
   bool codes16_valid = false;
   cudaEvent_t gram_e0 = nullptr, gram_e1 = nullptr;
+  // KING-robust kinship (king.cuh): raw code matrix (code 3 kept), M = H C^T blocks, dense slab, pair list and its sort
+  DevBuf<uint32_t> d_codes_raw;
+  bool codes_raw_valid = false;
+  DevBuf<int32_t> d_king_m;
+  DevBuf<double> d_king_out;
+  DevBuf<kgl_b200_king_pair> d_king_pairs, d_king_sorted;
+  DevBuf<unsigned long long> d_king_keys, d_king_keys2, d_king_cursor;
+  DevBuf<uint32_t> d_king_index, d_king_index2;
+  DevBuf<uint8_t> d_king_sort_temp;
 
   // iterative estimator state
   int algo = -1, phase = 0, iteration = 0;
@@ -1108,9 +1118,26 @@ int ensure_codes16(kgl_b200_ctx* c);
 
 constexpr uint64_t kIbsMaxTilesPerLaunch = 8192;     // 384 MB of accumulators
 
+// The genomes' heterozygous / hom-alt cells on the IBS planes (code 3 in neither), once per upload.
+int ensure_ibs_class(kgl_b200_ctx* c) {
+  if (c->ibs_class_valid) return KGL_B200_OK;
+  const uint64_t ld = (c->N + kGramN - 1) / kGramN * kGramN;
+  const size_t n_rows = (size_t)std::max<uint64_t>(c->n_gblocks * 32, ld);
+  KGL_CUDA(c, c->d_ibs_class.ensure(n_rows * 2));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_class.p, 0, n_rows * 2 * 4, c->stream));
+  const uint32_t wpc = 4096;
+  k_ibs_class_counts<<<dim3((unsigned)c->n_gblocks, (unsigned)((c->n_words + wpc - 1) / wpc)), 256, 0, c->stream>>>(
+      c->ibs_mode == 2 ? c->d_ibs_lo.p : c->d_sm_lo.p, c->ibs_mode == 2 ? c->d_ibs_hi.p : c->d_sm_hi.p, c->n_words, wpc, c->d_ibs_class.p);
+  KGL_LAUNCH_CHECK(c);
+  c->ibs_class_valid = true;
+  return KGL_B200_OK;
+}
+
 // Dense kernel (+ sparse repair) over a host tile list; leaves acc[n][3][4096] in d_ibs_acc. n <= kIbsMaxTilesPerLaunch.
 // `key` identifies the list: a repeated request (the benchmark loop, HallME-style reruns) skips the upload and its sync.
-int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const uint64_t (&key)[4], uint32_t n_cached = 0) {
+// want_blocks: build the 256 x 256 block list under the tiles also when the popcount kernel runs (KING's Gram runs use it).
+int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const uint64_t (&key)[4], uint32_t n_cached = 0,
+                      bool want_blocks = false) {
   const uint32_t n = tiles.empty() ? n_cached : (uint32_t)tiles.size();
   KGL_CUDA(c, c->d_ibs_tiles.ensure(n));
   KGL_CUDA(c, c->d_ibs_acc.ensure((size_t)n * 3 * kIbsTileCells));
@@ -1118,26 +1145,19 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const ui
   static const bool tensor_off = std::getenv("KGL_B200_IBS_POPCOUNT") != nullptr;
   c->gram_ld = (c->N + kGramN - 1) / kGramN * kGramN;
   const bool tensor = !tensor_off && c->ibs_tensor_enabled && c->ibs_mode != 1 && c->L < (1ull << 29);
+  const bool need_blocks = tensor || want_blocks;
   if (tensor) {
     int rc = ensure_codes16(c); if (rc) return rc;
-    if (!c->ibs_class_valid) {          // the genomes' heterozygous / hom-alt cells, once per upload
-      const size_t n_rows = (size_t)std::max<uint64_t>(c->n_gblocks * 32, c->gram_ld);
-      KGL_CUDA(c, c->d_ibs_class.ensure(n_rows * 2));
-      KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_class.p, 0, n_rows * 2 * 4, c->stream));
-      const uint32_t wpc = 4096;
-      k_ibs_class_counts<<<dim3((unsigned)c->n_gblocks, (unsigned)((c->n_words + wpc - 1) / wpc)), 256, 0, c->stream>>>(
-          c->ibs_mode == 2 ? c->d_ibs_lo.p : c->d_sm_lo.p, c->ibs_mode == 2 ? c->d_ibs_hi.p : c->d_sm_hi.p, c->n_words, wpc, c->d_ibs_class.p);
-      KGL_LAUNCH_CHECK(c);
-      c->ibs_class_valid = true;
-    }
+    rc = ensure_ibs_class(c); if (rc) return rc;
   }
-  if (std::memcmp(key, c->ibs_tiles_key, sizeof key) != 0 || (tensor && c->ibs_n_blocks == 0)) {
+  if (std::memcmp(key, c->ibs_tiles_key, sizeof key) != 0 || (need_blocks && c->ibs_n_blocks == 0)) {
     std::vector<uint2> list = tiles;
     if (list.empty()) return fail(c, KGL_B200_ERR_STATE, "tile list not available");
     KGL_CUDA(c, cudaMemcpyAsync(c->d_ibs_tiles.p, list.data(), (size_t)n * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
     std::vector<uint2> blocks;
     std::vector<uint32_t> tile_block;
-    if (tensor) {
+    c->ibs_n_blocks = 0;                 // a list uploaded without its blocks must not inherit the block count of the one before
+    if (need_blocks) {
       // the 256 x 256 Gram blocks under the tiles (upper triangle of the block grid; a tile below the diagonal uses the mirror block)
       std::unordered_map<uint64_t, uint32_t> index;
       tile_block.resize(list.size());
@@ -1246,11 +1266,71 @@ int ensure_codes16(kgl_b200_ctx* c) {
   const size_t words = (size_t)c->gram_ld * k_stages * 8;
   KGL_CUDA(c, c->d_codes16.ensure(words));
   KGL_CUDA(c, cudaMemsetAsync(c->d_codes16.p, 0, words * 4, c->stream));
-  k_codes16<<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks, c->n_words,
-                                                                                              k_stages, c->gram_ld, c->d_codes16.p);
+  k_codes16<false><<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks, c->n_words,
+                                                                                                     k_stages, c->gram_ld, c->d_codes16.p);
   KGL_LAUNCH_CHECK(c);
   c->codes16_valid = true;
   return KGL_B200_OK;
+}
+
+// The same layout with code 3 kept (k_codes16<true>): the code-3 indicator operand of KING's M = H C^T. Once per upload, and only
+// for populations that have code-3 cells.
+int ensure_codes_raw(kgl_b200_ctx* c) {
+  int rc = ensure_sample_major(c); if (rc) return rc;
+  if (c->codes_raw_valid) return KGL_B200_OK;
+  const uint64_t ld = (c->N + kGramN - 1) / kGramN * kGramN;
+  const uint64_t k_stages = (c->L + kGramK - 1) / kGramK;
+  const size_t words = (size_t)ld * k_stages * 8;
+  KGL_CUDA(c, c->d_codes_raw.ensure(words));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_codes_raw.p, 0, words * 4, c->stream));
+  k_codes16<true><<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks, c->n_words,
+                                                                                                    k_stages, ld, c->d_codes_raw.p);
+  KGL_LAUNCH_CHECK(c);
+  c->codes_raw_valid = true;
+  return KGL_B200_OK;
+}
+
+// ---- KING-robust kinship (king.cuh) -------------------------------------------------------------------------------------
+// One slab of tiles (<= kIbsMaxTilesPerLaunch): the IBS counts by ibs_compute_tiles in whichever form it picks, HH (already
+// filled by the tensor form, otherwise one Gram run) and, with code-3 cells, M = H C^T over the same blocks. Fills K.
+int king_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const uint64_t (&key)[4], KingTiles& K) {
+  int rc = ibs_compute_tiles(c, tiles, key, 0, true); if (rc) return rc;
+  rc = ensure_ibs_class(c); if (rc) return rc;
+  const uint32_t n = (uint32_t)tiles.size();
+  const size_t block_cells = (size_t)c->ibs_n_blocks * kGramM * kGramN;
+  const uint32_t k_stages = (uint32_t)((c->L + kGramK - 1) / kGramK);
+  const GramPlan gp = plan_gram(std::max<uint32_t>(c->ibs_n_blocks, 1), k_stages, c->sm_count);
+  GramParams G{};
+  G.k_stages = k_stages; G.tiles = c->d_ibs_blocks.p; G.n_tiles = c->ibs_n_blocks;
+  G.stages_per_chunk = gp.stages_per_chunk; G.n_chunks = gp.n_chunks; G.ld = c->gram_ld; G.compact = 1;
+  if (!c->ibs_used_tensor) {                       // the popcount kernel ran: HH is not there yet
+    rc = ensure_codes16(c); if (rc) return rc;
+    KGL_CUDA(c, c->d_gram_hh.ensure(block_cells));
+    G.codes = c->d_codes16.p; G.out = c->d_gram_hh.p; G.table_a = G.table_b = kGramTableHet;
+    if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(G.out, 0, block_cells * 4, c->stream));
+    KGL_CUDA(c, launch_gram(G, gp, c->stream));
+    ++c->launches;
+  }
+  if (c->n_dropped > 0) {
+    rc = ensure_codes_raw(c); if (rc) return rc;
+    KGL_CUDA(c, c->d_king_m.ensure(block_cells));
+    G.codes = c->d_codes_raw.p; G.out = c->d_king_m.p; G.table_a = kGramTableHet; G.table_b = kGramTableCode3;
+    if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(G.out, 0, block_cells * 4, c->stream));
+    KGL_CUDA(c, launch_gram(G, gp, c->stream));
+    ++c->launches;
+  }
+  K = KingTiles{};
+  K.acc = c->d_ibs_acc.p; K.tiles = c->d_ibs_tiles.p; K.n_tiles = n;
+  K.valid_mode = c->ibs_mode; K.seg = c->ibs_mode == 2 ? c->d_dropped_seg.p : nullptr; K.n_loci = (uint32_t)c->L; K.n_genomes = c->N;
+  K.hh = c->d_gram_hh.p; K.m = c->n_dropped > 0 ? c->d_king_m.p : nullptr; K.tile_block = c->d_ibs_tile_block.p; K.counts = c->d_ibs_class.p;
+  return KGL_B200_OK;
+}
+
+int king_check(kgl_b200_ctx* c) {
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  if (c->L >= (1ull << 29)) return fail(c, KGL_B200_ERR_INVALID, "KING: more than 2^29 loci would overflow the int32 Gram accumulators");
+  return ensure_ibs_planes(c);
 }
 
 // Tiles first, first + stride, ... of the upper-triangle tile list (rank r of R: first = r, stride = R); the rest of the
@@ -1357,6 +1437,8 @@ void kgl_b200_destroy(kgl_b200_ctx* c) {
   c->d_terms_table.release(); c->d_list_count.release();
   c->d_chain_u32.release(); c->d_chain_mark.release();
   c->d_list.release(); c->d_sm_codes.release(); c->d_limits.release(); c->d_slow_out.release(); c->d_lane_state.release(); c->d_n_slow.release();
+  c->d_codes_raw.release(); c->d_king_m.release(); c->d_king_out.release(); c->d_king_pairs.release(); c->d_king_sorted.release();
+  c->d_king_keys.release(); c->d_king_keys2.release(); c->d_king_cursor.release(); c->d_king_index.release(); c->d_king_index2.release(); c->d_king_sort_temp.release();
   c->d_codes16.release(); c->d_gram.release(); c->d_gram_tiles.release(); c->d_gp_chunks.release(); c->d_gp.release(); c->d_gram_out.release();
   if (c->gram_e0) cudaEventDestroy(c->gram_e0);
   if (c->gram_e1) cudaEventDestroy(c->gram_e1);
@@ -1433,7 +1515,7 @@ static int set_shape(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_loci, uint6
   c->n_multi = 0;                    // the side cells belong to the matrix: kgl_b200_upload_multi_allelic comes after it
   c->units = stream_units_padded(c->host_units); c->Npad = c->units * 64;
   c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key[0] = ~0ull; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
-  c->codes16_valid = false;
+  c->codes16_valid = false; c->codes_raw_valid = false;
   return KGL_B200_OK;
 }
 
@@ -2320,6 +2402,110 @@ int kgl_b200_run_ibs(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, uint
     KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)(r0 - row_begin) * c->N * 4, c->d_ibs.p, (size_t)(r1 - r0) * c->N * 16, cudaMemcpyDeviceToHost, c->stream));
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   }
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_king(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, double* kinship) {
+  if (!c || !kinship) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  int rc = king_check(c); if (rc) return rc;
+  if (row_begin >= row_end || row_end > c->N) return fail(c, KGL_B200_ERR_INVALID, "bad genome row range");
+  const uint64_t side = ibs_side(c);
+  KingTiles K{};
+  const bool whole = row_begin == 0 && row_end == c->N && c->N * c->N * 8 <= (2ull << 30);
+  if (whole) {
+    // the whole matrix: upper-triangle tiles, every tile also written transposed (the tile lists of kgl_b200_run_ibs)
+    KGL_CUDA(c, c->d_king_out.ensure((size_t)c->N * c->N));
+    std::vector<uint2> tiles;
+    for (uint64_t t0 = 0, n_upper = side * (side + 1) / 2; t0 < n_upper; t0 += kIbsMaxTilesPerLaunch) {
+      tiles.clear();
+      for (uint64_t t = t0; t < std::min(n_upper, t0 + kIbsMaxTilesPerLaunch); ++t) tiles.push_back(ibs_upper_tile(t, side));
+      const uint64_t key[4] = {1, t0, 1, tiles.size()};
+      rc = king_compute_tiles(c, tiles, key, K); if (rc) return rc;
+      k_king_dense<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, 0, c->N, 1, c->d_king_out.p);
+      KGL_LAUNCH_CHECK(c);
+    }
+    KGL_CUDA(c, cudaMemcpyAsync(kinship, c->d_king_out.p, (size_t)c->N * c->N * 8, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KGL_B200_OK;
+  }
+  // a band of rows: every tile of the band's tile rows, in slabs that keep the device result under ~1 GiB
+  const uint64_t slab_tile_rows = std::max<uint64_t>(1, std::min<uint64_t>((1ull << 30) / (c->N * 8 * kIbsT), kIbsMaxTilesPerLaunch / side));
+  std::vector<uint2> tiles;
+  for (uint64_t tr0 = row_begin / kIbsT; tr0 * kIbsT < row_end; tr0 += slab_tile_rows) {
+    const uint64_t tr1 = std::min((row_end + kIbsT - 1) / kIbsT, tr0 + slab_tile_rows);
+    const uint64_t r0 = std::max(row_begin, tr0 * kIbsT), r1 = std::min(row_end, tr1 * kIbsT);
+    tiles.clear();
+    for (uint64_t ta = tr0; ta < tr1; ++ta)
+      for (uint64_t tb = 0; tb < side; ++tb) tiles.push_back(make_uint2((uint32_t)ta, (uint32_t)tb));
+    KGL_CUDA(c, c->d_king_out.ensure((size_t)(r1 - r0) * c->N));
+    const uint64_t key[4] = {2, tr0, tr1, tiles.size()};
+    rc = king_compute_tiles(c, tiles, key, K); if (rc) return rc;
+    k_king_dense<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, r0, r1, 0, c->d_king_out.p);
+    KGL_LAUNCH_CHECK(c);
+    KGL_CUDA(c, cudaMemcpyAsync(kinship + (size_t)(r0 - row_begin) * c->N, c->d_king_out.p, (size_t)(r1 - r0) * c->N * 8, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  }
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* coords, double min_kinship, uint64_t capacity,
+                            kgl_b200_king_pair* pairs, uint64_t* n_pairs) {
+  if (!c || !pairs || !n_pairs) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  int rc = king_check(c); if (rc) return rc;
+  const uint64_t side = ibs_side(c), n_upper = side * (side + 1) / 2;
+  const bool all = coords == nullptr || n_coords == 0;
+  const uint64_t n_tiles = all ? n_upper : n_coords;
+  for (uint64_t i = 0; !all && i < n_coords; ++i) {
+    if (coords[2 * i] >= side || coords[2 * i + 1] >= side) return fail(c, KGL_B200_ERR_INVALID, "tile coordinate outside the grid");
+    if (coords[2 * i] > coords[2 * i + 1]) return fail(c, KGL_B200_ERR_INVALID, "tile below the diagonal (need tile row <= tile column)");
+  }
+  // device list: no more records than the tiles hold, and indices that fit the uint32 sort values
+  const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, n_tiles * kIbsTileCells), 0xFFFFFFFFull);
+  KGL_CUDA(c, c->d_king_pairs.ensure(dev_cap));
+  KGL_CUDA(c, c->d_king_keys.ensure(dev_cap));
+  KGL_CUDA(c, c->d_king_index.ensure(dev_cap));
+  KGL_CUDA(c, c->d_king_cursor.ensure(1));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_king_cursor.p, 0, 8, c->stream));
+  KingTiles K{};
+  std::vector<uint2> tiles;
+  for (uint64_t t0 = 0; t0 < n_tiles; t0 += kIbsMaxTilesPerLaunch) {
+    const uint64_t t1 = std::min(n_tiles, t0 + kIbsMaxTilesPerLaunch);
+    tiles.clear();
+    uint64_t hash = 1469598103934665603ull;                      // FNV-1a of the list, as kgl_b200_enqueue_ibs_tile_list
+    for (uint64_t t = t0; t < t1; ++t) {
+      const uint2 tc = all ? ibs_upper_tile(t, side) : make_uint2(coords[2 * t], coords[2 * t + 1]);
+      tiles.push_back(tc);
+      hash = (hash ^ tc.x) * 1099511628211ull; hash = (hash ^ tc.y) * 1099511628211ull;
+    }
+    const uint64_t key_all[4] = {1, t0, 1, tiles.size()}, key_list[4] = {3, hash, tiles.size(), side};
+    rc = king_compute_tiles(c, tiles, all ? key_all : key_list, K); if (rc) return rc;
+    k_king_pairs<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, min_kinship, dev_cap, c->d_king_pairs.p,
+                                                                                               c->d_king_keys.p, c->d_king_index.p, c->d_king_cursor.p);
+    KGL_LAUNCH_CHECK(c);
+  }
+  unsigned long long total = 0;
+  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_king_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  *n_pairs = total;
+  if (total > capacity || total > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, "more related pairs than capacity (*n_pairs holds the total)");
+  if (total == 0) return KGL_B200_OK;
+  // ascending (a, b) whatever the order in which the warps appended
+  const uint64_t n = total;
+  int end_bit = 32;                                                // b in the low word, a < N above it
+  for (uint64_t v = c->N - 1; v; v >>= 1) ++end_bit;
+  KGL_CUDA(c, c->d_king_keys2.ensure(n));
+  KGL_CUDA(c, c->d_king_index2.ensure(n));
+  KGL_CUDA(c, c->d_king_sorted.ensure(n));
+  size_t temp_bytes = 0;
+  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, c->d_king_keys.p, c->d_king_keys2.p, c->d_king_index.p, c->d_king_index2.p,
+                                              n, 0, end_bit, c->stream));
+  KGL_CUDA(c, c->d_king_sort_temp.ensure(temp_bytes));
+  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(c->d_king_sort_temp.p, temp_bytes, c->d_king_keys.p, c->d_king_keys2.p, c->d_king_index.p,
+                                              c->d_king_index2.p, n, 0, end_bit, c->stream));
+  k_king_gather<<<blocks_for(n, 256), 256, 0, c->stream>>>(c->d_king_pairs.p, c->d_king_index2.p, n, c->d_king_sorted.p);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, cudaMemcpyAsync(pairs, c->d_king_sorted.p, n * sizeof(kgl_b200_king_pair), cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   return KGL_B200_OK;
 }
 

@@ -6,6 +6,8 @@
 * pairwise IBS: the 64 x 64 sample-pair tiles of the upper triangle are dealt round-robin to the ranks (tile t belongs to
   rank t mod world); every rank holds the whole packed matrix; no collective in the data path. `gather_ibs` collects the
   compact tile blocks and `assemble_ibs` lays them out as the symmetric genome x genome matrix.
+* KING related-pair lists: the same tiles (block_tile_coords) go to kgl_b200_run_king_pairs on each rank; `gather_king_pairs`
+  joins the ranks' lists.
 
 Everything here works on CPU tensors with the gloo backend as well (tests/test_shards_gloo.py) -- the CUDA context is only
 touched through the KglB200 object the caller passes in.
@@ -185,3 +187,28 @@ def gather_ibs(n_genomes: int, my_blocks: np.ndarray, group=None) -> np.ndarray 
         return None
     blocks = [o.cpu().numpy().view(np.uint32)[: tiles_of_rank(n_up, r, world)] for r, o in enumerate(out)]
     return assemble_ibs(n_genomes, blocks)
+
+
+# ------------------------------------------------------------------------------------------------ KING pairs ---------
+def gather_king_pairs(my_pairs: np.ndarray, group=None) -> np.ndarray:
+    """Every rank's KING pair list (capi.KING_PAIR_DTYPE records, any length) joined and sorted by (a, b), returned on every
+    rank (torch.distributed all_gather of the lengths, then of the zero-padded records). Works with gloo (CPU tensors) and NCCL."""
+    import torch
+    import torch.distributed as dist
+    world = dist.get_world_size(group)
+    dev = "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+    recs = np.ascontiguousarray(my_pairs)
+    rec_bytes = recs.dtype.itemsize
+    n = torch.tensor([recs.shape[0]], dtype=torch.int64, device=dev)
+    counts = [torch.zeros_like(n) for _ in range(world)]
+    dist.all_gather(counts, n, group=group)
+    counts = [int(c.item()) for c in counts]
+    cap = max(max(counts), 1)
+    buf = torch.zeros(cap * rec_bytes, dtype=torch.uint8)
+    buf[: recs.nbytes] = torch.from_numpy(recs.view(np.uint8).reshape(-1))
+    buf = buf.to(dev)
+    out = [torch.empty_like(buf) for _ in range(world)]
+    dist.all_gather(out, buf, group=group)
+    parts = [o.cpu().numpy()[: c * rec_bytes].view(recs.dtype) for o, c in zip(out, counts)]
+    joined = np.concatenate(parts)
+    return joined[np.lexsort((joined["b"], joined["a"]))]
