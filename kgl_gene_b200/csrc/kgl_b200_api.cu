@@ -46,6 +46,10 @@ template <class T>
 struct DevBuf {
   T* p = nullptr;
   size_t cap = 0;   // elements
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { if (p) cudaFree(p); }
   cudaError_t ensure(size_t n) {
     if (n <= cap) return cudaSuccess;
     if (p) cudaFree(p);
@@ -57,7 +61,58 @@ struct DevBuf {
   // For buffers whose size follows the selection window (the moment tables): a quarter of head room, so that a run of windows of
   // similar sizes reallocates once, not every time a window is a little larger than all before it.
   cudaError_t ensure_roomy(size_t n) { return n <= cap ? cudaSuccess : ensure(n + n / 4); }
-  void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// Event pairs around the launches of one kind since the last reset (kgl_b200_kernel_timer_read, kgl_b200_ibs_timer_read).
+struct TimerRing {
+  static constexpr int kSlots = 256;
+  std::vector<cudaEvent_t> ev;
+  int used = 0;
+  TimerRing() = default;
+  TimerRing(const TimerRing&) = delete;
+  TimerRing& operator=(const TimerRing&) = delete;
+  ~TimerRing() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
+  // The next pair (its events are created on first use), or two null events when every slot has been used since the reset.
+  cudaError_t next(cudaEvent_t& e0, cudaEvent_t& e1) {
+    e0 = e1 = nullptr;
+    if (used == kSlots) return cudaSuccess;
+    while ((int)ev.size() < 2 * (used + 1)) {
+      cudaEvent_t e = nullptr;
+      const cudaError_t err = cudaEventCreate(&e);
+      if (err != cudaSuccess) return err;
+      ev.push_back(e);
+    }
+    e0 = ev[2 * used]; e1 = ev[2 * used + 1];
+    ++used;
+    return cudaSuccess;
+  }
+  // Milliseconds of the first min(used, capacity) pairs; the events must have completed.
+  cudaError_t read(float* ms, uint32_t capacity, uint32_t* n) const {
+    uint32_t k = 0;
+    for (; k < (uint32_t)used && k < capacity; ++k) {
+      const cudaError_t err = cudaEventElapsedTime(&ms[k], ev[2 * k], ev[2 * k + 1]);
+      if (err != cudaSuccess) return err;
+    }
+    *n = k;
+    return cudaSuccess;
+  }
+};
+
+// Identifies the IBS tile list on the device: a repeated request (the benchmark loop, HallME-style reruns) neither builds nor
+// uploads it again.
+struct TileKey {
+  enum Kind : uint64_t { kNone, kUpper, kBand, kList };
+  Kind kind = kNone;
+  uint64_t a = 0, b = 0;   // kUpper: first, stride; kBand: first and end tile row; kList: FNV-1a hash of the coordinates, tiles per side
+  uint64_t n = 0;          // tiles
+  bool operator==(const TileKey& o) const { return kind == o.kind && a == o.a && b == o.b && n == o.n; }
+};
+
+// A tile list: its key and, for a list of coordinates from the host, the coordinates. The tiles of a range of the upper triangle
+// or of a band of tile rows follow from the key (tile_coords).
+struct TileList {
+  TileKey key;
+  std::vector<uint2> coords;
 };
 
 }  // namespace
@@ -69,10 +124,7 @@ struct kgl_b200_ctx {
   cudaStream_t own_stream = nullptr, stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   bool ev_valid = false;
-  // ring of event pairs around every k_count_moments launch since the last reset (bench.py's live roofline timing)
-  static constexpr int kTimerSlots = 256;
-  std::vector<cudaEvent_t> timer_ev;
-  int timer_used = 0;
+  TimerRing timer;                        // around every launch of the streaming kernel (bench.py's live roofline timing)
   bool count_loci_in_accumulate = false;
   cudaEvent_t last_e0 = nullptr, last_e1 = nullptr;
   std::string err;
@@ -126,7 +178,6 @@ struct kgl_b200_ctx {
     unsigned long long* ecorr_fx() const { return reinterpret_cast<unsigned long long*>(acc.p + kEcorrOff); }
     uint32_t* nz_rare(uint64_t npad) const { return reinterpret_cast<uint32_t*>(acc.p + kEcorrOff + npad * 16); }
     double fx = 0.0;        // fixed-point scale of this set's sums (fx_scale_for the rows of the selection window it was prepared for)
-    void release() { flags16.release(); sum64.release(); selw.release(); acc.release(); }
   } prep[2];
   int par = 0;                                  // the set the current selection was prepared into
   // Three streams per pass (DESIGN 4): the streaming kernel on the context stream; the preparation of the NEXT pass and the
@@ -213,10 +264,9 @@ struct kgl_b200_ctx {
   DevBuf<uint32_t> d_ibs_lo, d_ibs_hi, d_sm_valid, d_ibs_acc, d_ibs_tiles_out;
   DevBuf<uint2> d_ibs_tiles;
   int ibs_mode = -1;                 // 0: no code-3 cell; 1: in-kernel validity plane; 2: pre-masked planes + sparse repair
-  std::vector<cudaEvent_t> ibs_timer_ev;
-  int ibs_timer_used = 0;
+  TimerRing ibs_timer;
   uint64_t ibs_last_count = 0;
-  uint64_t ibs_tiles_key[4] = {~0ull, 0, 0, 0};   // the tile list on the device: {kind, first, stride, count}
+  TileKey ibs_tiles_key;                 // the tile list on the device
   // AF-bin passes (CalcFWS): row mask, its 64-row summaries, the all-genomes population tables
   DevBuf<uint16_t> d_bin_flags, d_bin_sum64;
   DevBuf<uint32_t> d_bin_popmask32, d_bin_state;   // d_bin_state: [0] all-selected flag (always 0), [1] rows in the bin
@@ -235,8 +285,9 @@ struct kgl_b200_ctx {
   DevBuf<uint2> d_gram_tiles;
   DevBuf<double> d_gp_chunks, d_gp;
   DevBuf<uint8_t> d_gram_out;
-  uint64_t gram_ld = 0, gram_tiles_ld = 0, gram_n_tiles = 0, gram_first = 0, gram_stride = 1;
+  uint64_t gram_tiles_ld = 0, gram_n_tiles = 0, gram_first = 0, gram_stride = 1;
   bool codes16_valid = false;
+  bool gram_valid = false;             // d_gram holds the last kgl_b200_enqueue_gram[_tiles] result (the IBS tensor form lends it out)
   cudaEvent_t gram_e0 = nullptr, gram_e1 = nullptr;
   // KING-robust kinship (king.cuh): raw code matrix (code 3 kept), M = H C^T blocks, dense slab, pair list and its sort
   DevBuf<uint32_t> d_codes_raw;
@@ -252,6 +303,8 @@ struct kgl_b200_ctx {
   int algo = -1, phase = 0, iteration = 0;
   kgl_b200_inbreed_options opt{};
   std::vector<double> hall_start;
+
+  ~kgl_b200_ctx();
 };
 
 namespace {
@@ -591,17 +644,9 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
   P.cta_counts = want_genome ? c->d_cta_counts[c->cbuf].p : nullptr;
   P.n_genomes_padded = (uint32_t)c->Npad;
   stream_make_tensor_map(P, pl, c->padded_rows);          // wide populations: one 2-D TMA box per stage
-  cudaEvent_t e0 = c->ev0, e1 = c->ev1;
-  if (c->timer_used < kgl_b200_ctx::kTimerSlots) {
-    if ((int)c->timer_ev.size() < 2 * (c->timer_used + 1)) {
-      cudaEvent_t a0 = nullptr, a1 = nullptr;
-      KGL_CUDA(c, cudaEventCreate(&a0));
-      KGL_CUDA(c, cudaEventCreate(&a1));
-      c->timer_ev.push_back(a0); c->timer_ev.push_back(a1);
-    }
-    e0 = c->timer_ev[2 * c->timer_used]; e1 = c->timer_ev[2 * c->timer_used + 1];
-    ++c->timer_used;
-  }
+  cudaEvent_t e0, e1;
+  KGL_CUDA(c, c->timer.next(e0, e1));
+  if (!e0) { e0 = c->ev0; e1 = c->ev1; }       // the ring is full: kgl_b200_last_stream_kernel_ms still times this launch
   KGL_CUDA(c, cudaEventRecord(e0, c->stream));
   KGL_CUDA(c, launch_stream(P, pl, want_locus_counts, want_genome, c->stream));
   ++c->launches;
@@ -855,10 +900,7 @@ __global__ void k_mom_copy_limits(const double* __restrict__ src, uint64_t n, do
   if (g < n) { limits[g * 3 + 0] = src[g * 3 + 0]; limits[g * 3 + 1] = src[g * 3 + 1]; }
 }
 
-bool moments_enabled(const kgl_b200_ctx* c) {
-  static const bool on = std::getenv("KGL_B200_EXACT_SWEEPS") == nullptr;
-  return on && !c->opt.exact_sweeps;
-}
+bool moments_enabled(const kgl_b200_ctx* c) { return !c->opt.exact_sweeps; }
 
 // Tiles (of tile_genomes genomes) that hold a genome of each population, from the host copy of the assignment; returns the widest range.
 uint32_t moment_tile_ranges(const kgl_b200_ctx* c, uint32_t tile_genomes, uint32_t (&lo)[kMaxPop], uint32_t (&hi)[kMaxPop]) {
@@ -966,11 +1008,10 @@ int ensure_moments(kgl_b200_ctx* c, bool want_lists) {
   int sbits = 61; for (uint64_t v = longest; v; v >>= 1) --sbits;
   const double scale = std::ldexp(1.0, std::min(sbits, 46));          // the tensor-core payload has six 8-bit limbs for U + 2^s
   const uint32_t n_units = unit_out[0], n_btiles = unit_out[1];
-  static const bool mma_off = std::getenv("KGL_B200_MOMENTS_NO_MMA") != nullptr;
   // scratch of the tensor-core builder (payload tiles, per-unit counts and offsets)
   // (a quarter of the device's memory, from the properties read at kgl_b200_create: cudaMemGetInfo stalls the host for milliseconds)
   const uint64_t scratch_limit = std::max<uint64_t>(4ull << 30, c->total_memory / 4);
-  const bool use_mma = !mma_off && !c->opt.moments_on_cuda_cores && unit_out[2] <= kMomMaxUnits && n_units > 0 &&
+  const bool use_mma = !c->opt.moments_on_cuda_cores && unit_out[2] <= kMomMaxUnits && n_units > 0 &&
                        (uint64_t)n_btiles * 2 * kMmaBTile + (want_lists ? (uint64_t)n_units * npad * 8 : 0) <= scratch_limit;
   KGL_CUDA(c, c->d_mom_pm.ensure_roomy((size_t)c->n_pop * nbt * kMomJ));
   KGL_CUDA(c, c->d_mom_mi.ensure_roomy((size_t)npad * nbt * kMomJ));
@@ -1101,6 +1142,10 @@ int ensure_ibs_planes(kgl_b200_ctx* c) {
 
 uint64_t ibs_side(const kgl_b200_ctx* c) { return (c->N + kIbsT - 1) / kIbsT; }
 
+// Row pitch of the Gram matrices and code matrices (gram_i8.cuh), and the k-stages of a Gram run over all loci.
+uint64_t gram_ld(const kgl_b200_ctx* c) { return (c->N + kGramN - 1) / kGramN * kGramN; }
+uint32_t gram_k_stages(const kgl_b200_ctx* c) { return (uint32_t)((c->L + kGramK - 1) / kGramK); }
+
 // t-th tile of the row-major upper triangle (ti <= tj) of a side x side tile grid.
 uint2 ibs_upper_tile(uint64_t t, uint64_t side) {
   // row ti starts at ti*side - ti*(ti-1)/2
@@ -1114,15 +1159,82 @@ uint2 ibs_upper_tile(uint64_t t, uint64_t side) {
   return make_uint2((uint32_t)lo, (uint32_t)(lo + (t - start)));
 }
 
-int ensure_codes16(kgl_b200_ctx* c);
-
 constexpr uint64_t kIbsMaxTilesPerLaunch = 8192;     // 384 MB of accumulators
+
+// Tiles first, first + stride, ... (count of them) of the row-major upper triangle.
+TileList upper_tiles(uint64_t first, uint64_t stride, uint64_t count) { return {{TileKey::kUpper, first, stride, count}, {}}; }
+
+// Every tile of the tile rows [tr0, tr1).
+TileList band_tiles(uint64_t tr0, uint64_t tr1, uint64_t side) { return {{TileKey::kBand, tr0, tr1, (tr1 - tr0) * side}, {}}; }
+
+// count tiles {row, column} from the host, each inside the grid and, when upper_only, not below the diagonal.
+int listed_tiles(kgl_b200_ctx* c, const uint32_t* coords, uint64_t count, bool upper_only, TileList& out) {
+  const uint64_t side = ibs_side(c);
+  uint64_t hash = 1469598103934665603ull;
+  out.coords.resize(count);
+  for (uint64_t i = 0; i < count; ++i) {
+    const uint32_t ti = coords[2 * i], tj = coords[2 * i + 1];
+    if (ti >= side || tj >= side) return fail(c, KGL_B200_ERR_INVALID, "tile coordinate outside the grid");
+    if (upper_only && ti > tj) return fail(c, KGL_B200_ERR_INVALID, "tile below the diagonal (need tile row <= tile column)");
+    out.coords[i] = make_uint2(ti, tj);
+    hash = (hash ^ ti) * 1099511628211ull; hash = (hash ^ tj) * 1099511628211ull;
+  }
+  out.key = {TileKey::kList, hash, side, count};
+  return KGL_B200_OK;
+}
+
+std::vector<uint2> tile_coords(const TileList& list, uint64_t side) {
+  const TileKey& k = list.key;
+  if (k.kind == TileKey::kList) return list.coords;
+  std::vector<uint2> tiles;
+  tiles.reserve(k.n);
+  if (k.kind == TileKey::kUpper) {
+    for (uint64_t i = 0; i < k.n; ++i) tiles.push_back(ibs_upper_tile(k.a + i * k.b, side));
+  } else {
+    for (uint64_t ta = k.a; ta < k.b; ++ta)
+      for (uint64_t tb = 0; tb < side; ++tb) tiles.push_back(make_uint2((uint32_t)ta, (uint32_t)tb));
+  }
+  return tiles;
+}
+
+// The 2-bit code matrix of the Gram runs in row-block-major layout, once per upload. keep_code3: the copy that keeps code 3
+// (k_codes16<true>), the code-3 indicator operand of KING's M = H C^T, built only for populations that have code-3 cells.
+template <bool keep_code3>
+int ensure_codes(kgl_b200_ctx* c) {
+  DevBuf<uint32_t>& codes = keep_code3 ? c->d_codes_raw : c->d_codes16;
+  bool& valid = keep_code3 ? c->codes_raw_valid : c->codes16_valid;
+  int rc = ensure_sample_major(c); if (rc) return rc;
+  if (valid) return KGL_B200_OK;
+  const uint64_t ld = gram_ld(c), k_stages = gram_k_stages(c);
+  const size_t words = (size_t)ld * k_stages * 8;
+  KGL_CUDA(c, codes.ensure(words));
+  KGL_CUDA(c, cudaMemsetAsync(codes.p, 0, words * 4, c->stream));
+  k_codes16<keep_code3><<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks,
+                                                                                                          c->n_words, k_stages, ld, codes.p);
+  KGL_LAUNCH_CHECK(c);
+  valid = true;
+  return KGL_B200_OK;
+}
+
+// One Gram run, table_a x table_b, over the 256 x 256 blocks under the current IBS tile list, into compact blocks: plan, clear
+// the output when the run is chunked (the chunks add into it), launch.
+int run_gram_blocks(kgl_b200_ctx* c, const uint32_t* codes, uint32_t table_a, uint32_t table_b, int32_t* out) {
+  const uint32_t k_stages = gram_k_stages(c);
+  const GramPlan gp = plan_gram(std::max<uint32_t>(c->ibs_n_blocks, 1), k_stages, c->sm_count);
+  GramParams G{};
+  G.codes = codes; G.k_stages = k_stages; G.tiles = c->d_ibs_blocks.p; G.n_tiles = c->ibs_n_blocks;
+  G.stages_per_chunk = gp.stages_per_chunk; G.n_chunks = gp.n_chunks; G.out = out; G.ld = gram_ld(c); G.compact = 1;
+  G.table_a = table_a; G.table_b = table_b;
+  if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(out, 0, (size_t)c->ibs_n_blocks * kGramM * kGramN * 4, c->stream));
+  KGL_CUDA(c, launch_gram(G, gp, c->stream));
+  ++c->launches;
+  return KGL_B200_OK;
+}
 
 // The genomes' heterozygous / hom-alt cells on the IBS planes (code 3 in neither), once per upload.
 int ensure_ibs_class(kgl_b200_ctx* c) {
   if (c->ibs_class_valid) return KGL_B200_OK;
-  const uint64_t ld = (c->N + kGramN - 1) / kGramN * kGramN;
-  const size_t n_rows = (size_t)std::max<uint64_t>(c->n_gblocks * 32, ld);
+  const size_t n_rows = (size_t)std::max<uint64_t>(c->n_gblocks * 32, gram_ld(c));
   KGL_CUDA(c, c->d_ibs_class.ensure(n_rows * 2));
   KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_class.p, 0, n_rows * 2 * 4, c->stream));
   const uint32_t wpc = 4096;
@@ -1133,36 +1245,31 @@ int ensure_ibs_class(kgl_b200_ctx* c) {
   return KGL_B200_OK;
 }
 
-// Dense kernel (+ sparse repair) over a host tile list; leaves acc[n][3][4096] in d_ibs_acc. n <= kIbsMaxTilesPerLaunch.
-// `key` identifies the list: a repeated request (the benchmark loop, HallME-style reruns) skips the upload and its sync.
+// Dense kernel (+ sparse repair) over a tile list; leaves acc[n][3][4096] in d_ibs_acc. n <= kIbsMaxTilesPerLaunch.
 // want_blocks: build the 256 x 256 block list under the tiles also when the popcount kernel runs (KING's Gram runs use it).
-int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const uint64_t (&key)[4], uint32_t n_cached = 0,
-                      bool want_blocks = false) {
-  const uint32_t n = tiles.empty() ? n_cached : (uint32_t)tiles.size();
+int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = false) {
+  const uint32_t n = (uint32_t)list.key.n;
   KGL_CUDA(c, c->d_ibs_tiles.ensure(n));
   KGL_CUDA(c, c->d_ibs_acc.ensure((size_t)n * 3 * kIbsTileCells));
   // Tensor-core form of the dense part: populations whose code-3 cells are indexed (or absent), n_loci < 2^29
-  static const bool tensor_off = std::getenv("KGL_B200_IBS_POPCOUNT") != nullptr;
-  c->gram_ld = (c->N + kGramN - 1) / kGramN * kGramN;
-  const bool tensor = !tensor_off && c->ibs_tensor_enabled && c->ibs_mode != 1 && c->L < (1ull << 29);
+  const bool tensor = c->ibs_tensor_enabled && c->ibs_mode != 1 && c->L < (1ull << 29);
   const bool need_blocks = tensor || want_blocks;
   if (tensor) {
-    int rc = ensure_codes16(c); if (rc) return rc;
+    int rc = ensure_codes<false>(c); if (rc) return rc;
     rc = ensure_ibs_class(c); if (rc) return rc;
   }
-  if (std::memcmp(key, c->ibs_tiles_key, sizeof key) != 0 || (need_blocks && c->ibs_n_blocks == 0)) {
-    std::vector<uint2> list = tiles;
-    if (list.empty()) return fail(c, KGL_B200_ERR_STATE, "tile list not available");
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_ibs_tiles.p, list.data(), (size_t)n * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+  if (!(list.key == c->ibs_tiles_key) || (need_blocks && c->ibs_n_blocks == 0)) {
+    const std::vector<uint2> tiles = tile_coords(list, ibs_side(c));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_ibs_tiles.p, tiles.data(), (size_t)n * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
     std::vector<uint2> blocks;
     std::vector<uint32_t> tile_block;
     c->ibs_n_blocks = 0;                 // a list uploaded without its blocks must not inherit the block count of the one before
     if (need_blocks) {
       // the 256 x 256 Gram blocks under the tiles (upper triangle of the block grid; a tile below the diagonal uses the mirror block)
       std::unordered_map<uint64_t, uint32_t> index;
-      tile_block.resize(list.size());
-      for (size_t t = 0; t < list.size(); ++t) {
-        uint32_t bi = list[t].x / kIbsTilesPerBlock, bj = list[t].y / kIbsTilesPerBlock;
+      tile_block.resize(tiles.size());
+      for (size_t t = 0; t < tiles.size(); ++t) {
+        uint32_t bi = tiles[t].x / kIbsTilesPerBlock, bj = tiles[t].y / kIbsTilesPerBlock;
         const bool mirrored = bi > bj;
         if (mirrored) std::swap(bi, bj);
         const uint64_t k2 = ((uint64_t)bi << 32) | bj;
@@ -1177,10 +1284,11 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const ui
       c->ibs_n_blocks = (uint32_t)blocks.size();
     }
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));     // the lists are pageable host memory
-    std::memcpy(c->ibs_tiles_key, key, sizeof key);
+    c->ibs_tiles_key = list.key;
   }
   if (tensor) {
     const size_t block_cells = (size_t)c->ibs_n_blocks * kGramM * kGramN;
+    c->gram_valid = false;                                  // d_gram holds the dosage blocks from here on
     KGL_CUDA(c, c->d_gram.ensure(block_cells));             // (also kgl_b200_run_gram's matrix: that call sizes it for itself)
     KGL_CUDA(c, c->d_gram_hh.ensure(block_cells));
     KGL_CUDA(c, c->d_gram_aa.ensure(block_cells));
@@ -1195,33 +1303,15 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const ui
   P.n_words = c->n_words; P.words_used = words_used; P.tiles = c->d_ibs_tiles.p; P.n_tiles = n;
   P.words_per_chunk = pl.words_per_chunk; P.n_chunks = pl.n_chunks; P.acc = c->d_ibs_acc.p;
   if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_acc.p, 0, (size_t)n * 3 * kIbsTileCells * 4, c->stream));
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (c->ibs_timer_used < kgl_b200_ctx::kTimerSlots) {
-    if ((int)c->ibs_timer_ev.size() < 2 * (c->ibs_timer_used + 1)) {
-      KGL_CUDA(c, cudaEventCreate(&e0));
-      KGL_CUDA(c, cudaEventCreate(&e1));
-      c->ibs_timer_ev.push_back(e0); c->ibs_timer_ev.push_back(e1);
-    }
-    e0 = c->ibs_timer_ev[2 * c->ibs_timer_used]; e1 = c->ibs_timer_ev[2 * c->ibs_timer_used + 1];
-    ++c->ibs_timer_used;
-  }
+  cudaEvent_t e0, e1;
+  KGL_CUDA(c, c->ibs_timer.next(e0, e1));
   if (e0) KGL_CUDA(c, cudaEventRecord(e0, c->stream));
   if (tensor) {
     // dense part on the tensor cores: three Gram matrices over the blocks the tile list touches, then the tile cells (ibs_gram.cuh)
-    const uint64_t ld = c->gram_ld;
-    const uint32_t k_stages = (uint32_t)((c->L + kGramK - 1) / kGramK);
-    const GramPlan gp = plan_gram(std::max<uint32_t>(c->ibs_n_blocks, 1), k_stages, c->sm_count);
-    GramParams G{};
-    G.codes = c->d_codes16.p; G.k_stages = k_stages; G.tiles = c->d_ibs_blocks.p; G.n_tiles = c->ibs_n_blocks;
-    G.stages_per_chunk = gp.stages_per_chunk; G.n_chunks = gp.n_chunks; G.ld = ld; G.compact = 1;
-    const size_t block_cells = (size_t)c->ibs_n_blocks * kGramM * kGramN;
     int32_t* outs[3] = {c->d_gram.p, c->d_gram_hh.p, c->d_gram_aa.p};
     const uint32_t tables[3] = {kGramTableDosage, kGramTableHet, kGramTableHomAlt};
     for (int m = 0; m < 3; ++m) {
-      G.out = outs[m]; G.table_a = G.table_b = tables[m];
-      if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(outs[m], 0, block_cells * 4, c->stream));
-      KGL_CUDA(c, launch_gram(G, gp, c->stream));
-      ++c->launches;
+      int rc = run_gram_blocks(c, c->d_codes16.p, tables[m], tables[m], outs[m]); if (rc) return rc;
     }
     k_ibs_from_grams<<<blocks_for((uint64_t)n * kIbsTileCells, 256), 256, 0, c->stream>>>(c->d_gram.p, c->d_gram_hh.p, c->d_gram_aa.p,
                                                                                          c->d_ibs_class.p, c->d_ibs_tiles.p, c->d_ibs_tile_block.p, n, c->d_ibs_acc.p);
@@ -1257,70 +1347,75 @@ int ibs_finalize(kgl_b200_ctx* c, uint32_t n_tiles, int mode, uint64_t row_begin
   return KGL_B200_OK;
 }
 
-// ---- K5: Gram matrix on the tensor cores -------------------------------------------------------------------------------
-int ensure_codes16(kgl_b200_ctx* c) {
-  int rc = ensure_sample_major(c); if (rc) return rc;
-  if (c->codes16_valid) return KGL_B200_OK;
-  c->gram_ld = (c->N + kGramN - 1) / kGramN * kGramN;
-  const uint64_t k_stages = (c->L + kGramK - 1) / kGramK;
-  const size_t words = (size_t)c->gram_ld * k_stages * 8;
-  KGL_CUDA(c, c->d_codes16.ensure(words));
-  KGL_CUDA(c, cudaMemsetAsync(c->d_codes16.p, 0, words * 4, c->stream));
-  k_codes16<false><<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks, c->n_words,
-                                                                                                     k_stages, c->gram_ld, c->d_codes16.p);
-  KGL_LAUNCH_CHECK(c);
-  c->codes16_valid = true;
+// The tiles of `list` for kgl_b200_ibs_tiles_buffer (kgl_b200_enqueue_ibs_tiles, kgl_b200_enqueue_ibs_tile_list).
+int ibs_enqueue_tiles(kgl_b200_ctx* c, const TileList& list) {
+  int rc = ibs_compute_tiles(c, list); if (rc) return rc;
+  const uint64_t count = list.key.n;
+  KGL_CUDA(c, c->d_ibs_tiles_out.ensure((size_t)count * kIbsTileCells * 4));
+  rc = ibs_finalize(c, (uint32_t)count, 0, 0, 0, 0, c->d_ibs_tiles_out.p); if (rc) return rc;
+  c->ibs_last_count = count;
   return KGL_B200_OK;
 }
 
-// The same layout with code 3 kept (k_codes16<true>): the code-3 indicator operand of KING's M = H C^T. Once per upload, and only
-// for populations that have code-3 cells.
-int ensure_codes_raw(kgl_b200_ctx* c) {
-  int rc = ensure_sample_major(c); if (rc) return rc;
-  if (c->codes_raw_valid) return KGL_B200_OK;
-  const uint64_t ld = (c->N + kGramN - 1) / kGramN * kGramN;
-  const uint64_t k_stages = (c->L + kGramK - 1) / kGramK;
-  const size_t words = (size_t)ld * k_stages * 8;
-  KGL_CUDA(c, c->d_codes_raw.ensure(words));
-  KGL_CUDA(c, cudaMemsetAsync(c->d_codes_raw.p, 0, words * 4, c->stream));
-  k_codes16<true><<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks, c->n_words,
-                                                                                                    k_stages, ld, c->d_codes_raw.p);
-  KGL_LAUNCH_CHECK(c);
-  c->codes_raw_valid = true;
+// count tiles to the host in calls of at most kIbsMaxTilesPerLaunch: enqueue(done, n) computes tiles [done, done + n) of them.
+template <class Enqueue>
+int ibs_run_tiles(kgl_b200_ctx* c, uint64_t count, uint32_t* out, Enqueue enqueue) {
+  for (uint64_t done = 0; done < count; done += kIbsMaxTilesPerLaunch) {
+    const uint64_t n = std::min<uint64_t>(kIbsMaxTilesPerLaunch, count - done);
+    int rc = enqueue(done, n); if (rc) return rc;
+    KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)done * kIbsTileCells * 4, c->d_ibs_tiles_out.p, (size_t)n * kIbsTileCells * 16, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  }
+  return KGL_B200_OK;
+}
+
+// Dense pairwise output of genomes [row_begin, row_end) against all genomes, per_pair values of T a pair, through the device
+// buffer `buf` to `out`. The whole matrix when it takes at most 2 GiB: the upper-triangle tiles, every tile also written
+// transposed. Otherwise slabs of whole tile rows that keep the device result under ~1 GiB. slab(tiles, r0, r1, mirror) writes
+// rows [r0, r1) of buf from one tile list of at most kIbsMaxTilesPerLaunch tiles.
+template <class T, class Slab>
+int run_pairwise(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, uint64_t per_pair, DevBuf<T>& buf, T* out, Slab slab) {
+  const uint64_t N = c->N, side = ibs_side(c), bytes = per_pair * sizeof(T);
+  if (row_begin == 0 && row_end == N && N * N * bytes <= (2ull << 30)) {
+    KGL_CUDA(c, buf.ensure((size_t)N * N * per_pair));
+    for (uint64_t t0 = 0, n_upper = side * (side + 1) / 2; t0 < n_upper; t0 += kIbsMaxTilesPerLaunch) {
+      int rc = slab(upper_tiles(t0, 1, std::min(n_upper - t0, kIbsMaxTilesPerLaunch)), 0, N, 1); if (rc) return rc;
+    }
+    KGL_CUDA(c, cudaMemcpyAsync(out, buf.p, (size_t)N * N * bytes, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KGL_B200_OK;
+  }
+  const uint64_t slab_tile_rows = std::max<uint64_t>(1, std::min<uint64_t>((1ull << 30) / (N * bytes * kIbsT), kIbsMaxTilesPerLaunch / side));
+  for (uint64_t tr0 = row_begin / kIbsT; tr0 * kIbsT < row_end; tr0 += slab_tile_rows) {
+    const uint64_t tr1 = std::min((row_end + kIbsT - 1) / kIbsT, tr0 + slab_tile_rows);
+    const uint64_t r0 = std::max(row_begin, tr0 * kIbsT), r1 = std::min(row_end, tr1 * kIbsT);
+    KGL_CUDA(c, buf.ensure((size_t)(r1 - r0) * N * per_pair));
+    int rc = slab(band_tiles(tr0, tr1, side), r0, r1, 0); if (rc) return rc;
+    KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)(r0 - row_begin) * N * per_pair, buf.p, (size_t)(r1 - r0) * N * bytes, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  }
   return KGL_B200_OK;
 }
 
 // ---- KING-robust kinship (king.cuh) -------------------------------------------------------------------------------------
 // One slab of tiles (<= kIbsMaxTilesPerLaunch): the IBS counts by ibs_compute_tiles in whichever form it picks, HH (already
 // filled by the tensor form, otherwise one Gram run) and, with code-3 cells, M = H C^T over the same blocks. Fills K.
-int king_compute_tiles(kgl_b200_ctx* c, const std::vector<uint2>& tiles, const uint64_t (&key)[4], KingTiles& K) {
-  int rc = ibs_compute_tiles(c, tiles, key, 0, true); if (rc) return rc;
+int king_compute_tiles(kgl_b200_ctx* c, const TileList& list, KingTiles& K) {
+  int rc = ibs_compute_tiles(c, list, true); if (rc) return rc;
   rc = ensure_ibs_class(c); if (rc) return rc;
-  const uint32_t n = (uint32_t)tiles.size();
   const size_t block_cells = (size_t)c->ibs_n_blocks * kGramM * kGramN;
-  const uint32_t k_stages = (uint32_t)((c->L + kGramK - 1) / kGramK);
-  const GramPlan gp = plan_gram(std::max<uint32_t>(c->ibs_n_blocks, 1), k_stages, c->sm_count);
-  GramParams G{};
-  G.k_stages = k_stages; G.tiles = c->d_ibs_blocks.p; G.n_tiles = c->ibs_n_blocks;
-  G.stages_per_chunk = gp.stages_per_chunk; G.n_chunks = gp.n_chunks; G.ld = c->gram_ld; G.compact = 1;
   if (!c->ibs_used_tensor) {                       // the popcount kernel ran: HH is not there yet
-    rc = ensure_codes16(c); if (rc) return rc;
+    rc = ensure_codes<false>(c); if (rc) return rc;
     KGL_CUDA(c, c->d_gram_hh.ensure(block_cells));
-    G.codes = c->d_codes16.p; G.out = c->d_gram_hh.p; G.table_a = G.table_b = kGramTableHet;
-    if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(G.out, 0, block_cells * 4, c->stream));
-    KGL_CUDA(c, launch_gram(G, gp, c->stream));
-    ++c->launches;
+    rc = run_gram_blocks(c, c->d_codes16.p, kGramTableHet, kGramTableHet, c->d_gram_hh.p); if (rc) return rc;
   }
   if (c->n_dropped > 0) {
-    rc = ensure_codes_raw(c); if (rc) return rc;
+    rc = ensure_codes<true>(c); if (rc) return rc;
     KGL_CUDA(c, c->d_king_m.ensure(block_cells));
-    G.codes = c->d_codes_raw.p; G.out = c->d_king_m.p; G.table_a = kGramTableHet; G.table_b = kGramTableCode3;
-    if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(G.out, 0, block_cells * 4, c->stream));
-    KGL_CUDA(c, launch_gram(G, gp, c->stream));
-    ++c->launches;
+    rc = run_gram_blocks(c, c->d_codes_raw.p, kGramTableHet, kGramTableCode3, c->d_king_m.p); if (rc) return rc;
   }
   K = KingTiles{};
-  K.acc = c->d_ibs_acc.p; K.tiles = c->d_ibs_tiles.p; K.n_tiles = n;
+  K.acc = c->d_ibs_acc.p; K.tiles = c->d_ibs_tiles.p; K.n_tiles = (uint32_t)list.key.n;
   K.valid_mode = c->ibs_mode; K.seg = c->ibs_mode == 2 ? c->d_dropped_seg.p : nullptr; K.n_loci = (uint32_t)c->L; K.n_genomes = c->N;
   K.hh = c->d_gram_hh.p; K.m = c->n_dropped > 0 ? c->d_king_m.p : nullptr; K.tile_block = c->d_ibs_tile_block.p; K.counts = c->d_ibs_class.p;
   return KGL_B200_OK;
@@ -1335,9 +1430,12 @@ int king_check(kgl_b200_ctx* c) {
 
 // Tiles first, first + stride, ... of the upper-triangle tile list (rank r of R: first = r, stride = R); the rest of the
 // matrix is left zero so that a SUM all-reduce of the int32 matrix over the ranks assembles it.
+// Not run_gram_blocks: the tiles are those of the whole ld x ld matrix, the matrix is also cleared when only some of its tiles
+// run (stride > 1), and kgl_b200_last_gram_kernel_ms times the launch alone, without that clear.
 int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
-  int rc = ensure_codes16(c); if (rc) return rc;
-  const uint64_t ld = c->gram_ld;
+  int rc = ensure_codes<false>(c); if (rc) return rc;
+  c->gram_valid = false;
+  const uint64_t ld = gram_ld(c);
   if (c->gram_tiles_ld != ld || c->gram_first != first || c->gram_stride != stride) {
     const std::vector<uint2> all = gram_upper_tiles(ld);
     std::vector<uint2> tiles;
@@ -1350,7 +1448,7 @@ int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
     c->gram_tiles_ld = ld; c->gram_n_tiles = first < all.size() ? tiles.size() : 0;
   }
   KGL_CUDA(c, c->d_gram.ensure((size_t)ld * ld));
-  const uint32_t k_stages = (uint32_t)((c->L + kGramK - 1) / kGramK);
+  const uint32_t k_stages = gram_k_stages(c);
   const GramPlan pl = plan_gram((uint32_t)std::max<uint64_t>(c->gram_n_tiles, 1), k_stages, c->sm_count);
   GramParams P{};
   P.codes = c->d_codes16.p; P.k_stages = k_stages; P.tiles = c->d_gram_tiles.p; P.n_tiles = (uint32_t)c->gram_n_tiles;
@@ -1361,10 +1459,23 @@ int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
   KGL_CUDA(c, cudaEventRecord(c->gram_e0, c->stream));
   if (c->gram_n_tiles > 0) { KGL_CUDA(c, launch_gram(P, pl, c->stream)); ++c->launches; }
   KGL_CUDA(c, cudaEventRecord(c->gram_e1, c->stream));
+  c->gram_valid = true;
   return KGL_B200_OK;
 }
 
 }  // namespace
+
+// The device buffers free themselves (DevBuf) after this body, the peer regions that map d_xchg must be gone by then.
+kgl_b200_ctx::~kgl_b200_ctx() {
+  cudaSetDevice(device);
+  for (cudaStream_t s : {stream, tail_stream, prep_stream}) if (s) cudaStreamSynchronize(s);
+  peer_detach(this); peer_unregister(this);
+  for (cudaEvent_t e : {ev0, ev1, gram_e0, gram_e1, prep_done, inputs_ready}) if (e) cudaEventDestroy(e);
+  for (int i = 0; i < 2; ++i)
+    for (cudaEvent_t e : {readers_main[i], readers_tail[i], stream_done[i], tail_done[i]}) if (e) cudaEventDestroy(e);
+  for (cudaEvent_t e : chunk_ev) cudaEventDestroy(e);
+  for (cudaStream_t s : {prep_stream, tail_stream, copy_stream, own_stream}) if (s) cudaStreamDestroy(s);
+}
 
 // ---------------------------------------------------------------------------------------------------------------------
 extern "C" {
@@ -1415,50 +1526,7 @@ int kgl_b200_create(int device, kgl_b200_ctx** out) {
   return KGL_B200_OK;
 }
 
-void kgl_b200_destroy(kgl_b200_ctx* c) {
-  if (!c) return;
-  cudaSetDevice(c->device);
-  cudaStreamSynchronize(c->stream);
-  if (c->tail_stream) cudaStreamSynchronize(c->tail_stream);
-  if (c->prep_stream) cudaStreamSynchronize(c->prep_stream);
-  c->d_packed.release(); c->d_af.release(); c->d_superpop.release(); c->d_sel.release(); c->d_need32.release();
-  c->d_popmask.release(); c->prep[0].release(); c->prep[1].release();
-  c->d_sm_lo.release(); c->d_sm_hi.release(); c->d_locus_counts.release(); c->d_cta_counts[0].release(); c->d_cta_counts[1].release(); c->d_scratch.release(); c->d_dropped_cells.release(); c->d_zero_rare.release();
-  c->d_multi_rows.release(); c->d_multi_counts.release(); c->d_multi_af.release(); c->d_multi_cells.release(); c->d_multi_tab.release(); c->d_multi_out.release();
-  c->d_dropped.release(); c->d_dropped_seg.release(); c->d_dropped_counter.release(); c->d_dropped_unsorted.release(); c->d_sort_temp.release();
-  c->d_partials.release(); c->d_iter.release(); c->d_f.release();
-  c->d_bracket.release(); c->d_chunk_out.release(); c->d_inbreeding.release(); c->d_grid.release(); c->d_done.release();
-  c->d_flag.release(); c->d_genome_counts.release(); c->d_results.release(); c->d_ibs.release();
-  c->d_ibs_lo.release(); c->d_ibs_hi.release(); c->d_sm_valid.release(); c->d_ibs_acc.release(); c->d_ibs_tiles_out.release(); c->d_ibs_tiles.release(); c->d_offsets.release(); c->d_sel_counts.release(); c->d_locus_keep.release();
-  c->d_bin_flags.release(); c->d_bin_sum64.release(); c->d_bin_popmask32.release(); c->d_bin_state.release(); c->d_bin_need32.release();
-  c->d_zero_superpop.release(); c->d_bin_out.release();
-  peer_detach(c); peer_unregister(c);
-  c->d_xchg.release(); c->d_peer_error.release();
-  c->d_terms_table.release(); c->d_list_count.release();
-  c->d_chain_u32.release(); c->d_chain_mark.release();
-  c->d_list.release(); c->d_sm_codes.release(); c->d_limits.release(); c->d_slow_out.release(); c->d_lane_state.release(); c->d_n_slow.release();
-  c->d_codes_raw.release(); c->d_king_m.release(); c->d_king_out.release(); c->d_king_pairs.release(); c->d_king_sorted.release();
-  c->d_king_keys.release(); c->d_king_keys2.release(); c->d_king_cursor.release(); c->d_king_index.release(); c->d_king_index2.release(); c->d_king_sort_temp.release();
-  c->d_codes16.release(); c->d_gram.release(); c->d_gram_tiles.release(); c->d_gp_chunks.release(); c->d_gp.release(); c->d_gram_out.release();
-  if (c->gram_e0) cudaEventDestroy(c->gram_e0);
-  if (c->gram_e1) cudaEventDestroy(c->gram_e1);
-  for (cudaEvent_t e : c->timer_ev) cudaEventDestroy(e);
-  for (cudaEvent_t e : c->ibs_timer_ev) cudaEventDestroy(e);
-  if (c->ev0) cudaEventDestroy(c->ev0);
-  if (c->ev1) cudaEventDestroy(c->ev1);
-  if (c->tail_stream) cudaStreamSynchronize(c->tail_stream);
-  if (c->prep_stream) cudaStreamSynchronize(c->prep_stream);
-  if (c->prep_done) cudaEventDestroy(c->prep_done);
-  if (c->inputs_ready) cudaEventDestroy(c->inputs_ready);
-  for (int i = 0; i < 2; ++i)
-    for (cudaEvent_t e : {c->readers_main[i], c->readers_tail[i], c->stream_done[i], c->tail_done[i]}) if (e) cudaEventDestroy(e);
-  if (c->prep_stream) cudaStreamDestroy(c->prep_stream);
-  if (c->tail_stream) cudaStreamDestroy(c->tail_stream);
-  if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  for (cudaEvent_t ev : c->chunk_ev) cudaEventDestroy(ev);
-  if (c->own_stream) cudaStreamDestroy(c->own_stream);
-  delete c;
-}
+void kgl_b200_destroy(kgl_b200_ctx* c) { delete c; }
 
 const char* kgl_b200_last_error(const kgl_b200_ctx* c) { return c ? c->err.c_str() : tl_create_error.c_str(); }
 
@@ -1488,7 +1556,7 @@ float kgl_b200_last_stream_kernel_ms(kgl_b200_ctx* c) {
 
 int kgl_b200_kernel_timer_reset(kgl_b200_ctx* c) {
   if (!c) return KGL_B200_ERR_INVALID;
-  c->timer_used = 0;
+  c->timer.used = 0;
   return KGL_B200_OK;
 }
 
@@ -1496,10 +1564,7 @@ int kgl_b200_kernel_timer_read(kgl_b200_ctx* c, float* ms, uint32_t capacity, ui
   if (!c || !ms || !n) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   int rc = use_device(c); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  uint32_t k = 0;
-  for (int i = 0; i < c->timer_used && k < capacity; ++i, ++k)
-    KGL_CUDA(c, cudaEventElapsedTime(&ms[k], c->timer_ev[2 * i], c->timer_ev[2 * i + 1]));
-  *n = k;
+  KGL_CUDA(c, c->timer.read(ms, capacity, n));
   return KGL_B200_OK;
 }
 
@@ -1514,8 +1579,8 @@ static int set_shape(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_loci, uint6
   c->N = n_genomes; c->L = n_loci; c->row_bytes = row_bytes; c->host_units = row_bytes / 16;
   c->n_multi = 0;                    // the side cells belong to the matrix: kgl_b200_upload_multi_allelic comes after it
   c->units = stream_units_padded(c->host_units); c->Npad = c->units * 64;
-  c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key[0] = ~0ull; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
-  c->codes16_valid = false; c->codes_raw_valid = false;
+  c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
+  c->codes16_valid = false; c->codes_raw_valid = false; c->gram_valid = false;
   return KGL_B200_OK;
 }
 
@@ -2369,83 +2434,23 @@ int kgl_b200_run_ibs(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, uint
   rc = require_population(c, false); if (rc) return rc;
   if (row_begin >= row_end || row_end > c->N) return fail(c, KGL_B200_ERR_INVALID, "bad genome row range");
   rc = ensure_ibs_planes(c); if (rc) return rc;
-  const uint64_t side = ibs_side(c);
-  const bool whole = row_begin == 0 && row_end == c->N && c->N * c->N * 16 <= (2ull << 30);
-  if (whole) {
-    // the whole matrix: upper-triangle tiles, every tile also written transposed
-    KGL_CUDA(c, c->d_ibs.ensure((size_t)c->N * c->N * 4));
-    std::vector<uint2> tiles;
-    for (uint64_t t0 = 0, n_upper = side * (side + 1) / 2; t0 < n_upper; t0 += kIbsMaxTilesPerLaunch) {
-      tiles.clear();
-      for (uint64_t t = t0; t < std::min(n_upper, t0 + kIbsMaxTilesPerLaunch); ++t) tiles.push_back(ibs_upper_tile(t, side));
-      const uint64_t key[4] = {1, t0, 1, tiles.size()};
-      rc = ibs_compute_tiles(c, tiles, key); if (rc) return rc;
-      rc = ibs_finalize(c, (uint32_t)tiles.size(), 1, 0, c->N, 1, c->d_ibs.p); if (rc) return rc;
-    }
-    KGL_CUDA(c, cudaMemcpyAsync(out, c->d_ibs.p, (size_t)c->N * c->N * 16, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-    return KGL_B200_OK;
-  }
-  // a band of rows: every tile of the band's tile rows, in slabs that keep the device result under ~1 GiB
-  const uint64_t slab_tile_rows = std::max<uint64_t>(1, std::min<uint64_t>((1ull << 30) / (c->N * 16 * kIbsT), kIbsMaxTilesPerLaunch / side));
-  std::vector<uint2> tiles;
-  for (uint64_t tr0 = row_begin / kIbsT; tr0 * kIbsT < row_end; tr0 += slab_tile_rows) {
-    const uint64_t tr1 = std::min((row_end + kIbsT - 1) / kIbsT, tr0 + slab_tile_rows);
-    const uint64_t r0 = std::max(row_begin, tr0 * kIbsT), r1 = std::min(row_end, tr1 * kIbsT);
-    tiles.clear();
-    for (uint64_t ta = tr0; ta < tr1; ++ta)
-      for (uint64_t tb = 0; tb < side; ++tb) tiles.push_back(make_uint2((uint32_t)ta, (uint32_t)tb));
-    KGL_CUDA(c, c->d_ibs.ensure((size_t)(r1 - r0) * c->N * 4));
-    const uint64_t key[4] = {2, tr0, tr1, tiles.size()};
-    rc = ibs_compute_tiles(c, tiles, key); if (rc) return rc;
-    rc = ibs_finalize(c, (uint32_t)tiles.size(), 1, r0, r1, 0, c->d_ibs.p); if (rc) return rc;
-    KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)(r0 - row_begin) * c->N * 4, c->d_ibs.p, (size_t)(r1 - r0) * c->N * 16, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  }
-  return KGL_B200_OK;
+  return run_pairwise(c, row_begin, row_end, 4, c->d_ibs, out, [c](const TileList& tiles, uint64_t r0, uint64_t r1, int mirror) {
+    int rc = ibs_compute_tiles(c, tiles); if (rc) return rc;
+    return ibs_finalize(c, (uint32_t)tiles.key.n, 1, r0, r1, mirror, c->d_ibs.p);
+  });
 }
 
 int kgl_b200_run_king(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, double* kinship) {
   if (!c || !kinship) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   int rc = king_check(c); if (rc) return rc;
   if (row_begin >= row_end || row_end > c->N) return fail(c, KGL_B200_ERR_INVALID, "bad genome row range");
-  const uint64_t side = ibs_side(c);
-  KingTiles K{};
-  const bool whole = row_begin == 0 && row_end == c->N && c->N * c->N * 8 <= (2ull << 30);
-  if (whole) {
-    // the whole matrix: upper-triangle tiles, every tile also written transposed (the tile lists of kgl_b200_run_ibs)
-    KGL_CUDA(c, c->d_king_out.ensure((size_t)c->N * c->N));
-    std::vector<uint2> tiles;
-    for (uint64_t t0 = 0, n_upper = side * (side + 1) / 2; t0 < n_upper; t0 += kIbsMaxTilesPerLaunch) {
-      tiles.clear();
-      for (uint64_t t = t0; t < std::min(n_upper, t0 + kIbsMaxTilesPerLaunch); ++t) tiles.push_back(ibs_upper_tile(t, side));
-      const uint64_t key[4] = {1, t0, 1, tiles.size()};
-      rc = king_compute_tiles(c, tiles, key, K); if (rc) return rc;
-      k_king_dense<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, 0, c->N, 1, c->d_king_out.p);
-      KGL_LAUNCH_CHECK(c);
-    }
-    KGL_CUDA(c, cudaMemcpyAsync(kinship, c->d_king_out.p, (size_t)c->N * c->N * 8, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-    return KGL_B200_OK;
-  }
-  // a band of rows: every tile of the band's tile rows, in slabs that keep the device result under ~1 GiB
-  const uint64_t slab_tile_rows = std::max<uint64_t>(1, std::min<uint64_t>((1ull << 30) / (c->N * 8 * kIbsT), kIbsMaxTilesPerLaunch / side));
-  std::vector<uint2> tiles;
-  for (uint64_t tr0 = row_begin / kIbsT; tr0 * kIbsT < row_end; tr0 += slab_tile_rows) {
-    const uint64_t tr1 = std::min((row_end + kIbsT - 1) / kIbsT, tr0 + slab_tile_rows);
-    const uint64_t r0 = std::max(row_begin, tr0 * kIbsT), r1 = std::min(row_end, tr1 * kIbsT);
-    tiles.clear();
-    for (uint64_t ta = tr0; ta < tr1; ++ta)
-      for (uint64_t tb = 0; tb < side; ++tb) tiles.push_back(make_uint2((uint32_t)ta, (uint32_t)tb));
-    KGL_CUDA(c, c->d_king_out.ensure((size_t)(r1 - r0) * c->N));
-    const uint64_t key[4] = {2, tr0, tr1, tiles.size()};
-    rc = king_compute_tiles(c, tiles, key, K); if (rc) return rc;
-    k_king_dense<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, r0, r1, 0, c->d_king_out.p);
+  return run_pairwise(c, row_begin, row_end, 1, c->d_king_out, kinship, [c](const TileList& tiles, uint64_t r0, uint64_t r1, int mirror) {
+    KingTiles K{};
+    int rc = king_compute_tiles(c, tiles, K); if (rc) return rc;
+    k_king_dense<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, r0, r1, mirror, c->d_king_out.p);
     KGL_LAUNCH_CHECK(c);
-    KGL_CUDA(c, cudaMemcpyAsync(kinship + (size_t)(r0 - row_begin) * c->N, c->d_king_out.p, (size_t)(r1 - r0) * c->N * 8, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  }
-  return KGL_B200_OK;
+    return KGL_B200_OK;
+  });
 }
 
 int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* coords, double min_kinship, uint64_t capacity,
@@ -2455,9 +2460,15 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
   const uint64_t side = ibs_side(c), n_upper = side * (side + 1) / 2;
   const bool all = coords == nullptr || n_coords == 0;
   const uint64_t n_tiles = all ? n_upper : n_coords;
-  for (uint64_t i = 0; !all && i < n_coords; ++i) {
-    if (coords[2 * i] >= side || coords[2 * i + 1] >= side) return fail(c, KGL_B200_ERR_INVALID, "tile coordinate outside the grid");
-    if (coords[2 * i] > coords[2 * i + 1]) return fail(c, KGL_B200_ERR_INVALID, "tile below the diagonal (need tile row <= tile column)");
+  std::vector<TileList> slabs;           // every coordinate is checked before anything runs
+  for (uint64_t t0 = 0; t0 < n_tiles; t0 += kIbsMaxTilesPerLaunch) {
+    const uint64_t n = std::min(n_tiles - t0, kIbsMaxTilesPerLaunch);
+    if (all) {
+      slabs.push_back(upper_tiles(t0, 1, n));
+    } else {
+      slabs.emplace_back();
+      rc = listed_tiles(c, coords + 2 * t0, n, true, slabs.back()); if (rc) return rc;
+    }
   }
   // device list: no more records than the tiles hold, and indices that fit the uint32 sort values
   const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, n_tiles * kIbsTileCells), 0xFFFFFFFFull);
@@ -2467,18 +2478,8 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
   KGL_CUDA(c, c->d_king_cursor.ensure(1));
   KGL_CUDA(c, cudaMemsetAsync(c->d_king_cursor.p, 0, 8, c->stream));
   KingTiles K{};
-  std::vector<uint2> tiles;
-  for (uint64_t t0 = 0; t0 < n_tiles; t0 += kIbsMaxTilesPerLaunch) {
-    const uint64_t t1 = std::min(n_tiles, t0 + kIbsMaxTilesPerLaunch);
-    tiles.clear();
-    uint64_t hash = 1469598103934665603ull;                      // FNV-1a of the list, as kgl_b200_enqueue_ibs_tile_list
-    for (uint64_t t = t0; t < t1; ++t) {
-      const uint2 tc = all ? ibs_upper_tile(t, side) : make_uint2(coords[2 * t], coords[2 * t + 1]);
-      tiles.push_back(tc);
-      hash = (hash ^ tc.x) * 1099511628211ull; hash = (hash ^ tc.y) * 1099511628211ull;
-    }
-    const uint64_t key_all[4] = {1, t0, 1, tiles.size()}, key_list[4] = {3, hash, tiles.size(), side};
-    rc = king_compute_tiles(c, tiles, all ? key_all : key_list, K); if (rc) return rc;
+  for (const TileList& tiles : slabs) {
+    rc = king_compute_tiles(c, tiles, K); if (rc) return rc;
     k_king_pairs<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, min_kinship, dev_cap, c->d_king_pairs.p,
                                                                                                c->d_king_keys.p, c->d_king_index.p, c->d_king_cursor.p);
     KGL_LAUNCH_CHECK(c);
@@ -2512,7 +2513,7 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
 int kgl_b200_set_ibs_tensor_cores(kgl_b200_ctx* c, int enable) {
   if (!c) return KGL_B200_ERR_INVALID;
   c->ibs_tensor_enabled = enable != 0;
-  c->ibs_tiles_key[0] = ~0ull; c->ibs_n_blocks = 0;          // the cached tile list carries no block list for the other form
+  c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0;         // the cached tile list carries no block list for the other form
   return KGL_B200_OK;
 }
 
@@ -2535,61 +2536,28 @@ int kgl_b200_enqueue_ibs_tiles(kgl_b200_ctx* c, uint64_t first, uint64_t stride,
   if (stride == 0 || count == 0 || count > kIbsMaxTilesPerLaunch || first + (count - 1) * stride >= n_upper)
     return fail(c, KGL_B200_ERR_INVALID, "bad tile range (count must be 1..8192 per call and stay inside the upper triangle)");
   rc = ensure_ibs_planes(c); if (rc) return rc;
-  const uint64_t key[4] = {0, first, stride, count};
-  std::vector<uint2> tiles;
-  if (std::memcmp(key, c->ibs_tiles_key, sizeof key) != 0) {
-    tiles.resize(count);
-    for (uint64_t i = 0; i < count; ++i) tiles[i] = ibs_upper_tile(first + i * stride, side);
-  }
-  rc = ibs_compute_tiles(c, tiles, key, (uint32_t)count); if (rc) return rc;
-  KGL_CUDA(c, c->d_ibs_tiles_out.ensure((size_t)count * kIbsTileCells * 4));
-  rc = ibs_finalize(c, (uint32_t)count, 0, 0, 0, 0, c->d_ibs_tiles_out.p); if (rc) return rc;
-  c->ibs_last_count = count;
-  return KGL_B200_OK;
+  return ibs_enqueue_tiles(c, upper_tiles(first, stride, count));
 }
 
 int kgl_b200_enqueue_ibs_tile_list(kgl_b200_ctx* c, uint64_t count, const uint32_t* coords) {
   if (!c || !coords) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   int rc = use_device(c); if (rc) return rc;
   rc = require_population(c, false); if (rc) return rc;
-  const uint64_t side = ibs_side(c);
   if (count == 0 || count > kIbsMaxTilesPerLaunch) return fail(c, KGL_B200_ERR_INVALID, "bad tile count (1..8192 per call)");
-  uint64_t hash = 1469598103934665603ull;                       // FNV-1a of the list: a repeated request skips the upload
-  std::vector<uint2> tiles(count);
-  for (uint64_t i = 0; i < count; ++i) {
-    if (coords[2 * i] >= side || coords[2 * i + 1] >= side) return fail(c, KGL_B200_ERR_INVALID, "tile coordinate outside the grid");
-    tiles[i] = make_uint2(coords[2 * i], coords[2 * i + 1]);
-    hash = (hash ^ coords[2 * i]) * 1099511628211ull; hash = (hash ^ coords[2 * i + 1]) * 1099511628211ull;
-  }
+  TileList tiles;
+  rc = listed_tiles(c, coords, count, false, tiles); if (rc) return rc;
   rc = ensure_ibs_planes(c); if (rc) return rc;
-  const uint64_t key[4] = {3, hash, count, side};
-  rc = ibs_compute_tiles(c, tiles, key, (uint32_t)count); if (rc) return rc;
-  KGL_CUDA(c, c->d_ibs_tiles_out.ensure((size_t)count * kIbsTileCells * 4));
-  rc = ibs_finalize(c, (uint32_t)count, 0, 0, 0, 0, c->d_ibs_tiles_out.p); if (rc) return rc;
-  c->ibs_last_count = count;
-  return KGL_B200_OK;
+  return ibs_enqueue_tiles(c, tiles);
 }
 
 int kgl_b200_run_ibs_tile_list(kgl_b200_ctx* c, uint64_t count, const uint32_t* coords, uint32_t* out) {
   if (!c || !coords || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  for (uint64_t done = 0; done < count; done += kIbsMaxTilesPerLaunch) {
-    const uint64_t n = std::min<uint64_t>(kIbsMaxTilesPerLaunch, count - done);
-    int rc = kgl_b200_enqueue_ibs_tile_list(c, n, coords + 2 * done); if (rc) return rc;
-    KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)done * kIbsTileCells * 4, c->d_ibs_tiles_out.p, (size_t)n * kIbsTileCells * 16, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  }
-  return KGL_B200_OK;
+  return ibs_run_tiles(c, count, out, [&](uint64_t done, uint64_t n) { return kgl_b200_enqueue_ibs_tile_list(c, n, coords + 2 * done); });
 }
 
 int kgl_b200_run_ibs_tiles(kgl_b200_ctx* c, uint64_t first, uint64_t stride, uint64_t count, uint32_t* out) {
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  for (uint64_t done = 0; done < count; done += kIbsMaxTilesPerLaunch) {
-    const uint64_t n = std::min<uint64_t>(kIbsMaxTilesPerLaunch, count - done);
-    int rc = kgl_b200_enqueue_ibs_tiles(c, first + done * stride, stride, n); if (rc) return rc;
-    KGL_CUDA(c, cudaMemcpyAsync(out + (size_t)done * kIbsTileCells * 4, c->d_ibs_tiles_out.p, (size_t)n * kIbsTileCells * 16, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  }
-  return KGL_B200_OK;
+  return ibs_run_tiles(c, count, out, [&](uint64_t done, uint64_t n) { return kgl_b200_enqueue_ibs_tiles(c, first + done * stride, stride, n); });
 }
 
 int kgl_b200_ibs_tiles_buffer(kgl_b200_ctx* c, void** device_ptr, uint64_t* n_u32) {
@@ -2602,7 +2570,7 @@ int kgl_b200_ibs_tiles_buffer(kgl_b200_ctx* c, void** device_ptr, uint64_t* n_u3
 
 int kgl_b200_ibs_timer_reset(kgl_b200_ctx* c) {
   if (!c) return KGL_B200_ERR_INVALID;
-  c->ibs_timer_used = 0;
+  c->ibs_timer.used = 0;
   return KGL_B200_OK;
 }
 
@@ -2610,10 +2578,7 @@ int kgl_b200_ibs_timer_read(kgl_b200_ctx* c, float* ms, uint32_t capacity, uint3
   if (!c || !ms || !n) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   int rc = use_device(c); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  uint32_t k = 0;
-  for (int i = 0; i < c->ibs_timer_used && k < capacity; ++i, ++k)
-    KGL_CUDA(c, cudaEventElapsedTime(&ms[k], c->ibs_timer_ev[2 * i], c->ibs_timer_ev[2 * i + 1]));
-  *n = k;
+  KGL_CUDA(c, c->ibs_timer.read(ms, capacity, n));
   return KGL_B200_OK;
 }
 
@@ -2630,19 +2595,19 @@ int kgl_b200_enqueue_gram(kgl_b200_ctx* c) { return kgl_b200_enqueue_gram_tiles(
 
 int kgl_b200_gram_buffer(kgl_b200_ctx* c, void** device_ptr, uint64_t* n_int32, uint64_t* ld) {
   if (!c || !device_ptr || !n_int32) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  if (!c->d_gram.p) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
-  *device_ptr = c->d_gram.p; *n_int32 = c->gram_ld * c->gram_ld;
-  if (ld) *ld = c->gram_ld;
+  if (!c->gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
+  *device_ptr = c->d_gram.p; *n_int32 = gram_ld(c) * gram_ld(c);
+  if (ld) *ld = gram_ld(c);
   return KGL_B200_OK;
 }
 
 int kgl_b200_fetch_gram(kgl_b200_ctx* c, int32_t* out) {
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  if (!c->d_gram.p) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
+  if (!c->gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
   int rc = use_device(c); if (rc) return rc;
   const size_t n2 = (size_t)c->N * c->N;
   KGL_CUDA(c, c->d_gram_out.ensure(n2 * 4));
-  k_gram_finalize<<<blocks_for(n2, 256), 256, 0, c->stream>>>(c->d_gram.p, c->gram_ld, c->N, nullptr, 0, c->d_gram_out.p);
+  k_gram_finalize<<<blocks_for(n2, 256), 256, 0, c->stream>>>(c->d_gram.p, gram_ld(c), c->N, nullptr, 0, c->d_gram_out.p);
   KGL_LAUNCH_CHECK(c);
   KGL_CUDA(c, cudaMemcpyAsync(out, c->d_gram_out.p, n2 * 4, cudaMemcpyDeviceToHost, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -2679,7 +2644,7 @@ int kgl_b200_run_grm(kgl_b200_ctx* c, uint32_t pop, double* out) {
   KGL_LAUNCH_CHECK(c);
   const size_t n2 = (size_t)c->N * c->N;
   KGL_CUDA(c, c->d_gram_out.ensure(n2 * 8));
-  k_gram_finalize<<<blocks_for(n2, 256), 256, 0, c->stream>>>(c->d_gram.p, c->gram_ld, c->N, c->d_gp.p, rows, c->d_gram_out.p);
+  k_gram_finalize<<<blocks_for(n2, 256), 256, 0, c->stream>>>(c->d_gram.p, gram_ld(c), c->N, c->d_gp.p, rows, c->d_gram_out.p);
   KGL_LAUNCH_CHECK(c);
   KGL_CUDA(c, cudaMemcpyAsync(out, c->d_gram_out.p, n2 * 8, cudaMemcpyDeviceToHost, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
