@@ -219,6 +219,37 @@ int kgl_b200_run_king(kgl_b200_ctx* ctx, uint64_t row_begin, uint64_t row_end, d
 int kgl_b200_run_king_pairs(kgl_b200_ctx* ctx, uint64_t n_coords, const uint32_t* coords, double min_kinship, uint64_t capacity,
                             kgl_b200_king_pair* pairs, uint64_t* n_pairs);
 
+/* Genotype PCA (the ancestry axes of PLINK 2's --pca approx; Galinsky et al. 2016): the top principal components of the
+ * variance-standardised genotype matrix, matrix-free. For locus l with raw counts n0..n3 (kgl_b200_run_allele_count),
+ * v = n0 + n1 + n2 and p = (n1 + 2 n2) / (2 v). The used loci U are those with keep[l] != 0 (keep NULL = every locus) and
+ * 0 < p < 1; M = |U| (multi-allelic rows hold only 0 and 3: p = 0, never used). For l in U and a cell not coded 3,
+ *     z_lg = (g_lg - 2 p_l) / sqrt(2 p_l (1 - p_l)),   every other z_lg = 0    (code-3 cells mean-imputed, as PLINK does)
+ * and Psi = Z^T Z / M is PLINK's variance-standardised relationship matrix. It is never formed: Z^T Z times a block of <= 48
+ * columns runs as exact int8 Gram runs on the tensor cores against the block written as base-4 digits of a 30-bit fixed-point
+ * form (2^-29 of each column's largest entry; pca.cuh); the double arithmetic after the integer contractions is a fixed
+ * sequence of IEEE operations, so results are reproducible bit for bit. kgl_b200_run_pca is randomized subspace iteration
+ * (Halko, Martinsson & Tropp 2011, Alg. 4.4) on a block of b = 16 ceil((k + 6) / 16) columns from a Gaussian start block
+ * that is a pure function of (seed, genome, column): `iterations` products each followed by a Householder QR, then
+ * Rayleigh-Ritz with a cyclic Jacobi eigensolve of the b x b projection -- the QR and the eigensolve run on the host in
+ * double. Outputs: eigenvalues[k] of Psi in descending order; scores double[n_genomes][k], the unit eigenvectors, each signed
+ * so that its entry of largest magnitude is positive (the lowest index wins a tie); loadings (nullable) double[n_loci][k],
+ * u_i = Z v_i / sqrt(M lambda_i), 0 at unused loci; *n_loci_used = M (nullable). Needs a genotype upload
+ * (KGL_B200_ERR_STATE before it); KGL_B200_ERR_INVALID for k outside 1..40, k >= n_genomes, k > M, no used locus or
+ * n_loci >= 2^28. There is no popcount form: kgl_b200_set_ibs_tensor_cores does not apply. The device keeps a loci-major
+ * copy of the codes (n_genomes * n_loci / 4 bytes) from the first call after an upload. */
+typedef struct kgl_b200_pca_options {        /* zero-initialise for the defaults */
+  const uint8_t* keep;                       /* uint8[n_loci], 0 = leave the locus out; NULL = every locus */
+  uint32_t n_components;                     /* k, 1..40; 0 = 10 */
+  uint32_t iterations;                       /* q; 0 = 10 */
+  uint64_t seed;                             /* start block */
+} kgl_b200_pca_options;
+int kgl_b200_run_pca(kgl_b200_ctx* ctx, const kgl_b200_pca_options* options, double* eigenvalues /* [k] */,
+                     double* scores /* [n_genomes][k] */, double* loadings /* nullable, [n_loci][k] */, uint64_t* n_loci_used);
+/* y = Z^T Z x (not divided by M) for a block of 1 <= n_cols <= 48 columns: the operator itself, on the loci of `keep` (as
+ * above). A locus-sharded caller sums it over ranks. Same errors as kgl_b200_run_pca (n_cols outside 1..48: INVALID). */
+int kgl_b200_run_grm_product(kgl_b200_ctx* ctx, const uint8_t* keep, uint32_t n_cols, const double* x /* [n_genomes][n_cols] */,
+                             double* y /* [n_genomes][n_cols] */, uint64_t* n_loci_used);
+
 /* CalcFWS::updateGenomeFWSMap (kga_PfEMP/kga_analysis_PfEMP_FWS.cpp:15-101): for each of n_bins allele-frequency bins
  * [lower[b], upper[b]) of AF column `pop` (the P7FrequencyFilter pair AF >= lower and not AF >= upper,
  * kgl_variant_filter_Pf7.cpp:20-66; a locus without AF is in no bin) the AlleleSummmary of every genome over the bin's loci:

@@ -37,7 +37,7 @@ EXPORTS = [
     "kgl_b200_set_stream", "kgl_b200_synchronize", "kgl_b200_upload_genotypes", "kgl_b200_upload_loci",
     "kgl_b200_set_genome_superpop", "kgl_b200_upload_multi_allelic", "kgl_b200_run_multi_allele_count", "kgl_b200_set_unphased", "kgl_b200_select_loci", "kgl_b200_set_locus_selection",
     "kgl_b200_get_locus_selection", "kgl_b200_count_loci", "kgl_b200_set_locus_filter", "kgl_b200_synth_genotypes", "kgl_b200_download_genotypes", "kgl_b200_run_allele_count",
-    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
+    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
     "kgl_b200_run_binned_genome_counts", "kgl_b200_run_hetero_homo", "kgl_b200_location_fis", "kgl_b200_run_gram", "kgl_b200_run_grm", "kgl_b200_enqueue_gram", "kgl_b200_last_gram_kernel_ms", "kgl_b200_enqueue_gram_tiles", "kgl_b200_gram_buffer", "kgl_b200_fetch_gram",
     "kgl_b200_enqueue_ibs_tiles", "kgl_b200_ibs_tiles_buffer", "kgl_b200_ibs_timer_reset", "kgl_b200_ibs_timer_read",
     "kgl_b200_enqueue_count_and_inbreed", "kgl_b200_flush", "kgl_b200_launch_count", "kgl_b200_last_stream_kernel_ms",
@@ -50,6 +50,11 @@ EXPORTS = [
 class InbreedOptions(C.Structure):
     _fields_ = [("hall_start", C.POINTER(C.c_double)), ("hall_sweeps", C.c_int32), ("ll_tolerance", C.c_double),
                 ("ll_max_iterations", C.c_int32), ("count_loci", C.c_int32), ("exact_sweeps", C.c_int32), ("moments_on_cuda_cores", C.c_int32), ("sweep_by_sweep", C.c_int32)]
+
+
+class PcaOptions(C.Structure):
+    """kgl_b200_pca_options (include/kgl_b200.h), 24 bytes; zero = the defaults."""
+    _fields_ = [("keep", C.c_void_p), ("n_components", C.c_uint32), ("iterations", C.c_uint32), ("seed", C.c_uint64)]
 
 
 class KglError(RuntimeError):
@@ -318,6 +323,46 @@ class KglB200:
             self._check(rc, "run_king_pairs")
             break
         return out[: n.value].copy()
+
+    def _keep(self, keep):
+        if keep is None:
+            return None
+        k = np.ascontiguousarray(keep, dtype=np.uint8)
+        if k.shape != (self.n_loci,):
+            raise ValueError(f"keep must be uint8[{self.n_loci}]")
+        return k
+
+    def pca(self, k: int = 10, iterations: int = 10, seed: int = 0, keep=None, loadings: bool = False):
+        """Top-k principal components of the variance-standardised genotype matrix (PLINK 2 --pca approx; k = 0 and
+        iterations = 0 mean 10): a dict with eigenvalues float64[k] (descending), scores float64[N][k] (unit eigenvectors, largest
+        entry positive), n_loci_used and, with loadings=True, loadings float64[L][k]."""
+        k = int(k) or 10                                          # 0 = the default of the C ABI, which the buffers must match
+        if k < 0 or iterations < 0:
+            raise ValueError("k and iterations must be >= 0")
+        kp = self._keep(keep)
+        opt = PcaOptions(keep=None if kp is None else kp.ctypes.data, n_components=k, iterations=int(iterations), seed=int(seed))
+        ev = np.zeros(k, dtype=np.float64)
+        sc = np.zeros((self.n_genomes, k), dtype=np.float64)
+        ld = np.zeros((self.n_loci, k), dtype=np.float64) if loadings else None
+        m = C.c_uint64(0)
+        self._check(self.lib.kgl_b200_run_pca(self.h, C.byref(opt), _ptr(ev), _ptr(sc), _ptr(ld), C.byref(m)), "run_pca")
+        out = {"eigenvalues": ev, "scores": sc, "n_loci_used": int(m.value)}
+        if loadings:
+            out["loadings"] = ld
+        return out
+
+    def grm_product(self, x, keep=None):
+        """Z^T Z x (not divided by M) for x float64[N][n_cols], n_cols <= 48: (y float64[N][n_cols], n_loci_used)."""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        one = x.ndim == 1
+        x2 = x[:, None] if one else x
+        if x2.shape[0] != self.n_genomes:
+            raise ValueError(f"x must have {self.n_genomes} rows")
+        kp = self._keep(keep)
+        y = np.zeros_like(x2)
+        m = C.c_uint64(0)
+        self._check(self.lib.kgl_b200_run_grm_product(self.h, _ptr(kp), C.c_uint32(x2.shape[1]), _ptr(x2), _ptr(y), C.byref(m)), "run_grm_product")
+        return (y[:, 0] if one else y), int(m.value)
 
     def binned_genome_counts(self, lower, upper, pop: int = 0, present_only: bool = True):
         """(counts uint64[n_bins][N][4], rows uint64[n_bins]) -- CalcFWS' per-genome AlleleSummmary per AF bin."""

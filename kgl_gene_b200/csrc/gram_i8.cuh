@@ -45,11 +45,14 @@ __host__ __device__ inline uint64_t gram_code_index(uint64_t row, uint64_t word,
 
 struct GramParams {
   const uint32_t* codes;      // layout above
+  // B operand (the rows tile column tj selects); nullptr = codes. Its own rows in the same layout and k_stages: the Gram runs of
+  // pca.cuh contract a code matrix with a block of base-4 digit rows, a rectangular output written with ld as its row pitch
+  const uint32_t* codes_b;
   uint32_t k_stages;          // ceil(n_loci / 128)
   const uint2* tiles;         // (ti, tj): rows 128 ti .., columns 256 tj ..
   uint32_t n_tiles;
   uint32_t stages_per_chunk, n_chunks;
-  int32_t* out;               // [ld][ld]
+  int32_t* out;               // [ld][ld] (rectangular products: rows of A x ld, ld >= 256 x the largest tile column + 256)
   uint64_t ld;
   // value of a 2-bit code as an operand byte: byte c of the table is the value of code c (code 3 is stored as 0). 0x00020100 is the
   // dosage {0,1,2}; 0x00000100 / 0x00010000 are the indicators "heterozygous" / "homozygous alternate" (pairwise IBS, ibs_gram.cuh)
@@ -123,6 +126,7 @@ k_gram_i8(const GramParams P) {
     const uint32_t r = is_b ? t - kGramM : t;                    // row inside the A tile / the B tile
     const uint32_t sw = r & 7;                                   // swizzle phase of the row
     const uint32_t table = is_b ? P.table_b : P.table_a;
+    const uint32_t* codes = is_b && P.codes_b ? P.codes_b : P.codes;
     const uint32_t row_off = (is_b ? kGramABytes : 0u) + (r >> 3) * 1024 + sw * 128;
     uint32_t s = 0, ph = 0, it = 0;
     constexpr int D = 3;                                          // register prefetch depth in stages (L2/HBM latency ~ one stage time)
@@ -141,7 +145,7 @@ k_gram_i8(const GramParams P) {
       const uint2 tc = P.tiles[tile];
       const uint64_t ks = (uint64_t)chunk * P.stages_per_chunk + c.ks;
       const uint64_t block = (uint64_t)2 * (is_b ? tc.y : tc.x) + (r >> 7);
-      const uint4* src = reinterpret_cast<const uint4*>(P.codes + (block * P.k_stages + ks) * 1024 + (uint64_t)(r & 127) * 8);
+      const uint4* src = reinterpret_cast<const uint4*>(codes + (block * P.k_stages + ks) * 1024 + (uint64_t)(r & 127) * 8);
       dst[0] = __ldg(src); dst[1] = __ldg(src + 1);
     };
     Cursor cons{blockIdx.x, 0, 0}, pre;

@@ -16,6 +16,7 @@
 #include "gram_launch.cuh"
 #include "ibs_gram.cuh"
 #include "king.cuh"
+#include "pca.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -298,6 +299,16 @@ struct kgl_b200_ctx {
   DevBuf<unsigned long long> d_king_keys, d_king_keys2, d_king_cursor;
   DevBuf<uint32_t> d_king_index, d_king_index2;
   DevBuf<uint8_t> d_king_sort_temp;
+  // genotype PCA (pca.cuh): loci-major codes (code 3 kept), per-locus p / d / used, the product's blocks, digits and Gram outputs
+  DevBuf<uint32_t> d_codes_loci;
+  bool codes_loci_valid = false;
+  DevBuf<uint8_t> d_pca_keep, d_pca_used;
+  DevBuf<uint32_t> d_pca_counts;            // raw per-locus counts of PCA's own counting pass (d_locus_counts stays the caller's)
+  DevBuf<double> d_pca_p, d_pca_d, d_pca_x, d_pca_y, d_pca_wv, d_pca_out;
+  DevBuf<uint32_t> d_pca_digits;
+  DevBuf<int32_t> d_pca_acc;
+  DevBuf<unsigned long long> d_pca_stats;   // max bits and sums of X (2 x 48), of W | V (2 x 96), |U|
+  DevBuf<uint2> d_pca_tiles;
 
   // iterative estimator state
   int algo = -1, phase = 0, iteration = 0;
@@ -603,8 +614,10 @@ struct MaskOverride {
 // when simple_results); otherwise it leaves the raw per-genome counts d_gcounts {set lo bits, set hi bits} and d_n3.
 // defer_join: the tail stays on the tail stream and the context stream is NOT ordered after it (the resident pass: the next
 // pass's streaming kernel may start while this tail runs); the next entry point joins (use_device).
+// counts: where the per-locus counts go (null = d_locus_counts, the buffer kgl_b200_fetch_locus_counts reads).
 int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_genome, bool simple_results = false, bool want_moments = false,
-                 const MaskOverride* mo = nullptr, bool defer_join = false) {
+                 const MaskOverride* mo = nullptr, bool defer_join = false, DevBuf<uint32_t>* counts = nullptr) {
+  DevBuf<uint32_t>& lc = counts ? *counts : c->d_locus_counts;
   int rc = mo ? KGL_B200_OK : build_unit_tables(c);
   if (rc) return rc;
   rc = build_dropped_index(c);
@@ -612,8 +625,8 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
   const StreamPlan pl = plan_stream(c->units, c->L, c->sm_count);
   if (pl.padded_rows > c->padded_rows) return fail(c, KGL_B200_ERR_STATE, "internal: stream plan needs more padded rows than allocated");
   if (want_locus_counts) {
-    KGL_CUDA(c, c->d_locus_counts.ensure((size_t)c->L * 4));
-    if (pl.slices > 1) KGL_CUDA(c, cudaMemsetAsync(c->d_locus_counts.p, 0, (size_t)c->L * 16, c->stream));
+    KGL_CUDA(c, lc.ensure((size_t)c->L * 4));
+    if (pl.slices > 1) KGL_CUDA(c, cudaMemsetAsync(lc.p, 0, (size_t)c->L * 16, c->stream));
   }
   const bool indexed = c->dropped_indexed || c->n_dropped == 0;
   rc = ensure_side_streams(c); if (rc) return rc;
@@ -640,7 +653,7 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
   P.popmask32 = mo ? mo->popmask32 : reinterpret_cast<const uint32_t*>(c->d_popmask.p);     // little endian: u64 mask = {low half, high half}
   P.need32 = mo ? mo->need32 : c->d_need32.p;
   P.n_pop = (raw || mo) ? 1 : c->n_pop;
-  P.locus_counts = want_locus_counts ? c->d_locus_counts.p : nullptr;
+  P.locus_counts = want_locus_counts ? lc.p : nullptr;
   P.cta_counts = want_genome ? c->d_cta_counts[c->cbuf].p : nullptr;
   P.n_genomes_padded = (uint32_t)c->Npad;
   stream_make_tensor_map(P, pl, c->padded_rows);          // wide populations: one 2-D TMA box per stage
@@ -654,7 +667,7 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
   c->ev_valid = true;
   c->last_e0 = e0; c->last_e1 = e1;
   if (want_locus_counts && pl.slices > 1) {
-    k_fix_locus_n0<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(c->d_locus_counts.p, c->L, (uint32_t)c->N);
+    k_fix_locus_n0<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(lc.p, c->L, (uint32_t)c->N);
     KGL_LAUNCH_CHECK(c);
   }
   if (!want_genome) return KGL_B200_OK;
@@ -1463,6 +1476,157 @@ int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
   return KGL_B200_OK;
 }
 
+// Raw counting needs no super-populations: without them everyone counts as population 0.
+int default_superpop(kgl_b200_ctx* c) {
+  if (c->have_superpop) return KGL_B200_OK;
+  std::vector<uint8_t> zeros(c->N, 0);
+  int rc = kgl_b200_set_genome_superpop(c, c->N, zeros.data()); if (rc) return rc;
+  c->have_superpop = false;
+  return KGL_B200_OK;
+}
+
+// ---- genotype PCA (pca.cuh) ---------------------------------------------------------------------------------------------
+constexpr uint64_t kPcaSlabBytes = 1ull << 30;     // int32 outputs of one slab of pass-1 loci (both runs)
+// d_pca_stats: max bits and sums of the X block, of the W | V block, and |U|
+constexpr size_t kPcaStatX = 0, kPcaStatXSum = kPcaMaxCols, kPcaStatWV = 2 * kPcaMaxCols, kPcaStatWVSum = 4 * kPcaMaxCols,
+                 kPcaStatUsed = 6 * kPcaMaxCols, kPcaStats = 6 * kPcaMaxCols + 1;
+
+// Loci-major codes of the pass-1 runs (K = genomes), once per upload.
+int ensure_codes_loci(kgl_b200_ctx* c) {
+  if (c->codes_loci_valid) return KGL_B200_OK;
+  const uint64_t ks = (c->N + kGramK - 1) / kGramK, words = c->padded_rows * ks * 8;
+  KGL_CUDA(c, c->d_codes_loci.ensure(words));
+  k_codes16_loci<<<blocks_for(words, 256), 256, 0, c->stream>>>(reinterpret_cast<const uint32_t*>(c->d_packed.p), c->units, c->padded_rows, ks,
+                                                                c->d_codes_loci.p);
+  KGL_LAUNCH_CHECK(c);
+  c->codes_loci_valid = true;
+  return KGL_B200_OK;
+}
+
+// p_l, d_l and the used loci for the keep mask (NULL = every locus) from one raw counting pass; m = |U|.
+int pca_prepare(kgl_b200_ctx* c, const uint8_t* keep, uint64_t& m) {
+  if (c->L >= (1ull << 28)) return fail(c, KGL_B200_ERR_INVALID, "PCA: n_loci must be < 2^28 (int32 digit accumulators)");
+  int rc = default_superpop(c); if (rc) return rc;
+  rc = launch_count(c, true, true, false, false, false, nullptr, false, &c->d_pca_counts); if (rc) return rc;
+  if (keep) {
+    KGL_CUDA(c, c->d_pca_keep.ensure(c->L));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_keep.p, keep, c->L, cudaMemcpyHostToDevice, c->stream));
+  }
+  KGL_CUDA(c, c->d_pca_p.ensure(c->L));
+  KGL_CUDA(c, c->d_pca_d.ensure(c->L));
+  KGL_CUDA(c, c->d_pca_used.ensure(c->L));
+  KGL_CUDA(c, c->d_pca_stats.ensure(kPcaStats));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_pca_stats.p + kPcaStatUsed, 0, 8, c->stream));
+  k_pca_loci<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(c->d_pca_counts.p, keep ? c->d_pca_keep.p : nullptr, c->L, c->d_pca_p.p, c->d_pca_d.p,
+                                                           c->d_pca_used.p, c->d_pca_stats.p + kPcaStatUsed);
+  KGL_LAUNCH_CHECK(c);
+  unsigned long long used = 0;
+  KGL_CUDA(c, cudaMemcpyAsync(&used, c->d_pca_stats.p + kPcaStatUsed, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  m = used;
+  return KGL_B200_OK;
+}
+
+// Column maxima and digits of F [k_count][cols] into d_pca_digits (B operand of k_stages), sums next to the maxima.
+int pca_digits(kgl_b200_ctx* c, const double* F, uint64_t k_count, uint32_t cols, const uint8_t* used, uint64_t k_stages,
+               unsigned long long* max_bits, unsigned long long* sums) {
+  KGL_CUDA(c, cudaMemsetAsync(max_bits, 0, cols * 8, c->stream));
+  KGL_CUDA(c, cudaMemsetAsync(sums, 0, cols * 8, c->stream));
+  k_pca_colmax<<<dim3((unsigned)std::min<uint64_t>(blocks_for(k_count, 256), 64), cols), 256, 0, c->stream>>>(F, k_count, cols, max_bits);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, c->d_pca_digits.ensure((size_t)cols / kPcaColsPerBlock * kGramN * k_stages * 8));
+  const uint64_t threads = (uint64_t)cols * k_stages * 8;
+  k_pca_digits<<<(unsigned)std::min<uint64_t>(blocks_for(threads, 256), (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
+      F, k_count, cols, max_bits, used, k_stages, c->d_pca_digits.p, sums);
+  KGL_LAUNCH_CHECK(c);
+  return KGL_B200_OK;
+}
+
+// One digit Gram run: A rows of `codes` (tiles' rows) against the digit blocks, into out with row pitch ld.
+int pca_gram(kgl_b200_ctx* c, const uint32_t* codes, uint32_t table_a, uint64_t k_stages, const uint2* tiles, uint32_t n_tiles, const GramPlan& pl,
+             int32_t* out, uint64_t ld) {
+  GramParams G{};
+  G.codes = codes; G.codes_b = c->d_pca_digits.p; G.k_stages = (uint32_t)k_stages; G.tiles = tiles; G.n_tiles = n_tiles;
+  G.stages_per_chunk = pl.stages_per_chunk; G.n_chunks = pl.n_chunks; G.out = out; G.ld = ld;
+  G.table_a = table_a; G.table_b = kPcaTableDigit;
+  KGL_CUDA(c, launch_gram(G, pl, c->stream));
+  ++c->launches;
+  return KGL_B200_OK;
+}
+
+// y = Z^T Z x for x [N][n_in] (host, n_in <= 48) after pca_prepare. With loci_out: only pass 1, Y = Z x [L][n_in] to loci_out.
+int pca_apply(kgl_b200_ctx* c, uint32_t n_in, const double* x, double* y, double* loci_out) {
+  const uint32_t nb = (n_in + kPcaColsPerBlock - 1) / kPcaColsPerBlock, cols = nb * kPcaColsPerBlock;
+  const uint64_t N = c->N, L = c->L, ld1 = (uint64_t)cols / kPcaColsPerBlock * kGramN, ld2 = 2 * ld1, ldg = gram_ld(c);
+  const uint64_t ks1 = (N + kGramK - 1) / kGramK, ks2 = gram_k_stages(c);
+  const bool code3 = c->n_dropped > 0;
+  const int runs = code3 ? 2 : 1;
+  int rc = ensure_codes_loci(c); if (rc) return rc;
+  if (!loci_out) {
+    rc = ensure_codes<false>(c); if (rc) return rc;
+    if (code3) { rc = ensure_codes<true>(c); if (rc) return rc; }
+  }
+  // tile lists: a pass-1 slab (loci tiles x digit blocks), then pass 2 against the W blocks and against the V blocks
+  const uint64_t slab = std::min<uint64_t>(c->padded_rows, std::max<uint64_t>(kGramM, kPcaSlabBytes / (runs * ld1 * 4) / kGramM * kGramM));
+  std::vector<uint2> tiles;
+  for (uint32_t ti = 0; ti < slab / kGramM; ++ti)
+    for (uint32_t tj = 0; tj < nb; ++tj) tiles.push_back(make_uint2(ti, tj));
+  const size_t n1 = tiles.size();
+  for (uint32_t part = 0; part < 2; ++part)
+    for (uint32_t ti = 0; ti < ldg / kGramM; ++ti)
+      for (uint32_t tj = 0; tj < nb; ++tj) tiles.push_back(make_uint2(ti, part * nb + tj));
+  const uint32_t n2 = (uint32_t)(ldg / kGramM * nb);
+  std::vector<double> xp((size_t)N * cols, 0.0);
+  for (uint64_t g = 0; g < N; ++g) std::copy(x + g * n_in, x + (g + 1) * n_in, xp.begin() + g * cols);
+  KGL_CUDA(c, c->d_pca_tiles.ensure(tiles.size()));
+  KGL_CUDA(c, c->d_pca_x.ensure(xp.size()));
+  if (loci_out) KGL_CUDA(c, c->d_pca_y.ensure((size_t)L * cols));
+  else KGL_CUDA(c, c->d_pca_wv.ensure((size_t)L * 2 * cols));
+  KGL_CUDA(c, c->d_pca_acc.ensure(std::max<uint64_t>(runs * slab * ld1, ldg * ld2)));
+  KGL_CUDA(c, c->d_pca_out.ensure((size_t)N * cols));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_tiles.p, tiles.data(), tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_x.p, xp.data(), xp.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  unsigned long long* st = c->d_pca_stats.p;
+  int32_t* acc = c->d_pca_acc.p;
+
+  // pass 1: Y = Z X over slabs of loci; K = genomes
+  rc = pca_digits(c, c->d_pca_x.p, N, cols, nullptr, ks1, st + kPcaStatX, st + kPcaStatXSum); if (rc) return rc;
+  for (uint64_t r0 = 0; r0 < L; r0 += slab) {
+    const uint64_t rows = std::min<uint64_t>(slab, c->padded_rows - r0);
+    const uint32_t n_tiles = (uint32_t)(rows / kGramM * nb);
+    const GramPlan pl = plan_gram(n_tiles, (uint32_t)ks1, c->sm_count);
+    if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(acc, 0, (size_t)runs * slab * ld1 * 4, c->stream));
+    for (int run = 0; run < runs; ++run) {
+      rc = pca_gram(c, c->d_codes_loci.p + r0 / 128 * ks1 * 1024, run ? kGramTableCode3 : kPcaTableDosage, ks1, c->d_pca_tiles.p, n_tiles, pl,
+                    acc + (size_t)run * slab * ld1, ld1);
+      if (rc) return rc;
+    }
+    const uint64_t n = std::min<uint64_t>(rows, L - r0);
+    k_pca_recombine_loci<<<blocks_for(n * cols, 256), 256, 0, c->stream>>>(acc, code3 ? acc + slab * ld1 : nullptr, ld1, r0, n, cols, c->d_pca_p.p,
+                                                                           c->d_pca_d.p, c->d_pca_used.p, st + kPcaStatX, st + kPcaStatXSum,
+                                                                           loci_out ? c->d_pca_y.p : nullptr, c->d_pca_wv.p);
+    KGL_LAUNCH_CHECK(c);
+  }
+  if (loci_out) {
+    KGL_CUDA(c, cudaMemcpy2DAsync(loci_out, n_in * 8, c->d_pca_y.p, cols * 8, n_in * 8, L, cudaMemcpyDeviceToHost, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+    return KGL_B200_OK;
+  }
+
+  // pass 2: X' = Z^T Y from the digits of W | V; K = loci, the used ones count
+  rc = pca_digits(c, c->d_pca_wv.p, L, 2 * cols, c->d_pca_used.p, ks2, st + kPcaStatWV, st + kPcaStatWVSum); if (rc) return rc;
+  const GramPlan pl = plan_gram(n2, (uint32_t)ks2, c->sm_count);
+  if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(acc, 0, (size_t)ldg * ld2 * 4, c->stream));
+  rc = pca_gram(c, c->d_codes16.p, kPcaTableDosage, ks2, c->d_pca_tiles.p + n1, n2, pl, acc, ld2); if (rc) return rc;
+  if (code3) { rc = pca_gram(c, c->d_codes_raw.p, kGramTableCode3, ks2, c->d_pca_tiles.p + n1 + n2, n2, pl, acc, ld2); if (rc) return rc; }
+  k_pca_recombine_genomes<<<blocks_for(N * cols, 256), 256, 0, c->stream>>>(acc, ld2, N, cols, code3 ? 1 : 0, st + kPcaStatWV, st + kPcaStatWVSum,
+                                                                            c->d_pca_out.p);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, cudaMemcpy2DAsync(y, n_in * 8, c->d_pca_out.p, cols * 8, n_in * 8, N, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
 }  // namespace
 
 // The device buffers free themselves (DevBuf) after this body, the peer regions that map d_xchg must be gone by then.
@@ -1580,7 +1744,7 @@ static int set_shape(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_loci, uint6
   c->n_multi = 0;                    // the side cells belong to the matrix: kgl_b200_upload_multi_allelic comes after it
   c->units = stream_units_padded(c->host_units); c->Npad = c->units * 64;
   c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
-  c->codes16_valid = false; c->codes_raw_valid = false; c->gram_valid = false;
+  c->codes16_valid = false; c->codes_raw_valid = false; c->gram_valid = false; c->codes_loci_valid = false;
   return KGL_B200_OK;
 }
 
@@ -1924,11 +2088,7 @@ int kgl_b200_run_allele_count(kgl_b200_ctx* c, uint32_t* locus_counts, uint64_t*
   if (!c) return KGL_B200_ERR_INVALID;
   int rc = use_device(c); if (rc) return rc;
   rc = require_population(c, false); if (rc) return rc;
-  if (!c->have_superpop) {   // raw counting needs no super-populations: treat everyone as population 0
-    std::vector<uint8_t> zeros(c->N, 0);
-    rc = kgl_b200_set_genome_superpop(c, c->N, zeros.data()); if (rc) return rc;
-    c->have_superpop = false;
-  }
+  rc = default_superpop(c); if (rc) return rc;
   if (genome_counts) KGL_CUDA(c, c->d_genome_counts.ensure((size_t)c->N * 4));
   rc = launch_count(c, true, locus_counts != nullptr, genome_counts != nullptr); if (rc) return rc;
   if (locus_counts)
@@ -1946,11 +2106,7 @@ int kgl_b200_run_hetero_homo(kgl_b200_ctx* c, int other_allele_entries, uint64_t
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   int rc = use_device(c); if (rc) return rc;
   rc = require_population(c, false); if (rc) return rc;
-  if (!c->have_superpop) {   // raw counting needs no super-populations: treat everyone as population 0
-    std::vector<uint8_t> zeros(c->N, 0);
-    rc = kgl_b200_set_genome_superpop(c, c->N, zeros.data()); if (rc) return rc;
-    c->have_superpop = false;
-  }
+  rc = default_superpop(c); if (rc) return rc;
   rc = launch_count(c, true, false, true); if (rc) return rc;
   KGL_CUDA(c, c->d_genome_counts.ensure((size_t)c->N * 7));
   k_hetero_homo<<<blocks_for(c->N, 128), 128, 0, c->stream>>>(c->d_gcounts, c->d_n3, c->n_multi ? c->d_multi_cells.p : nullptr, c->n_multi, c->N,
@@ -2706,6 +2862,83 @@ int kgl_b200_run_binned_genome_counts(kgl_b200_ctx* c, uint32_t pop, uint32_t n_
   KGL_CUDA(c, cudaMemcpyAsync(genome_counts, c->d_bin_out.p, (size_t)n_bins * c->N * 32, cudaMemcpyDeviceToHost, c->stream));
   if (bin_rows) KGL_CUDA(c, cudaMemcpyAsync(bin_rows, c->d_bin_out.p + (size_t)n_bins * c->N * 4, (size_t)n_bins * 8, cudaMemcpyDeviceToHost, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_grm_product(kgl_b200_ctx* c, const uint8_t* keep, uint32_t n_cols, const double* x, double* y, uint64_t* n_loci_used) {
+  if (!c || !x || !y) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  if (n_cols == 0 || n_cols > (uint32_t)kPcaMaxCols) return fail(c, KGL_B200_ERR_INVALID, "n_cols must be 1..48");
+  uint64_t m = 0;
+  rc = pca_prepare(c, keep, m); if (rc) return rc;
+  if (m == 0) return fail(c, KGL_B200_ERR_INVALID, "no used locus (keep, and 0 < p < 1)");
+  rc = pca_apply(c, n_cols, x, y, nullptr); if (rc) return rc;
+  if (n_loci_used) *n_loci_used = m;
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_pca(kgl_b200_ctx* c, const kgl_b200_pca_options* options, double* eigenvalues, double* scores, double* loadings,
+                     uint64_t* n_loci_used) {
+  if (!c || !eigenvalues || !scores) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  const kgl_b200_pca_options opt = options ? *options : kgl_b200_pca_options{};
+  const uint32_t k = opt.n_components ? opt.n_components : 10, q = opt.iterations ? opt.iterations : 10;
+  const uint64_t N = c->N, L = c->L;
+  if (k > 40 || k >= N) return fail(c, KGL_B200_ERR_INVALID, "n_components must be 1..40 and below n_genomes");
+  uint64_t m = 0;
+  rc = pca_prepare(c, opt.keep, m); if (rc) return rc;
+  if (m == 0) return fail(c, KGL_B200_ERR_INVALID, "no used locus (keep, and 0 < p < 1)");
+  if (k > m) return fail(c, KGL_B200_ERR_INVALID, "n_components exceeds the used loci");
+  // block width 16 ceil((k + 6) / 16), at most the genomes
+  const uint32_t b = (uint32_t)std::min<uint64_t>(N, (k + 6 + 15) / 16 * 16);
+  std::vector<double> qb((size_t)N * b), aq((size_t)N * b);
+  for (uint64_t g = 0; g < N; ++g)
+    for (uint32_t j = 0; j < b; ++j) qb[g * b + j] = pca_start_entry(opt.seed, g, j);
+  pca_orth(qb, N, b);
+  for (uint32_t it = 0; it < q; ++it) {
+    rc = pca_apply(c, b, qb.data(), aq.data(), nullptr); if (rc) return rc;
+    qb.swap(aq);
+    pca_orth(qb, N, b);
+  }
+  // Rayleigh-Ritz: T = Q^T (Z^T Z Q), symmetrised
+  rc = pca_apply(c, b, qb.data(), aq.data(), nullptr); if (rc) return rc;
+  std::vector<double> t((size_t)b * b, 0.0), u;
+  for (uint64_t g = 0; g < N; ++g)
+    for (uint32_t i = 0; i < b; ++i)
+      for (uint32_t j = 0; j < b; ++j) t[(size_t)i * b + j] += qb[g * b + i] * aq[g * b + j];
+  for (uint32_t i = 0; i < b; ++i)
+    for (uint32_t j = i + 1; j < b; ++j) t[(size_t)i * b + j] = t[(size_t)j * b + i] = 0.5 * (t[(size_t)i * b + j] + t[(size_t)j * b + i]);
+  pca_jacobi(t, b, u);
+  std::vector<uint32_t> order(b);
+  for (uint32_t i = 0; i < b; ++i) order[i] = i;
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return t[(size_t)x * b + x] > t[(size_t)y * b + y]; });
+  std::vector<double> v((size_t)N * k, 0.0), theta(k);
+  for (uint32_t i = 0; i < k; ++i) {
+    const uint32_t o = order[i];
+    theta[i] = t[(size_t)o * b + o];
+    eigenvalues[i] = theta[i] / (double)m;
+    double best = -1.0;
+    uint64_t arg = 0;
+    for (uint64_t g = 0; g < N; ++g) {
+      double s = 0.0;
+      for (uint32_t j = 0; j < b; ++j) s += qb[g * b + j] * u[(size_t)j * b + o];
+      v[g * k + i] = s;
+      if (std::fabs(s) > best) { best = std::fabs(s); arg = g; }     // the lowest index wins a tie
+    }
+    if (v[arg * k + i] < 0.0)
+      for (uint64_t g = 0; g < N; ++g) v[g * k + i] = -v[g * k + i];
+  }
+  std::copy(v.begin(), v.end(), scores);
+  if (loadings) {                                    // u_i = Z v_i / sqrt(M lambda_i)
+    rc = pca_apply(c, k, v.data(), nullptr, loadings); if (rc) return rc;
+    for (uint32_t i = 0; i < k; ++i) {
+      const double s = theta[i] > 0.0 ? std::sqrt((double)m * eigenvalues[i]) : 0.0;
+      for (uint64_t l = 0; l < L; ++l) loadings[l * k + i] = s > 0.0 ? loadings[l * k + i] / s : 0.0;
+    }
+  }
+  if (n_loci_used) *n_loci_used = m;
   return KGL_B200_OK;
 }
 
