@@ -292,7 +292,9 @@ int kgl_b200_run_grm(kgl_b200_ctx* ctx, uint32_t pop, double* grm);
  * streaming kernel on the context stream, the preparation of a pass and the tail of the pass before it on two internal
  * streams, where they run next to the streaming kernel -- so consecutive calls overlap. Every other entry point orders the
  * context stream after the pending tail before it does anything; kgl_b200_flush does only that (no host synchronisation), e.g.
- * before an event is recorded on the context stream to time a sequence of passes. */
+ * before an event is recorded on the context stream to time a sequence of passes. The results of the last pass:
+ * kgl_b200_inbreed_fetch (its per-genome Simple results; the pass ends an estimator begun with kgl_b200_inbreed_begin) and
+ * kgl_b200_fetch_locus_counts. */
 int kgl_b200_enqueue_count_and_inbreed(kgl_b200_ctx* ctx);
 int kgl_b200_flush(kgl_b200_ctx* ctx);
 /* Number of kernels this context has launched so far. */
@@ -333,7 +335,8 @@ int kgl_b200_fetch_locus_counts(kgl_b200_ctx* ctx, uint32_t* locus_counts);
  * accumulate() fills the context's per-genome partial-sum buffer (device, doubles) for the current iterate;
  * the caller all-reduces (SUM) that buffer across ranks (partials_buffer() exposes it); update() consumes the reduced
  * partials and reports whether the iteration has finished; fetch() copies the LocusResults to the host.
- * On one GPU run_inbreed() is exactly begin + (accumulate + update)* + fetch. */
+ * On one GPU run_inbreed() is exactly begin + (accumulate + update)* + fetch. After kgl_b200_enqueue_count_and_inbreed[_peer]
+ * fetch() returns that pass's per-genome Simple results instead. */
 int kgl_b200_inbreed_begin(kgl_b200_ctx* ctx, int algorithm, const kgl_b200_inbreed_options* options);
 int kgl_b200_inbreed_accumulate(kgl_b200_ctx* ctx);
 int kgl_b200_inbreed_partials_buffer(kgl_b200_ctx* ctx, void** device_ptr, uint64_t* n_doubles);

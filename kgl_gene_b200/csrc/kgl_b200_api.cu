@@ -2165,6 +2165,7 @@ int kgl_b200_enqueue_count_and_inbreed(kgl_b200_ctx* c) {
     rc = join_tail(c); if (rc) return rc;
     rc = multi_add<MULTI_MOMENTS>(c, c->d_partials.p, c->d_results.p); if (rc) return rc;
   }
+  c->algo = KGL_B200_ALGO_SIMPLE; c->phase = 0;     // kgl_b200_inbreed_fetch copies d_results
   return KGL_B200_OK;
 }
 

@@ -173,6 +173,23 @@ size_t kgl_oracle_select_loci(const uint32_t* offsets, const float* af, size_t n
   return n_selected;
 }
 
+/* Per-genome sums over the loci (expected class frequencies, Ritland's locus sum). By default they are added locus by locus
+ * in double, the reference's order and precision, which the golden cases match bit for bit. Over millions of loci that
+ * sum drifts from the exact one by up to one rounding per locus, and terms that repeat (frequencies clipped to one value)
+ * make the roundings add up; kgl_oracle_set_compensated_sums(1) adds them with Neumaier's compensation instead, for
+ * comparisons with implementations whose sums are exact at that size (the device's fixed-point totals). */
+static int g_compensated = 0;
+void kgl_oracle_set_compensated_sums(int on) { g_compensated = on; }
+
+typedef struct { double s, c; } oracle_sum;
+static inline void sum_add(oracle_sum* a, double x) {
+  if (!g_compensated) { a->s += x; return; }
+  const double t = a->s + x;
+  a->c += fabs(a->s) >= fabs(x) ? (a->s - t) + x : (x - t) + a->s;
+  a->s = t;
+}
+static inline double sum_value(const oracle_sum* a) { return a->s + a->c; }
+
 /* One classified locus of one genome: the information AlleleFreqInfo carries for the estimators. */
 typedef struct { uint8_t cls; double first, second; } locus_term;
 enum { CLS_MAJOR_HOM = 0, CLS_MAJOR_HET = 1, CLS_MINOR_HET = 2, CLS_MINOR_HOM = 3 };
@@ -183,6 +200,7 @@ static size_t generate_frequencies(const uint8_t* packed, size_t row_bytes, size
                                    locus_term* terms, kgl_oracle_locus_results* r) {
   size_t n = 0;
   memset(r, 0, sizeof *r);
+  oracle_sum f_major_homo = {0, 0}, f_major_hetero = {0, 0}, f_minor_homo = {0, 0}, f_minor_hetero = {0, 0};
   for (size_t l = 0; l < n_loci; ++l) {
     if (!sel_pop[l]) continue;                               /* locus_list holds only the selected loci (:439) */
     const int m = multi_index(l);
@@ -215,7 +233,7 @@ static size_t generate_frequencies(const uint8_t* packed, size_t row_bytes, size
       terms[n++] = t;
       double cf[4];
       vector_class_freqs(&v, cf);
-      r->major_homo_freq += cf[0]; r->major_hetero_freq += cf[1]; r->minor_homo_freq += cf[2]; r->minor_hetero_freq += cf[3];
+      sum_add(&f_major_homo, cf[0]); sum_add(&f_major_hetero, cf[1]); sum_add(&f_minor_homo, cf[2]); sum_add(&f_minor_hetero, cf[3]);
       switch (t.cls) {
         case CLS_MINOR_HOM: ++r->minor_homo_count; break;
         case CLS_MAJOR_HET: ++r->major_hetero_count; break;
@@ -258,10 +276,10 @@ static size_t generate_frequencies(const uint8_t* packed, size_t row_bytes, size
     minor_homozygous = fmax(0.0, minor_homozygous);
     minor_heterozygous = fmax(0.0, minor_heterozygous);
     const double sum_freqs = major_homozygous + major_heterozygous + minor_homozygous + minor_heterozygous;
-    r->major_homo_freq += major_homozygous / sum_freqs;       /* :553-556 */
-    r->minor_homo_freq += minor_homozygous / sum_freqs;
-    r->major_hetero_freq += major_heterozygous / sum_freqs;
-    r->minor_hetero_freq += minor_heterozygous / sum_freqs;
+    sum_add(&f_major_homo, major_homozygous / sum_freqs);     /* :553-556 */
+    sum_add(&f_minor_homo, minor_homozygous / sum_freqs);
+    sum_add(&f_major_hetero, major_heterozygous / sum_freqs);
+    sum_add(&f_minor_hetero, minor_heterozygous / sum_freqs);
     switch (t.cls) {                                          /* :559-577 */
       case CLS_MINOR_HOM: ++r->minor_homo_count; break;
       case CLS_MAJOR_HET: ++r->major_hetero_count; break;
@@ -269,6 +287,8 @@ static size_t generate_frequencies(const uint8_t* packed, size_t row_bytes, size
       default: ++r->major_homo_count; break;
     }
   }
+  r->major_homo_freq = sum_value(&f_major_homo); r->major_hetero_freq = sum_value(&f_major_hetero);
+  r->minor_homo_freq = sum_value(&f_minor_homo); r->minor_hetero_freq = sum_value(&f_minor_hetero);
   r->total_allele_count = n;                                  /* :548 */
   return n;
 }
@@ -397,21 +417,21 @@ void kgl_oracle_inbreed_some(const uint8_t* packed, size_t row_bytes, size_t n_g
         case KGL_ORACLE_RITLAND: {                             /* processRitlandLocus (calc.cpp:375-431) */
           const double minimum_frequency = 0.001;
           size_t sum_allele = 0;
-          double locus_allele_sum = 0.0;
+          oracle_sum locus_allele_sum = {0, 0};
           for (size_t i = 0; i < n; ++i) {
             if (terms[i].cls == CLS_MAJOR_HOM || terms[i].cls == CLS_MINOR_HOM) {
               if (terms[i].first > minimum_frequency) {
                 const double ratio = (1.0 / terms[i].first);
-                locus_allele_sum += ratio;
-                locus_allele_sum -= 1.0;
+                sum_add(&locus_allele_sum, ratio);
+                sum_add(&locus_allele_sum, -1.0);
                 ++sum_allele;
               }
             } else {
-              locus_allele_sum -= 1.0;
+              sum_add(&locus_allele_sum, -1.0);
               ++sum_allele;
             }
           }
-          r.inbred_allele_sum = (sum_allele > 0 ? locus_allele_sum / (double)sum_allele : 0.0);
+          r.inbred_allele_sum = (sum_allele > 0 ? sum_value(&locus_allele_sum) / (double)sum_allele : 0.0);
         } break;
         case KGL_ORACLE_HALLME: {                              /* processHallME (calc.cpp:226-307); Q1: 50 sweeps */
           double f = start ? start[g] : 0.25;

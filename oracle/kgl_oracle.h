@@ -69,6 +69,10 @@ void kgl_oracle_inbreed_some(const uint8_t* packed, size_t row_bytes, size_t n_g
                              int unphased, int algorithm, const double* start, int sweeps,
                              const uint32_t* genomes, size_t n_some, kgl_oracle_locus_results* out);
 
+/* != 0: the per-genome sums of the calls above (expected class frequencies, Ritland's locus sum) are added with Neumaier's
+ * compensation instead of in the reference's order and precision. Set it around a call, not across threads. */
+void kgl_oracle_set_compensated_sums(int on);
+
 /* InbreedingCalculation::logLikelihood (kga_analysis_inbreed_calc.cpp:94-129) on a grid of f values. out[g][i]. */
 void kgl_oracle_loglik_grid(const uint8_t* packed, size_t row_bytes, size_t n_genomes, size_t n_loci,
                             const float* af, size_t n_pop, const uint8_t* selected, const uint8_t* superpop,

@@ -88,8 +88,10 @@ def select_all_pops(pop, lower=0, upper=10**9, spacing=0, count=10**9, min_af=0.
     return np.stack(out)
 
 
-def inbreed(pop, selected, algorithm: str, start=None, sweeps: int = 50, genomes=None) -> np.ndarray:
-    """genomes: optional list of genome indices -- the result then has one row per listed genome (start stays indexed by genome)."""
+def inbreed(pop, selected, algorithm: str, start=None, sweeps: int = 50, genomes=None, compensated: bool = False) -> np.ndarray:
+    """genomes: optional list of genome indices -- the result then has one row per listed genome (start stays indexed by genome).
+    compensated: the per-genome sums over the loci are added with Neumaier's compensation instead of in the reference's order
+    and precision (double, locus by locus), whose rounding grows with the number of loci."""
     set_multi(pop)
     gl = None if genomes is None else np.ascontiguousarray(genomes, dtype=np.uint32)
     n_some = pop.n_genomes if gl is None else gl.shape[0]
@@ -99,10 +101,14 @@ def inbreed(pop, selected, algorithm: str, start=None, sweeps: int = 50, genomes
     selected = np.ascontiguousarray(selected, dtype=np.uint8)
     sp = np.ascontiguousarray(pop.superpop, dtype=np.uint8)
     st = None if start is None else np.ascontiguousarray(start, dtype=np.float64)
-    lib().kgl_oracle_inbreed_some(_p(packed), C.c_size_t(pop.row_bytes), C.c_size_t(pop.n_genomes), C.c_size_t(pop.n_loci),
-                                  _p(af), C.c_size_t(af.shape[0]), _p(selected), _p(sp), C.c_int(int(pop.unphased)),
-                                  C.c_int(ALGORITHMS[algorithm]), None if st is None else _p(st), C.c_int(sweeps),
-                                  None if gl is None else _p(gl), C.c_size_t(n_some), _p(out))
+    lib().kgl_oracle_set_compensated_sums(C.c_int(int(compensated)))
+    try:
+        lib().kgl_oracle_inbreed_some(_p(packed), C.c_size_t(pop.row_bytes), C.c_size_t(pop.n_genomes), C.c_size_t(pop.n_loci),
+                                      _p(af), C.c_size_t(af.shape[0]), _p(selected), _p(sp), C.c_int(int(pop.unphased)),
+                                      C.c_int(ALGORITHMS[algorithm]), None if st is None else _p(st), C.c_int(sweeps),
+                                      None if gl is None else _p(gl), C.c_size_t(n_some), _p(out))
+    finally:
+        lib().kgl_oracle_set_compensated_sums(C.c_int(0))
     return out
 
 

@@ -134,7 +134,8 @@ def test_wide_population_100k_genomes():
 
 def test_c1_width_full_contig():
     """BASELINE config 1 shape: 500 genomes x 500,000 loci (one of the 14 contigs), unphased (Pf7, SURVEY Q6): the <8,256>
-    kernel over many counter flushes, all four estimators against the oracle."""
+    kernel, all four estimators against the oracle. At 148 SMs a CTA runs 14 stages, one counter chunk; the flushes between
+    chunks are tested in tests/test_gpu_stream_plans.py."""
     from kgl_gene_b200.capi import KglB200
     gpu = KglB200(0)
     try:

@@ -32,6 +32,43 @@ def test_closed_form_estimators_bit_exact(golden, algo):
     assert np.array_equal(mine[present], ref[algo + "_coeff"][present], equal_nan=True)      # NaN: a genome without any term
 
 
+def test_compensated_sums_agree_on_golden(golden):
+    """oracle_py.inbreed(compensated=True), what the device's fixed-point sums are compared with at millions of loci, agrees
+    with the reference's order to rounding on the golden cases."""
+    name, pop, ref, sel_kw = golden
+    sel = O.select_all_pops(pop, **sel_kw)
+    for algo in ("Simple", "RitlandLocus"):
+        a, b = O.inbreed(pop, sel, algo), O.inbreed(pop, sel, algo, compensated=True)
+        assert np.array_equal(results_matrix(a)[0], results_matrix(b)[0]), (name, algo)
+        assert np.allclose(results_matrix(b)[1], results_matrix(a)[1], rtol=1e-12, atol=0), (name, algo)
+        assert np.allclose(b["inbred_allele_sum"], a["inbred_allele_sum"], rtol=1e-10, atol=1e-12, equal_nan=True), (name, algo)
+
+
+def test_compensated_sums_are_exact():
+    """Where one term repeats over 2 M loci (64 genomes heterozygous everywhere, one frequency) the compensated sums are
+    exactly L times the term, while the reference's locus-by-locus double sum drifts (5e-11 relative; Simple's F, whose
+    denominator cancels, moves by 3e-7)."""
+    from fractions import Fraction
+    from kgl_gene_b200.flatfile import FlatPopulation
+
+    def repeated(n_loci):
+        packed = np.zeros((n_loci, 16), np.uint8)
+        packed[:, :8] = 0xFF                                                          # code 1 in every cell
+        return FlatPopulation((1000 + 10 * np.arange(n_loci)).astype(np.uint32), np.full((6, n_loci), np.float32(1e-4)),
+                              np.zeros(64, np.uint8), packed, 64, False)
+    one = repeated(1)
+    term = O.inbreed(one, O.select_all_pops(one), "Simple", compensated=True)[0]
+    n_loci = 2_000_000
+    many = repeated(n_loci)
+    sel = O.select_all_pops(many)
+    exact = O.inbreed(many, sel, "Simple", compensated=True)[0]
+    drift = O.inbreed(many, sel, "Simple")[0]
+    for f in ("major_homo_freq", "major_hetero_freq", "minor_homo_freq"):
+        want = float(Fraction(float(term[f])) * n_loci)
+        assert exact[f] == want, f
+        assert drift[f] != want, f
+
+
 def test_loglikelihood_grid_bit_exact(golden):
     name, pop, ref, sel_kw = golden
     sel = O.select_all_pops(pop, **sel_kw)
