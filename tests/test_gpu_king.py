@@ -68,7 +68,8 @@ def check_dense(gpu, pop, want, band):
                                       (300, 20000, 0.03),    # too many code-3 cells to index: in-kernel validity plane
                                       (64, 64, 0.5),         # exactly one tile, half the cells dropped
                                       (1, 40, 0.1),          # a single genome
-                                      (129, 33000, 0.002)])  # several word chunks per tile
+                                      (129, 33000, 0.002),   # several word chunks per tile
+                                      (600, 20000, 0.002)])  # 6 blocks x 157 stages: the HH and M Gram runs split in two chunks
 def test_king_modes_and_edges(gpu, n, l, miss):
     from kgl_gene_b200.synth import make_population
     pop, _ = make_population(n, l, seed=3 + n, missing_rate=miss)

@@ -46,7 +46,11 @@ def check_product(gpu, pop, cols, seed, keep=None):
                                            (63, 3333, 0.002, 17),     # few code-3 cells (indexed)
                                            (1000, 777, 0.03, 48),     # 3 % code-3 cells, still indexed: N L / 64 < 2^16
                                            (1000, 5001, 0.03, 48),    # more than 1.5 % code-3 cells and N L / 64 > 2^16: not indexed
-                                           (2, 130, 0.05, 1)])
+                                           (2, 130, 0.05, 1),
+                                           # 20,000 genomes: pass 1 (K = genomes, 157 stages) split in two chunks, red.add into
+                                           # the cleared slab; pass 2 237 units, two per CTA at 148 SMs (tests/test_gram_plan.py)
+                                           (20_000, 700, 0.0, 48),
+                                           (20_000, 700, 0.002, 48)])
 def test_product_bit_equal(gpu, n, l, miss, cols):
     pop, _ = make_population(n, l, seed=100 + n, missing_rate=miss)
     if l == 5001:      # the premise: more code-3 cells than the index takes (kgl_b200_upload_genotypes: max(2^16, N L / 64))
