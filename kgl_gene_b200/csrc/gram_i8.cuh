@@ -37,7 +37,7 @@ constexpr uint32_t kGramStageBytes = kGramABytes + kGramBBytes;  // 64 KB
 constexpr size_t kGramSmem = (size_t)kGramStages * kGramStageBytes + 1024 /* alignment slack */ + 256 /* barriers */;
 
 // Code matrix layout ("row-block major"): uint32 [ld / 128][k_stages][128 rows][8 words]; a word holds 16 loci, 2 bits each,
-// code 3 stored as 0, rows >= n_genomes and loci >= n_loci zero. One K-stage of one 128-row block is 4 KB contiguous, so the
+// code 3 kept (also at loci >= n_loci: the sample-major planes code them 3), rows >= n_genomes zero. One K-stage of one 128-row block is 4 KB contiguous, so the
 // expanders' loads are fully coalesced (16 B per lane, 512 B per warp).
 __host__ __device__ inline uint64_t gram_code_index(uint64_t row, uint64_t word, uint64_t k_stages) {
   return (((row >> 7) * k_stages + (word >> 3)) * 128 + (row & 127)) * 8 + (word & 7);
@@ -54,8 +54,8 @@ struct GramParams {
   uint32_t stages_per_chunk, n_chunks;
   int32_t* out;               // [ld][ld] (rectangular products: rows of A x ld, ld >= 256 x the largest tile column + 256)
   uint64_t ld;
-  // value of a 2-bit code as an operand byte: byte c of the table is the value of code c (code 3 is stored as 0). 0x00020100 is the
-  // dosage {0,1,2}; 0x00000100 / 0x00010000 are the indicators "heterozygous" / "homozygous alternate" (pairwise IBS, ibs_gram.cuh)
+  // value of a 2-bit code as an operand byte: byte c of the table is the value of code c. 0x00020100 is the dosage {0,1,2} with
+  // code 3 read as 0; 0x00000100 / 0x00010000 are the indicators "heterozygous" / "homozygous alternate" (pairwise IBS, ibs_gram.cuh)
   uint32_t table_a, table_b;
   // != 0: tile t of the list is written as its own 256 x 256 block at out + t * 65536 (row stride 256) instead of into the ld x ld
   // matrix -- populations whose N x N matrix would not fit (pairwise IBS, ibs_gram.cuh)
@@ -242,21 +242,15 @@ k_gram_i8(const GramParams P) {
   if (warp == 4) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(512) : "memory");
 }
 
-// Genome-major 2-bit codes from the sample-major planes: codes[g][w16] holds loci 16 w16 .. 16 w16 + 15 of genome g,
-// code 3 -> 0 (KEEP3: code 3 stays 3, for the code-3 indicator of the KING Gram run, king.cuh). One thread per
-// (genome, 32-locus word) -> two output words.
-template <bool KEEP3 = false>
+// Genome-major 2-bit codes from the sample-major planes: codes[g][w16] holds loci 16 w16 .. 16 w16 + 15 of genome g, code 3
+// kept. One thread per (genome, 32-locus word) -> two output words.
 __global__ void __launch_bounds__(256)
 k_codes16(const uint32_t* __restrict__ sm_lo, const uint32_t* __restrict__ sm_hi, uint64_t n_gblocks, uint64_t n_words,
           uint64_t k_stages, uint64_t n_rows, uint32_t* __restrict__ codes /* zeroed */) {
   const uint64_t idx = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;     // ((gb * n_words) + w) * 32 + lane
   if (idx >= n_gblocks * n_words * 32) return;
   const uint64_t lane = idx & 31, w = (idx >> 5) % n_words, gb = (idx >> 5) / n_words;
-  uint32_t lo = sm_lo[idx], hi = sm_hi[idx];
-  if (!KEEP3) {
-    const uint32_t both = lo & hi;
-    lo &= ~both; hi &= ~both;
-  }
+  const uint32_t lo = sm_lo[idx], hi = sm_hi[idx];
   uint32_t out[2];
 #pragma unroll
   for (int h = 0; h < 2; ++h) {

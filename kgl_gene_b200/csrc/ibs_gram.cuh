@@ -15,7 +15,7 @@
 
 namespace kgl {
 
-constexpr uint32_t kGramTableDosage = 0x03020100u, kGramTableHet = 0x00000100u, kGramTableHomAlt = 0x00010000u;
+constexpr uint32_t kGramTableDosage = 0x00020100u, kGramTableHet = 0x00000100u, kGramTableHomAlt = 0x00010000u;
 constexpr uint32_t kIbsTilesPerBlock = kGramM / kIbsT;            // 64-genome tiles per side of a 256 x 256 Gram block
 
 // counts[g] = {heterozygous cells, hom-alt cells} of genome g on the sample-major planes (code 3 in neither). Block = (genome

@@ -5,7 +5,7 @@
 // IBS0 / IBS1 / valid come from the IBS tile accumulators (ibs_compute_tiles, any form). The rest from two Gram matrices over the
 // 256 x 256 blocks under the tiles (ibs_gram.cuh):
 //     HH = H H^T                     het/het loci (code 3 is 0 in the het indicator, so exact in every missing-cell mode)
-//     M  = H C^T                     M[a][b] = loci where a is heterozygous and b is coded 3 (raw codes, C = code-3 indicator)
+//     M  = H C^T                     M[a][b] = loci where a is heterozygous and b is coded 3 (C = code-3 indicator)
 //     het_a = h_a - M[a][b],   het_b = IBS1 + 2 HH - het_a               (h_a = all heterozygous loci of a, k_ibs_class_counts)
 // Without code-3 cells M = 0 and het_a = h_a, het_b = h_b. For a tile below the diagonal the block list holds the mirror block,
 // where the stored value is M[b][a]: there it gives het_b and the identity gives het_a.
@@ -20,7 +20,7 @@ namespace kgl {
 static_assert(sizeof(kgl_b200_king_pair) == 40 && offsetof(kgl_b200_king_pair, het_b) == 28 && offsetof(kgl_b200_king_pair, kinship) == 32,
               "kgl_b200_king_pair: the 40-byte layout of include/kgl_b200.h");
 
-constexpr uint32_t kGramTableCode3 = 0x01000000u;   // operand byte of code c = byte c: 1 for code 3 (raw codes, k_codes16<true>)
+constexpr uint32_t kGramTableCode3 = 0x01000000u;   // operand byte of code c = byte c: 1 for code 3 (k_codes16 keeps code 3)
 
 struct KingTiles {
   const uint32_t* acc;          // [n_tiles][3][64*64] of ibs_compute_tiles

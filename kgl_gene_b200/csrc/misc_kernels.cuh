@@ -36,19 +36,6 @@ k_ritland_partials(const double* __restrict__ chunk_out, uint64_t n_chunks, uint
   P[PART_RCOUNT] = P[PART_NMAJHOM] + (P[PART_NMINHOM] - c2x) + n_het;
 }
 
-// Reduce the per-chunk outputs of an iterative pass into iter[g][slot0 .. slot0+n_take).
-__global__ void __launch_bounds__(256)
-k_iter_reduce(const double* __restrict__ chunk_out, uint64_t n_chunks, uint64_t n_genomes_padded, int n_out,
-              uint64_t n_genomes, int slot0, int n_take, double* __restrict__ iter) {
-  const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (g >= n_genomes) return;
-  for (int j = 0; j < n_take; ++j) {
-    double s = 0.0;
-    for (uint64_t c = 0; c < n_chunks; ++c) s += chunk_out[(c * n_genomes_padded + g) * n_out + j];
-    iter[g * ITER_COUNT + slot0 + j] = s;
-  }
-}
-
 __device__ __forceinline__ void fill_results(const double* P, kgl_b200_locus_results& r) {
   r.major_homo_count = (uint64_t)llrint(P[PART_NMAJHOM]);   r.major_homo_freq = P[PART_EMAJHOM];
   r.major_hetero_count = (uint64_t)llrint(P[PART_NMAJHET]); r.major_hetero_freq = P[PART_EMAJHET];
@@ -119,7 +106,7 @@ __device__ __forceinline__ void moment_partials_from(uint64_t g, double n_lo, do
 }
 
 // Fallback path (populations whose code-3 cells are not indexed): assembles the partials from the arrays the separate kernels
-// left (k_sum_cta_counts, k_dropped_scan, k_rare_rows).
+// left (k_sum_cta_counts, k_dropped_scan, k_locus_prepare).
 __global__ void __launch_bounds__(256)
 k_moment_partials(const uint32_t* __restrict__ gcounts /* [g]{set lo bits, set hi bits} over the selected rows */,
                   const uint32_t* __restrict__ n3s, const DenseTotals totals,

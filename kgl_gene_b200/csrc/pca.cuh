@@ -11,7 +11,7 @@
 //   int64: every int32 accumulator is <= 2 * 3 * K < 2^31 for K < 2^28.
 //   pass 1 (K = genomes): GX = G X, CX = C X on the loci-major codes (G dosage, C the code-3 indicator), S = sum_g X_q; then
 //     Y_l = d_l 2^-s (GX - 2 p_l (S - CX)),  W_l = d_l Y_l,  V_l = 2 p_l W_l   (0 outside U)
-//   pass 2 (K = loci, the positions that count are U): GW on the genome-major dosage codes, CV on the raw codes, T = sum_l V_q;
+//   pass 2 (K = loci, the positions that count are U): GW and CV on the genome-major codes, T = sum_l V_q;
 //     X'_g = 2^-t GW - 2^-t' (T - CV)
 // Every contraction is an exact integer; the double arithmetic after it is a fixed sequence of IEEE operations written with
 // explicit _rn intrinsics (no contraction into fused multiply-adds), so the result does not depend on the schedule and a host
@@ -27,7 +27,6 @@ namespace kgl {
 constexpr int kPcaDigits = 15, kPcaColsPerBlock = 16, kPcaIndicatorRow = 240;
 constexpr int kPcaMaxCols = 48;
 constexpr uint32_t kPcaTableDigit = 0x03020100u;     // a B digit (code 0..3) is its own value
-constexpr uint32_t kPcaTableDosage = 0x00020100u;    // dosage with code 3 read as 0 (the loci-major codes keep code 3)
 constexpr double kPcaQMax = 536870911.0;             // 2^29 - 1
 constexpr long long kPcaOffset = 1ll << 29;
 

@@ -31,7 +31,7 @@ struct TailParams {
   const uint8_t* superpop;
   int want_moments;                        // 1: partial sums (+ Simple closed form when results != null); 0: counts only
   int unphased;
-  const uint32_t* nz_rare; const unsigned long long* ecorr_rare_fx; double fx_inv;   // k_rare_rows (null with want_moments == 0)
+  const uint32_t* nz_rare; const unsigned long long* ecorr_rare_fx; double fx_inv;   // k_locus_prepare (null with want_moments == 0)
   DenseTotals totals; double* partials; kgl_b200_locus_results* results;
   uint32_t* gcounts; uint32_t* n3;         // counts-only consumers (raw / AF-bin passes): [g]{lo, hi}, [g]
 };
@@ -94,7 +94,7 @@ k_tail(const TailParams P) {
   sa = warp_sum(sa); sm = warp_sum(sm);
   if (lane == 0) { s_n[gi][wi] = n; s_sum[gi][wi][0] = sa; s_sum[gi][wi][1] = sm; }
 
-  // ---- everything below reads what the streaming kernel (and, on the preparation stream, k_rare_rows) wrote ----
+  // ---- everything below reads what the streaming kernel (and, on the preparation stream, k_locus_prepare) wrote ----
   asm volatile("griddepcontrol.wait;" ::: "memory");
   // per-genome counts: thread t adds the CTAs t, t + 256, ... for the block's four genomes and both planes (16-byte loads)
   uint32_t c8[GPB * 2];

@@ -89,17 +89,13 @@ k_to_sample_codes(const uint32_t* __restrict__ sm_lo, const uint32_t* __restrict
 
 // 1/d without the IEEE divide: x0 = MUFU.RCP64H, one Newton step x = x0 (1 + e), e = 1 - d x0. Measured on the B200
 // (tools/kbench, 2^26 arguments over [2^-40, 2^40]): max relative error of x0 9.9e-7 (2^-19.9), of x 9.9e-13; a second-order
-// step x0 (1 + e + e^2) reaches 2.2e-16 for one more DFMA per cell (KGL_FAST_RCP_EXACT). The estimators' contract is 1e-6
+// step x0 (1 + e + e^2) reaches 2.2e-16 for one more DFMA per cell. The estimators' contract is 1e-6
 // relative on F; a 1e-12 relative error in every term moves the HallME fixed point and the likelihood root by < 1e-12.
 __device__ __forceinline__ double fast_rcp(double d) {
   double x;
   asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x) : "d"(d));
   const double e = fma(-d, x, 1.0);
-#ifdef KGL_FAST_RCP_EXACT
-  return fma(x, fma(e, e, e), x);
-#else
   return fma(x, e, x);
-#endif
 }
 
 inline size_t fast_smem_bytes(int mode, uint32_t slots, int warps) {
