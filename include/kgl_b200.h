@@ -235,7 +235,7 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* ctx, uint64_t n_coords, const uint32_t
  * so that its entry of largest magnitude is positive (the lowest index wins a tie); loadings (nullable) double[n_loci][k],
  * u_i = Z v_i / sqrt(M lambda_i), 0 at unused loci; *n_loci_used = M (nullable). Needs a genotype upload
  * (KGL_B200_ERR_STATE before it); KGL_B200_ERR_INVALID for k outside 1..40, k >= n_genomes, k > M, no used locus or
- * n_loci >= 2^28. There is no popcount form: kgl_b200_set_ibs_tensor_cores does not apply. The device keeps a loci-major
+ * n_loci >= 2^28. LD pruning (kgl_b200_run_ld_prune below) gives a keep mask for it. There is no popcount form: kgl_b200_set_ibs_tensor_cores does not apply. The device keeps a loci-major
  * copy of the codes (n_genomes * n_loci / 4 bytes) from the first call after an upload. */
 typedef struct kgl_b200_pca_options {        /* zero-initialise for the defaults */
   const uint8_t* keep;                       /* uint8[n_loci], 0 = leave the locus out; NULL = every locus */
@@ -249,6 +249,49 @@ int kgl_b200_run_pca(kgl_b200_ctx* ctx, const kgl_b200_pca_options* options, dou
  * above). A locus-sharded caller sums it over ranks. Same errors as kgl_b200_run_pca (n_cols outside 1..48: INVALID). */
 int kgl_b200_run_grm_product(kgl_b200_ctx* ctx, const uint8_t* keep, uint32_t n_cols, const double* x /* [n_genomes][n_cols] */,
                              double* y /* [n_genomes][n_cols] */, uint64_t* n_loci_used);
+
+/* Linkage disequilibrium between loci: the genotypic r^2 of locus pairs inside a window, and LD pruning -- what PCA and KING are
+ * normally run on. No phasing is involved.
+ * Eligible loci: exactly PCA's used set U above (keep[l] != 0, keep NULL = every locus, and 0 < p < 1 from the raw counts;
+ * multi-allelic rows have p = 0 and are never eligible). rank(l) = index of l among the eligible loci.
+ * Window: eligible i < j (locus rows) form an in-window pair iff
+ *     (window_loci == 0 || rank(j) - rank(i) < window_loci)   -- the eligible loci are counted, as PLINK counts variants after filtering
+ * and (window_bp == 0 || offset[j] - offset[i] <= window_bp)  -- the offsets of kgl_b200_upload_loci (sorted; KGL_B200_ERR_STATE
+ *                                                                without them, KGL_B200_ERR_INVALID when they decrease)
+ * Both limits 0: KGL_B200_ERR_INVALID.
+ * r^2 is the squared Pearson correlation of the allele counts g in {0,1,2} over the genomes where neither cell is coded 3. With
+ * q = g^2, c = the code-3 indicator, per-locus totals s = n1 + 2 n2, q = n1 + 4 n2, c = n3 and, over genomes, GG = sum g_i g_j,
+ * CC = sum c_i c_j, GC_ij = sum g_i c_j, QC_ij = sum q_i c_j:
+ *     n = N - c_i - c_j + CC,  S_i = s_i - GC_ij,  S_j = s_j - GC_ji,  Q_i = q_i - QC_ij,  Q_j = q_j - QC_ji
+ *     cov = n GG - S_i S_j,  var_i = n Q_i - S_i^2,  var_j = n Q_j - S_j^2          (exact integers)
+ *     r^2 = (cov * cov) / (var_i * var_j)                                           (each int64 exactly a double; three IEEE ops)
+ * NaN when var_i or var_j is 0; a NaN never qualifies for the pair list and never prunes. The sums are exact int8 Gram runs on
+ * the tensor cores over 256 x 256 tiles of loci along the diagonal (ld.cuh), so results are bit-reproducible.
+ * Limits: n_genomes < 2^25 (every term < 4 N^2 < 2^53; else KGL_B200_ERR_INVALID), n_loci < 2^32. The device keeps PCA's
+ * loci-major copy of the codes (n_genomes * n_loci / 4 bytes) from the first call after an upload.
+ * Both entry points need a genotype upload (KGL_B200_ERR_STATE before it) and return KGL_B200_ERR_INVALID for a NaN threshold,
+ * both windows 0 or a null output pointer. */
+typedef struct kgl_b200_ld_options {         /* zero-initialise; 16 bytes */
+  const uint8_t* keep;                       /* uint8[n_loci], 0 = leave the locus out; NULL = every locus (PCA's meaning) */
+  uint32_t window_loci;                      /* 0 = no limit on the eligible-locus distance */
+  uint32_t window_bp;                        /* 0 = no limit on the offset distance */
+} kgl_b200_ld_options;
+typedef struct kgl_b200_ld_pair {            /* 24 bytes */
+  uint32_t a, b;                             /* locus rows, a < b */
+  uint32_t n_valid, reserved;                /* n above (genomes valid at both loci); reserved = 0 */
+  double r2;
+} kgl_b200_ld_pair;
+/* Every in-window pair with r^2 >= min_r2, in ascending (a, b) order. *n_pairs = the true total; if it exceeds capacity nothing is
+ * copied and the call returns KGL_B200_ERR_NOMEM: retry with capacity = *n_pairs (the retry computes everything again). */
+int kgl_b200_run_ld_pairs(kgl_b200_ctx* ctx, const kgl_b200_ld_options* options, double min_r2, uint64_t capacity,
+                          kgl_b200_ld_pair* pairs, uint64_t* n_pairs);
+/* Greedy LD pruning in locus order: eligible l is kept unless an EARLIER KEPT eligible locus i has (i, l) in the window and
+ * r^2(i, l) > max_r2. keep_out uint8[n_loci] = 0/1 (0 for every ineligible locus), *n_kept = its sum. It is meant to be
+ * passed straight to kgl_b200_pca_options.keep (run_pca then reports n_loci_used == n_kept), or used to drop loci before KING.
+ * This is not PLINK's --indep-pairwise window/step procedure: it is the rule defined by the locus order alone, with one answer
+ * whatever a step size would be. */
+int kgl_b200_run_ld_prune(kgl_b200_ctx* ctx, const kgl_b200_ld_options* options, double max_r2, uint8_t* keep_out /* [n_loci] */,
+                          uint64_t* n_kept);
 
 /* CalcFWS::updateGenomeFWSMap (kga_PfEMP/kga_analysis_PfEMP_FWS.cpp:15-101): for each of n_bins allele-frequency bins
  * [lower[b], upper[b]) of AF column `pop` (the P7FrequencyFilter pair AF >= lower and not AF >= upper,

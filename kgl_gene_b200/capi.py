@@ -37,7 +37,7 @@ EXPORTS = [
     "kgl_b200_set_stream", "kgl_b200_synchronize", "kgl_b200_upload_genotypes", "kgl_b200_upload_loci",
     "kgl_b200_set_genome_superpop", "kgl_b200_upload_multi_allelic", "kgl_b200_run_multi_allele_count", "kgl_b200_set_unphased", "kgl_b200_select_loci", "kgl_b200_set_locus_selection",
     "kgl_b200_get_locus_selection", "kgl_b200_count_loci", "kgl_b200_set_locus_filter", "kgl_b200_synth_genotypes", "kgl_b200_download_genotypes", "kgl_b200_run_allele_count",
-    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
+    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_run_ld_pairs", "kgl_b200_run_ld_prune", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
     "kgl_b200_run_binned_genome_counts", "kgl_b200_run_hetero_homo", "kgl_b200_location_fis", "kgl_b200_run_gram", "kgl_b200_run_grm", "kgl_b200_enqueue_gram", "kgl_b200_last_gram_kernel_ms", "kgl_b200_enqueue_gram_tiles", "kgl_b200_gram_buffer", "kgl_b200_fetch_gram",
     "kgl_b200_enqueue_ibs_tiles", "kgl_b200_ibs_tiles_buffer", "kgl_b200_ibs_timer_reset", "kgl_b200_ibs_timer_read",
     "kgl_b200_enqueue_count_and_inbreed", "kgl_b200_flush", "kgl_b200_launch_count", "kgl_b200_last_stream_kernel_ms",
@@ -55,6 +55,19 @@ class InbreedOptions(C.Structure):
 class PcaOptions(C.Structure):
     """kgl_b200_pca_options (include/kgl_b200.h), 24 bytes; zero = the defaults."""
     _fields_ = [("keep", C.c_void_p), ("n_components", C.c_uint32), ("iterations", C.c_uint32), ("seed", C.c_uint64)]
+
+
+class LdOptions(C.Structure):
+    """kgl_b200_ld_options (include/kgl_b200.h), 16 bytes; window limits of 0 mean no limit (not both)."""
+    _fields_ = [("keep", C.c_void_p), ("window_loci", C.c_uint32), ("window_bp", C.c_uint32)]
+
+
+class LdPair(C.Structure):
+    """kgl_b200_ld_pair (include/kgl_b200.h), 24 bytes."""
+    _fields_ = [("a", C.c_uint32), ("b", C.c_uint32), ("n_valid", C.c_uint32), ("reserved", C.c_uint32), ("r2", C.c_double)]
+
+
+LD_PAIR_DTYPE = np.dtype([(name, "<f8" if ctype is C.c_double else "<u4") for name, ctype in LdPair._fields_])
 
 
 class KglError(RuntimeError):
@@ -363,6 +376,35 @@ class KglB200:
         m = C.c_uint64(0)
         self._check(self.lib.kgl_b200_run_grm_product(self.h, _ptr(kp), C.c_uint32(x2.shape[1]), _ptr(x2), _ptr(y), C.byref(m)), "run_grm_product")
         return (y[:, 0] if one else y), int(m.value)
+
+    def _ld_options(self, window_loci, window_bp, keep):
+        kp = self._keep(keep)
+        return LdOptions(keep=None if kp is None else kp.ctypes.data, window_loci=int(window_loci), window_bp=int(window_bp)), kp
+
+    def ld_pairs(self, min_r2: float, window_loci: int = 0, window_bp: int = 0, keep=None, capacity: int = 1 << 22) -> np.ndarray:
+        """Every in-window pair of eligible loci (PCA's used set) with genotypic r^2 >= min_r2, sorted by (a, b): an LD_PAIR_DTYPE
+        array. The window counts eligible loci (window_loci) and / or offset distance (window_bp); 0 = no limit, not both. Retries
+        once with the exact capacity (a retry computes everything again)."""
+        opt, kp = self._ld_options(window_loci, window_bp, keep)
+        n = C.c_uint64(0)
+        for attempt in range(2):
+            out = np.zeros(max(int(capacity), 1), dtype=LD_PAIR_DTYPE)
+            rc = self.lib.kgl_b200_run_ld_pairs(self.h, C.byref(opt), C.c_double(min_r2), C.c_uint64(capacity), _ptr(out), C.byref(n))
+            if rc == KGL_B200_ERR_NOMEM and attempt == 0:
+                capacity = int(n.value)
+                continue
+            self._check(rc, "run_ld_pairs")
+            break
+        return out[: n.value].copy()
+
+    def ld_prune(self, max_r2: float, window_loci: int = 0, window_bp: int = 0, keep=None):
+        """Greedy LD pruning in locus order (an eligible locus is kept unless an earlier kept one in its window has r^2 > max_r2):
+        (keep uint8[L], n_kept). The mask is meant for pca(keep=...)."""
+        opt, kp = self._ld_options(window_loci, window_bp, keep)
+        out = np.zeros(self.n_loci, dtype=np.uint8)
+        n = C.c_uint64(0)
+        self._check(self.lib.kgl_b200_run_ld_prune(self.h, C.byref(opt), C.c_double(max_r2), _ptr(out), C.byref(n)), "run_ld_prune")
+        return out, int(n.value)
 
     def binned_genome_counts(self, lower, upper, pop: int = 0, present_only: bool = True):
         """(counts uint64[n_bins][N][4], rows uint64[n_bins]) -- CalcFWS' per-genome AlleleSummmary per AF bin."""

@@ -17,6 +17,7 @@
 #include "ibs_gram.cuh"
 #include "king.cuh"
 #include "pca.cuh"
+#include "ld.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -287,13 +288,14 @@ struct kgl_b200_ctx {
   bool codes16_valid = false;
   bool gram_valid = false;             // d_gram holds the last kgl_b200_enqueue_gram[_tiles] result (the IBS tensor form lends it out)
   cudaEvent_t gram_e0 = nullptr, gram_e1 = nullptr;
-  // KING-robust kinship (king.cuh): M = H C^T blocks, dense slab, pair list and its sort
+  // KING-robust kinship (king.cuh): M = H C^T blocks, dense slab, pair list
   DevBuf<int32_t> d_king_m;
   DevBuf<double> d_king_out;
   DevBuf<kgl_b200_king_pair> d_king_pairs, d_king_sorted;
-  DevBuf<unsigned long long> d_king_keys, d_king_keys2, d_king_cursor;
-  DevBuf<uint32_t> d_king_index, d_king_index2;
-  DevBuf<uint8_t> d_king_sort_temp;
+  // append cursor, sort keys and append positions of the KING and LD pair lists (sort_pair_keys)
+  DevBuf<unsigned long long> d_pair_keys, d_pair_keys2, d_pair_cursor;
+  DevBuf<uint32_t> d_pair_index, d_pair_index2;
+  DevBuf<uint8_t> d_pair_sort_temp;
   // genotype PCA (pca.cuh): loci-major codes (code 3 kept), per-locus p / d / used, the product's blocks, digits and Gram outputs
   DevBuf<uint32_t> d_codes_loci;
   bool codes_loci_valid = false;
@@ -304,6 +306,11 @@ struct kgl_b200_ctx {
   DevBuf<int32_t> d_pca_acc;
   DevBuf<unsigned long long> d_pca_stats;   // max bits and sums of X (2 x 48), of W | V (2 x 96), |U|
   DevBuf<uint2> d_pca_tiles;
+  // linkage disequilibrium (ld.cuh): eligible ranks, the band's tile lists, one slab's Gram blocks, the pair list
+  DevBuf<uint32_t> d_ld_rank, d_ld_mirror;
+  DevBuf<uint2> d_ld_tiles;
+  DevBuf<int32_t> d_ld_acc;
+  DevBuf<kgl_b200_ld_pair> d_ld_pairs, d_ld_sorted;
 
   // iterative estimator state
   int algo = -1, phase = 0, iteration = 0;
@@ -1257,19 +1264,26 @@ int ensure_codes(kgl_b200_ctx* c) {
   return KGL_B200_OK;
 }
 
-// One Gram run, table_a x table_b, over the 256 x 256 blocks under the current IBS tile list, into compact blocks: plan, clear
-// the output when the run is chunked (the chunks add into it), launch.
+// One k_gram_i8 run: A rows of `codes` (tile rows) against B rows of `codes_b` (nullptr = codes), each code read through its
+// byte table, K = k_stages x 128. ld == 0: every tile is written as its own compact 256 x 256 block, and a chunked run first
+// clears them (the chunks add into them); otherwise into `out` with row pitch ld, cleared by the caller when pl is chunked.
+int gram_run(kgl_b200_ctx* c, const uint32_t* codes, const uint32_t* codes_b, uint64_t k_stages, const uint2* tiles, uint32_t n_tiles,
+             const GramPlan& pl, uint32_t table_a, uint32_t table_b, int32_t* out, uint64_t ld) {
+  GramParams G{};
+  G.codes = codes; G.codes_b = codes_b; G.k_stages = (uint32_t)k_stages; G.tiles = tiles; G.n_tiles = n_tiles;
+  G.stages_per_chunk = pl.stages_per_chunk; G.n_chunks = pl.n_chunks; G.out = out; G.ld = ld; G.compact = ld == 0 ? 1 : 0;
+  G.table_a = table_a; G.table_b = table_b;
+  if (ld == 0 && pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(out, 0, (size_t)n_tiles * kGramM * kGramN * 4, c->stream));
+  KGL_CUDA(c, launch_gram(G, pl, c->stream));
+  ++c->launches;
+  return KGL_B200_OK;
+}
+
+// One Gram run, table_a x table_b, over the 256 x 256 blocks under the current IBS tile list (K = loci), into compact blocks.
 int run_gram_blocks(kgl_b200_ctx* c, const uint32_t* codes, uint32_t table_a, uint32_t table_b, int32_t* out) {
   const uint32_t k_stages = gram_k_stages(c);
   const GramPlan gp = plan_gram(std::max<uint32_t>(c->ibs_n_blocks, 1), k_stages, c->sm_count);
-  GramParams G{};
-  G.codes = codes; G.k_stages = k_stages; G.tiles = c->d_ibs_blocks.p; G.n_tiles = c->ibs_n_blocks;
-  G.stages_per_chunk = gp.stages_per_chunk; G.n_chunks = gp.n_chunks; G.out = out; G.ld = gram_ld(c); G.compact = 1;
-  G.table_a = table_a; G.table_b = table_b;
-  if (gp.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(out, 0, (size_t)c->ibs_n_blocks * kGramM * kGramN * 4, c->stream));
-  KGL_CUDA(c, launch_gram(G, gp, c->stream));
-  ++c->launches;
-  return KGL_B200_OK;
+  return gram_run(c, codes, nullptr, k_stages, c->d_ibs_blocks.p, c->ibs_n_blocks, gp, table_a, table_b, out, 0);
 }
 
 // The genomes' heterozygous / hom-alt cells on the IBS planes (code 3 in neither), once per upload.
@@ -1461,6 +1475,38 @@ int king_compute_tiles(kgl_b200_ctx* c, const TileList& list, KingTiles& K) {
   return KGL_B200_OK;
 }
 
+// The first n keys of a pair list (d_pair_keys, with their append positions in d_pair_index) sorted ascending over bits
+// [0, end_bit) into d_pair_keys2 / d_pair_index2: the order is then independent of the order in which the warps appended.
+int sort_pair_keys(kgl_b200_ctx* c, uint64_t n, int end_bit) {
+  KGL_CUDA(c, c->d_pair_keys2.ensure(n));
+  KGL_CUDA(c, c->d_pair_index2.ensure(n));
+  size_t temp_bytes = 0;
+  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, c->d_pair_keys.p, c->d_pair_keys2.p, c->d_pair_index.p, c->d_pair_index2.p,
+                                              n, 0, end_bit, c->stream));
+  KGL_CUDA(c, c->d_pair_sort_temp.ensure(temp_bytes));
+  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(c->d_pair_sort_temp.p, temp_bytes, c->d_pair_keys.p, c->d_pair_keys2.p, c->d_pair_index.p,
+                                              c->d_pair_index2.p, n, 0, end_bit, c->stream));
+  return KGL_B200_OK;
+}
+
+// The first n records of `pairs` in the order sort_pair_keys left, through `sorted` to the host.
+template <class Pair>
+int fetch_sorted_pairs(kgl_b200_ctx* c, const DevBuf<Pair>& pairs, DevBuf<Pair>& sorted, uint64_t n, Pair* out) {
+  KGL_CUDA(c, sorted.ensure(n));
+  k_gather_pairs<<<blocks_for(n, 256), 256, 0, c->stream>>>(pairs.p, c->d_pair_index2.p, n, sorted.p);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, cudaMemcpyAsync(out, sorted.p, n * sizeof(Pair), cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
+// Bits of the sort key (hi << 32) | lo with hi < n.
+int pair_key_bits(uint64_t n) {
+  int end_bit = 32;
+  for (uint64_t v = n - 1; v; v >>= 1) ++end_bit;
+  return end_bit;
+}
+
 int king_check(kgl_b200_ctx* c) {
   int rc = use_device(c); if (rc) return rc;
   rc = require_population(c, false); if (rc) return rc;
@@ -1530,9 +1576,9 @@ int ensure_codes_loci(kgl_b200_ctx* c) {
   return KGL_B200_OK;
 }
 
-// p_l, d_l and the used loci for the keep mask (NULL = every locus) from one raw counting pass; m = |U|.
+// p_l, d_l and the used loci for the keep mask (NULL = every locus) from one raw counting pass into d_pca_counts; m = |U|. PCA
+// and LD (whose eligible loci are PCA's used set).
 int pca_prepare(kgl_b200_ctx* c, const uint8_t* keep, uint64_t& m) {
-  if (c->L >= (1ull << 28)) return fail(c, KGL_B200_ERR_INVALID, "PCA: n_loci must be < 2^28 (int32 digit accumulators)");
   int rc = default_superpop(c); if (rc) return rc;
   rc = launch_count(c, true, true, false, false, false, nullptr, false, &c->d_pca_counts); if (rc) return rc;
   if (keep) {
@@ -1566,18 +1612,6 @@ int pca_digits(kgl_b200_ctx* c, const double* F, uint64_t k_count, uint32_t cols
   k_pca_digits<<<(unsigned)std::min<uint64_t>(blocks_for(threads, 256), (uint64_t)c->sm_count * 16), 256, 0, c->stream>>>(
       F, k_count, cols, max_bits, used, k_stages, c->d_pca_digits.p, sums);
   KGL_LAUNCH_CHECK(c);
-  return KGL_B200_OK;
-}
-
-// One digit Gram run: A rows of `codes` (tiles' rows) against the digit blocks, into out with row pitch ld.
-int pca_gram(kgl_b200_ctx* c, const uint32_t* codes, uint32_t table_a, uint64_t k_stages, const uint2* tiles, uint32_t n_tiles, const GramPlan& pl,
-             int32_t* out, uint64_t ld) {
-  GramParams G{};
-  G.codes = codes; G.codes_b = c->d_pca_digits.p; G.k_stages = (uint32_t)k_stages; G.tiles = tiles; G.n_tiles = n_tiles;
-  G.stages_per_chunk = pl.stages_per_chunk; G.n_chunks = pl.n_chunks; G.out = out; G.ld = ld;
-  G.table_a = table_a; G.table_b = kPcaTableDigit;
-  KGL_CUDA(c, launch_gram(G, pl, c->stream));
-  ++c->launches;
   return KGL_B200_OK;
 }
 
@@ -1621,8 +1655,8 @@ int pca_apply(kgl_b200_ctx* c, uint32_t n_in, const double* x, double* y, double
     const GramPlan pl = plan_gram(n_tiles, (uint32_t)ks1, c->sm_count);
     if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(acc, 0, (size_t)runs * slab * ld1 * 4, c->stream));
     for (int run = 0; run < runs; ++run) {
-      rc = pca_gram(c, c->d_codes_loci.p + r0 / 128 * ks1 * 1024, run ? kGramTableCode3 : kGramTableDosage, ks1, c->d_pca_tiles.p, n_tiles, pl,
-                    acc + (size_t)run * slab * ld1, ld1);
+      rc = gram_run(c, c->d_codes_loci.p + r0 / 128 * ks1 * 1024, c->d_pca_digits.p, ks1, c->d_pca_tiles.p, n_tiles, pl,
+                    run ? kGramTableCode3 : kGramTableDosage, kPcaTableDigit, acc + (size_t)run * slab * ld1, ld1);
       if (rc) return rc;
     }
     const uint64_t n = std::min<uint64_t>(rows, L - r0);
@@ -1641,13 +1675,112 @@ int pca_apply(kgl_b200_ctx* c, uint32_t n_in, const double* x, double* y, double
   rc = pca_digits(c, c->d_pca_wv.p, L, 2 * cols, c->d_pca_used.p, ks2, st + kPcaStatWV, st + kPcaStatWVSum); if (rc) return rc;
   const GramPlan pl = plan_gram(n2, (uint32_t)ks2, c->sm_count);
   if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(acc, 0, (size_t)ldg * ld2 * 4, c->stream));
-  rc = pca_gram(c, c->d_codes16.p, kGramTableDosage, ks2, c->d_pca_tiles.p + n1, n2, pl, acc, ld2); if (rc) return rc;
-  if (code3) { rc = pca_gram(c, c->d_codes16.p, kGramTableCode3, ks2, c->d_pca_tiles.p + n1 + n2, n2, pl, acc, ld2); if (rc) return rc; }
+  rc = gram_run(c, c->d_codes16.p, c->d_pca_digits.p, ks2, c->d_pca_tiles.p + n1, n2, pl, kGramTableDosage, kPcaTableDigit, acc, ld2);
+  if (rc) return rc;
+  if (code3) {
+    rc = gram_run(c, c->d_codes16.p, c->d_pca_digits.p, ks2, c->d_pca_tiles.p + n1 + n2, n2, pl, kGramTableCode3, kPcaTableDigit, acc, ld2);
+    if (rc) return rc;
+  }
   k_pca_recombine_genomes<<<blocks_for(N * cols, 256), 256, 0, c->stream>>>(acc, ld2, N, cols, code3 ? 1 : 0, st + kPcaStatWV, st + kPcaStatWVSum,
                                                                             c->d_pca_out.p);
   KGL_LAUNCH_CHECK(c);
   KGL_CUDA(c, cudaMemcpy2DAsync(y, n_in * 8, c->d_pca_out.p, cols * 8, n_in * 8, N, cudaMemcpyDeviceToHost, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
+// ---- linkage disequilibrium (ld.cuh) ------------------------------------------------------------------------------------
+constexpr uint64_t kLdSlabBytes = 1ull << 30;      // int32 Gram blocks of one slab of band tiles (every run)
+
+// What both LD entry points check and prepare: the eligible loci (PCA's used set, one raw counting pass), their ranks on the
+// host and the device, the band and its slabs, the loci-major codes, and the device tile list: per slab its band tiles, then the
+// mirror (J, I) of each off-diagonal one, with d_ld_mirror[t] = the mirror's position relative to the slab's first tile.
+struct LdPlan {
+  LdBand band;
+  std::vector<uint8_t> eligible;
+  std::vector<uint64_t> list_begin;      // per slab: its first entry of d_ld_tiles, with the list's length at the end
+  bool code3 = false;
+};
+
+int ld_prepare(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double threshold, LdPlan& P, LdTiles& T) {
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  const kgl_b200_ld_options opt = options ? *options : kgl_b200_ld_options{};
+  if (std::isnan(threshold)) return fail(c, KGL_B200_ERR_INVALID, "LD: the r^2 threshold is NaN");
+  if (opt.window_loci == 0 && opt.window_bp == 0) return fail(c, KGL_B200_ERR_INVALID, "LD: window_loci and window_bp are both 0");
+  if (c->N >= (1ull << 25)) return fail(c, KGL_B200_ERR_INVALID, "LD: n_genomes must be < 2^25 (exact int64 -> double terms)");
+  if (opt.window_bp != 0) {
+    if (!c->have_offsets || c->h_offsets.size() != c->L) return fail(c, KGL_B200_ERR_STATE, "LD: window_bp needs the locus offsets (kgl_b200_upload_loci)");
+    if (!std::is_sorted(c->h_offsets.begin(), c->h_offsets.end())) return fail(c, KGL_B200_ERR_INVALID, "LD: the locus offsets are not sorted");
+  }
+  const uint64_t L = c->L;
+  uint64_t m = 0;
+  rc = pca_prepare(c, opt.keep, m); if (rc) return rc;
+  P.eligible.resize(L);
+  KGL_CUDA(c, cudaMemcpyAsync(P.eligible.data(), c->d_pca_used.p, L, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  std::vector<uint32_t> rank(L);
+  uint32_t next = 0;
+  for (uint64_t l = 0; l < L; ++l) rank[l] = P.eligible[l] ? next++ : kLdNotEligible;
+  P.code3 = c->n_dropped > 0;
+  P.band = ld_band(rank.data(), c->h_offsets.data(), L, opt.window_loci, opt.window_bp, P.code3, kLdSlabBytes);
+  std::vector<uint2> list;
+  std::vector<uint32_t> mirror;
+  const size_t n_slabs = P.band.slab_begin.size() - 1;
+  for (size_t s = 0; s < n_slabs; ++s) {
+    P.list_begin.push_back(list.size());
+    const uint32_t t0 = P.band.slab_begin[s], t1 = P.band.slab_begin[s + 1];
+    list.insert(list.end(), P.band.tiles.begin() + t0, P.band.tiles.begin() + t1);
+    uint32_t pos = t1 - t0;
+    for (uint32_t t = t0; t < t1; ++t) {
+      const uint2 tc = P.band.tiles[t];
+      if (tc.x == tc.y) { mirror.push_back(t - t0); continue; }
+      mirror.push_back(pos++);
+      list.push_back(make_uint2(tc.y, tc.x));
+    }
+  }
+  P.list_begin.push_back(list.size());
+  rc = ensure_codes_loci(c); if (rc) return rc;
+  KGL_CUDA(c, c->d_ld_rank.ensure(L));
+  KGL_CUDA(c, c->d_ld_tiles.ensure(list.size()));
+  KGL_CUDA(c, c->d_ld_mirror.ensure(mirror.size()));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_rank.p, rank.data(), L * 4, cudaMemcpyHostToDevice, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_tiles.p, list.data(), list.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_mirror.p, mirror.data(), mirror.size() * 4, cudaMemcpyHostToDevice, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // pageable host memory
+  T = LdTiles{};
+  T.counts = c->d_pca_counts.p; T.rank = c->d_ld_rank.p; T.offsets = opt.window_bp ? c->d_offsets.p : nullptr;
+  T.n_loci = L; T.n_genomes = c->N; T.window_loci = opt.window_loci; T.window_bp = opt.window_bp;
+  return KGL_B200_OK;
+}
+
+// The Gram runs of slab s (K = genomes) into d_ld_acc: GG and CC over the nb band tiles, GC and QC over the nl tiles of the band
+// and its mirrors. Fills the slab's fields of T.
+int ld_slab_grams(kgl_b200_ctx* c, const LdPlan& P, size_t s, LdTiles& T) {
+  const uint32_t nb = P.band.slab_begin[s + 1] - P.band.slab_begin[s];
+  const uint32_t nl = (uint32_t)(P.list_begin[s + 1] - P.list_begin[s]);
+  const size_t blk = (size_t)kGramM * kGramN;
+  KGL_CUDA(c, c->d_ld_acc.ensure((P.code3 ? 2 * (size_t)nb + 2 * (size_t)nl : nb) * blk));
+  const uint2* tiles = c->d_ld_tiles.p + P.list_begin[s];
+  const uint64_t ks = (c->N + kGramK - 1) / kGramK;
+  const uint32_t* codes = c->d_codes_loci.p;
+  int32_t *gg = c->d_ld_acc.p, *cc = gg + nb * blk, *gc = cc + nb * blk, *qc = gc + nl * blk;
+  T.tiles = tiles; T.mirror = c->d_ld_mirror.p + P.band.slab_begin[s]; T.n_tiles = nb;
+  T.gg = gg; T.cc = T.gc = T.qc = nullptr;
+  const GramPlan pb = plan_gram(nb, (uint32_t)ks, c->sm_count);
+  int rc = gram_run(c, codes, nullptr, ks, tiles, nb, pb, kGramTableDosage, kGramTableDosage, gg, 0); if (rc) return rc;
+  if (!P.code3) return KGL_B200_OK;
+  T.cc = cc; T.gc = gc; T.qc = qc;
+  rc = gram_run(c, codes, nullptr, ks, tiles, nb, pb, kGramTableCode3, kGramTableCode3, cc, 0); if (rc) return rc;
+  const GramPlan pl = plan_gram(nl, (uint32_t)ks, c->sm_count);
+  rc = gram_run(c, codes, nullptr, ks, tiles, nl, pl, kGramTableDosage, kGramTableCode3, gc, 0); if (rc) return rc;
+  return gram_run(c, codes, nullptr, ks, tiles, nl, pl, kGramTableSquare, kGramTableCode3, qc, 0);
+}
+
+int ld_slab_pairs(kgl_b200_ctx* c, const LdTiles& T, double threshold, int prune, uint64_t capacity, kgl_b200_ld_pair* pairs) {
+  k_ld_pairs<<<blocks_for((uint64_t)T.n_tiles * kGramM * kGramN, 256), 256, 0, c->stream>>>(T, threshold, prune, capacity, pairs, c->d_pair_keys.p,
+                                                                                           c->d_pair_index.p, c->d_pair_cursor.p);
+  KGL_LAUNCH_CHECK(c);
   return KGL_B200_OK;
 }
 
@@ -2609,41 +2742,26 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
   // device list: no more records than the tiles hold, and indices that fit the uint32 sort values
   const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, n_tiles * kIbsTileCells), 0xFFFFFFFFull);
   KGL_CUDA(c, c->d_king_pairs.ensure(dev_cap));
-  KGL_CUDA(c, c->d_king_keys.ensure(dev_cap));
-  KGL_CUDA(c, c->d_king_index.ensure(dev_cap));
-  KGL_CUDA(c, c->d_king_cursor.ensure(1));
-  KGL_CUDA(c, cudaMemsetAsync(c->d_king_cursor.p, 0, 8, c->stream));
+  KGL_CUDA(c, c->d_pair_keys.ensure(dev_cap));
+  KGL_CUDA(c, c->d_pair_index.ensure(dev_cap));
+  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
   KingTiles K{};
   for (const TileList& tiles : slabs) {
     rc = king_compute_tiles(c, tiles, K); if (rc) return rc;
     k_king_pairs<<<blocks_for((uint64_t)K.n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(K, min_kinship, dev_cap, c->d_king_pairs.p,
-                                                                                               c->d_king_keys.p, c->d_king_index.p, c->d_king_cursor.p);
+                                                                                               c->d_pair_keys.p, c->d_pair_index.p, c->d_pair_cursor.p);
     KGL_LAUNCH_CHECK(c);
   }
   unsigned long long total = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_king_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   *n_pairs = total;
   if (total > capacity || total > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, "more related pairs than capacity (*n_pairs holds the total)");
   if (total == 0) return KGL_B200_OK;
   // ascending (a, b) whatever the order in which the warps appended
-  const uint64_t n = total;
-  int end_bit = 32;                                                // b in the low word, a < N above it
-  for (uint64_t v = c->N - 1; v; v >>= 1) ++end_bit;
-  KGL_CUDA(c, c->d_king_keys2.ensure(n));
-  KGL_CUDA(c, c->d_king_index2.ensure(n));
-  KGL_CUDA(c, c->d_king_sorted.ensure(n));
-  size_t temp_bytes = 0;
-  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(nullptr, temp_bytes, c->d_king_keys.p, c->d_king_keys2.p, c->d_king_index.p, c->d_king_index2.p,
-                                              n, 0, end_bit, c->stream));
-  KGL_CUDA(c, c->d_king_sort_temp.ensure(temp_bytes));
-  KGL_CUDA(c, cub::DeviceRadixSort::SortPairs(c->d_king_sort_temp.p, temp_bytes, c->d_king_keys.p, c->d_king_keys2.p, c->d_king_index.p,
-                                              c->d_king_index2.p, n, 0, end_bit, c->stream));
-  k_king_gather<<<blocks_for(n, 256), 256, 0, c->stream>>>(c->d_king_pairs.p, c->d_king_index2.p, n, c->d_king_sorted.p);
-  KGL_LAUNCH_CHECK(c);
-  KGL_CUDA(c, cudaMemcpyAsync(pairs, c->d_king_sorted.p, n * sizeof(kgl_b200_king_pair), cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  return KGL_B200_OK;
+  rc = sort_pair_keys(c, total, pair_key_bits(c->N)); if (rc) return rc;
+  return fetch_sorted_pairs(c, c->d_king_pairs, c->d_king_sorted, total, pairs);
 }
 
 int kgl_b200_set_ibs_tensor_cores(kgl_b200_ctx* c, int enable) {
@@ -2844,6 +2962,7 @@ int kgl_b200_run_grm_product(kgl_b200_ctx* c, const uint8_t* keep, uint32_t n_co
   int rc = use_device(c); if (rc) return rc;
   rc = require_population(c, false); if (rc) return rc;
   if (n_cols == 0 || n_cols > (uint32_t)kPcaMaxCols) return fail(c, KGL_B200_ERR_INVALID, "n_cols must be 1..48");
+  if (c->L >= (1ull << 28)) return fail(c, KGL_B200_ERR_INVALID, "PCA: n_loci must be < 2^28 (int32 digit accumulators)");
   uint64_t m = 0;
   rc = pca_prepare(c, keep, m); if (rc) return rc;
   if (m == 0) return fail(c, KGL_B200_ERR_INVALID, "no used locus (keep, and 0 < p < 1)");
@@ -2861,6 +2980,7 @@ int kgl_b200_run_pca(kgl_b200_ctx* c, const kgl_b200_pca_options* options, doubl
   const uint32_t k = opt.n_components ? opt.n_components : 10, q = opt.iterations ? opt.iterations : 10;
   const uint64_t N = c->N, L = c->L;
   if (k > 40 || k >= N) return fail(c, KGL_B200_ERR_INVALID, "n_components must be 1..40 and below n_genomes");
+  if (L >= (1ull << 28)) return fail(c, KGL_B200_ERR_INVALID, "PCA: n_loci must be < 2^28 (int32 digit accumulators)");
   uint64_t m = 0;
   rc = pca_prepare(c, opt.keep, m); if (rc) return rc;
   if (m == 0) return fail(c, KGL_B200_ERR_INVALID, "no used locus (keep, and 0 < p < 1)");
@@ -2913,6 +3033,91 @@ int kgl_b200_run_pca(kgl_b200_ctx* c, const kgl_b200_pca_options* options, doubl
     }
   }
   if (n_loci_used) *n_loci_used = m;
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_ld_pairs(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double min_r2, uint64_t capacity, kgl_b200_ld_pair* pairs,
+                          uint64_t* n_pairs) {
+  if (!c || !pairs || !n_pairs) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  LdPlan P;
+  LdTiles T{};
+  int rc = ld_prepare(c, options, min_r2, P, T); if (rc) return rc;
+  // device list: no more records than the band's cells, and indices that fit the uint32 sort values
+  const uint64_t cells = (uint64_t)P.band.tiles.size() * kGramM * kGramN;
+  const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, cells), 0xFFFFFFFFull);
+  KGL_CUDA(c, c->d_ld_pairs.ensure(dev_cap));
+  KGL_CUDA(c, c->d_pair_keys.ensure(dev_cap));
+  KGL_CUDA(c, c->d_pair_index.ensure(dev_cap));
+  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+  for (size_t s = 0; s + 1 < P.band.slab_begin.size(); ++s) {
+    rc = ld_slab_grams(c, P, s, T); if (rc) return rc;
+    rc = ld_slab_pairs(c, T, min_r2, 0, dev_cap, c->d_ld_pairs.p); if (rc) return rc;
+  }
+  unsigned long long total = 0;
+  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  *n_pairs = total;
+  if (total > capacity || total > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, "more LD pairs than capacity (*n_pairs holds the total)");
+  if (total == 0) return KGL_B200_OK;
+  rc = sort_pair_keys(c, total, pair_key_bits(c->L)); if (rc) return rc;
+  return fetch_sorted_pairs(c, c->d_ld_pairs, c->d_ld_sorted, total, pairs);
+}
+
+int kgl_b200_run_ld_prune(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double max_r2, uint8_t* keep_out, uint64_t* n_kept) {
+  if (!c || !keep_out || !n_kept) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  LdPlan P;
+  LdTiles T{};
+  int rc = ld_prepare(c, options, max_r2, P, T); if (rc) return rc;
+  const uint64_t L = c->L;
+  const int end_bit = pair_key_bits(L);
+  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
+  KGL_CUDA(c, c->d_pair_keys.ensure(1u << 20));
+  KGL_CUDA(c, c->d_pair_index.ensure(1u << 20));
+  // The greedy scan, slab by slab: pairs (i, l) with r^2 > max_r2 as keys (l << 32) | i, ascending. After slab s every pair whose
+  // l lies before the next slab's first block row is known (i <= l, and the tiles ascend), so those loci are final: walk them in
+  // order against the pending pairs. Loci [0, done) are final.
+  std::vector<unsigned long long> pending, slab, merged;
+  uint64_t done = 0;
+  auto finish = [&](uint64_t upto) {
+    size_t p = 0;
+    for (uint64_t l = done; l < upto; ++l) {
+      uint8_t kept = P.eligible[l];
+      for (; p < pending.size() && (pending[p] >> 32) == l; ++p)
+        if (keep_out[(uint32_t)pending[p]]) kept = 0;
+      keep_out[l] = kept;
+    }
+    pending.erase(pending.begin(), pending.begin() + p);
+    done = upto;
+  };
+  const size_t n_slabs = P.band.slab_begin.size() - 1;
+  for (size_t s = 0; s < n_slabs; ++s) {
+    rc = ld_slab_grams(c, P, s, T); if (rc) return rc;
+    unsigned long long n = 0;
+    for (int attempt = 0; attempt < 2; ++attempt) {      // a slab with more pairs than the key buffer runs again into a larger one
+      KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+      rc = ld_slab_pairs(c, T, max_r2, 1, c->d_pair_keys.cap, nullptr); if (rc) return rc;
+      KGL_CUDA(c, cudaMemcpyAsync(&n, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
+      KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+      if (n <= c->d_pair_keys.cap) break;
+      KGL_CUDA(c, c->d_pair_keys.ensure(n));
+      KGL_CUDA(c, c->d_pair_index.ensure(n));
+    }
+    slab.resize(n);
+    if (n > 0) {
+      rc = sort_pair_keys(c, n, end_bit); if (rc) return rc;
+      KGL_CUDA(c, cudaMemcpyAsync(slab.data(), c->d_pair_keys2.p, n * 8, cudaMemcpyDeviceToHost, c->stream));
+      KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
+    merged.resize(pending.size() + slab.size());
+    std::merge(pending.begin(), pending.end(), slab.begin(), slab.end(), merged.begin());
+    pending.swap(merged);
+    finish(s + 1 < n_slabs ? std::min<uint64_t>(L, (uint64_t)P.band.tiles[P.band.slab_begin[s + 1]].x * kGramM) : L);
+  }
+  finish(L);
+  uint64_t kept = 0;
+  for (uint64_t l = 0; l < L; ++l) kept += keep_out[l];
+  *n_kept = kept;
   return KGL_B200_OK;
 }
 

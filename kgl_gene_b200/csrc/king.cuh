@@ -114,10 +114,10 @@ k_king_pairs(const KingTiles K, double min_kinship, uint64_t capacity, kgl_b200_
   index[pos] = (uint32_t)pos;
 }
 
-// sorted[i] = pairs[order[i]]
+// sorted[i] = pairs[order[i]] (the KING and LD pair lists)
+template <class Pair>
 __global__ void __launch_bounds__(256)
-k_king_gather(const kgl_b200_king_pair* __restrict__ pairs, const uint32_t* __restrict__ order, uint64_t n,
-              kgl_b200_king_pair* __restrict__ sorted) {
+k_gather_pairs(const Pair* __restrict__ pairs, const uint32_t* __restrict__ order, uint64_t n, Pair* __restrict__ sorted) {
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) sorted[i] = pairs[order[i]];
 }
