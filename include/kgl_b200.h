@@ -293,6 +293,56 @@ int kgl_b200_run_ld_pairs(kgl_b200_ctx* ctx, const kgl_b200_ld_options* options,
 int kgl_b200_run_ld_prune(kgl_b200_ctx* ctx, const kgl_b200_ld_options* options, double max_r2, uint8_t* keep_out /* [n_loci] */,
                           uint64_t* n_kept);
 
+/* Population differentiation between groups of genomes (the super-populations, Pf7 locations, or any labelling).
+ * kgl_b200_run_group_counts: counts uint32[n_loci][n_groups][4], counts[l][k][c] = genomes of group k whose cell at locus l has
+ * code c, counted as kgl_b200_run_allele_count counts them (multi-allelic rows: their matrix codes 0 and 3), so the sum over the
+ * groups plus the genomes in no group is its locus_counts. group uint8[n_genomes]: 0 .. n_groups-1, or 0xFF = in no group;
+ * group == NULL: the labels of kgl_b200_set_genome_superpop with n_groups = KGL_B200_MAX_POP (the argument is ignored). One read of
+ * the resident matrix (fst.cuh). Errors: KGL_B200_ERR_STATE before a genotype upload, or for group == NULL without super-population
+ * labels; KGL_B200_ERR_INVALID for n_groups outside 1..64 or a label >= n_groups other than 0xFF. */
+int kgl_b200_run_group_counts(kgl_b200_ctx* ctx, uint32_t n_groups, const uint8_t* group /* [n_genomes] or NULL */,
+                              uint32_t* counts /* [n_loci][n_groups][4] */);
+/* F_ST between pairs of groups. Per group k at locus l, from its counts n0..n3 (code-3 cells are missing):
+ *     v_k = n0 + n1 + n2,   p_k = (n1 + 2 n2) / (2 v_k),   h_k = n1 / v_k
+ * Hudson (Hudson, Slatkin & Maddison 1992, as Bhatia et al. 2013 eq. 10; scikit-allel's hudson_fst), groups a, b:
+ *     num = (p_a - p_b)^2 - p_a (1 - p_a) / (2 v_a - 1) - p_b (1 - p_b) / (2 v_b - 1)
+ *     den = p_a (1 - p_b) + p_b (1 - p_a)
+ * Weir & Cockerham 1984 (r = 2 groups; the alt allele's a, b, c -- for two alleles each allele has the same ones):
+ *     n_bar = (v_a + v_b) / 2,   n_c = 2 v_a v_b / (v_a + v_b)            (= (r n_bar - sum v^2 / (r n_bar)) / (r - 1))
+ *     p_bar = (s_a + s_b) / (2 (v_a + v_b)) with s = n1 + 2 n2,   s2 = (v_a (p_a - p_bar)^2 + v_b (p_b - p_bar)^2) / n_bar
+ *     h_bar = (n1_a + n1_b) / (v_a + v_b),   pq = p_bar (1 - p_bar)
+ *     a = (n_bar / n_c) (s2 - (pq - s2 / 2 - h_bar / 4) / (n_bar - 1))
+ *     b = (n_bar / (n_bar - 1)) (pq - s2 / 2 - ((2 n_bar - 1) / (4 n_bar)) h_bar)
+ *     c = h_bar / 2,   num = a,   den = (a + b) + c
+ * Each formula is evaluated exactly as written, left to right, one IEEE round-to-nearest double operation at a time (no FMA), from
+ * the exact integer counts (v, s, 2 v - 1, v_a v_b, v_a + v_b, n1_a + n1_b are integers converted once), so results are
+ * reproducible bit for bit. A locus is used for a pair when keep[l] != 0 (keep NULL = every locus), v_a >= 1 and v_b >= 1
+ * (Hudson: then 2 v - 1 >= 1; Weir-Cockerham: n_c > 0) and, for Weir-Cockerham, n_bar > 1 (v_a + v_b >= 3), and den != 0 (a locus
+ * monomorphic across both groups contributes nothing). Genome-wide F_ST = sum num / sum den over the used loci, NaN when none is
+ * used. Summation order, independent of the GPU and of any launch plan: the loci in blocks of 256 (rows 256 x .. 256 x + 255; a
+ * locus that is not used, or past the last row, adds 0.0), each block summed as a halving tree (element i += element i + s for
+ * s = 128, 64, .., 1), then the block sums added in block order from 0.0.
+ * Windows (window_bp != 0; step_bp == 0 means step = window_bp): window w = 0 .. floor(max offset / step) covers the loci with
+ * offsets in [w step, w step + window_bp), the offsets of kgl_b200_upload_loci (sorted; KGL_B200_ERR_STATE without them,
+ * KGL_B200_ERR_INVALID when they decrease). Its sums add the used loci in row order from 0.0.
+ * Outputs: fst double[n_pairs]; per_locus (nullable) double[n_pairs][n_loci][2] = (num, den), (0, 0) where not used; windows
+ * (nullable) double[n_pairs][n_windows][3] = (sum num, sum den, loci used); *n_windows (nullable) = the number of windows (0 without), set only when the call succeeds.
+ * The pairs are `pairs` [n_pairs][2] with a < b < n_groups, or, for n_pairs == 0 or pairs == NULL, every pair a < b in order
+ * (0,1), (0,2), .., (1,2), ... The group counts stay on the device. Errors: those of kgl_b200_run_group_counts, and
+ * KGL_B200_ERR_INVALID for a method other than 0 / 1, a bad pair, no pair (one group) or a null fst. */
+#define KGL_B200_FST_HUDSON 0
+#define KGL_B200_FST_WEIR_COCKERHAM 1
+typedef struct kgl_b200_fst_options {       /* zero-initialise; 56 bytes */
+  const uint8_t* group;   uint32_t n_groups;  /* as kgl_b200_run_group_counts */
+  const uint8_t* keep;                        /* uint8[n_loci], NULL = every locus */
+  uint32_t method;                            /* KGL_B200_FST_HUDSON or KGL_B200_FST_WEIR_COCKERHAM */
+  uint32_t n_pairs;   const uint32_t* pairs;  /* [n_pairs][2] (a < b); 0 / NULL = every pair a < b */
+  uint64_t window_bp, step_bp;                /* 0 = no windows */
+} kgl_b200_fst_options;
+int kgl_b200_run_fst(kgl_b200_ctx* ctx, const kgl_b200_fst_options* options, double* fst /* [n_pairs] */,
+                     double* per_locus /* nullable, [n_pairs][n_loci][2] */, double* windows /* nullable, [n_pairs][n_windows][3] */,
+                     uint64_t* n_windows);
+
 /* CalcFWS::updateGenomeFWSMap (kga_PfEMP/kga_analysis_PfEMP_FWS.cpp:15-101): for each of n_bins allele-frequency bins
  * [lower[b], upper[b]) of AF column `pop` (the P7FrequencyFilter pair AF >= lower and not AF >= upper,
  * kgl_variant_filter_Pf7.cpp:20-66; a locus without AF is in no bin) the AlleleSummmary of every genome over the bin's loci:

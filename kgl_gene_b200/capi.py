@@ -37,7 +37,7 @@ EXPORTS = [
     "kgl_b200_set_stream", "kgl_b200_synchronize", "kgl_b200_upload_genotypes", "kgl_b200_upload_loci",
     "kgl_b200_set_genome_superpop", "kgl_b200_upload_multi_allelic", "kgl_b200_run_multi_allele_count", "kgl_b200_set_unphased", "kgl_b200_select_loci", "kgl_b200_set_locus_selection",
     "kgl_b200_get_locus_selection", "kgl_b200_count_loci", "kgl_b200_set_locus_filter", "kgl_b200_synth_genotypes", "kgl_b200_download_genotypes", "kgl_b200_run_allele_count",
-    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_run_ld_pairs", "kgl_b200_run_ld_prune", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
+    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_run_ld_pairs", "kgl_b200_run_ld_prune", "kgl_b200_run_group_counts", "kgl_b200_run_fst", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
     "kgl_b200_run_binned_genome_counts", "kgl_b200_run_hetero_homo", "kgl_b200_location_fis", "kgl_b200_run_gram", "kgl_b200_run_grm", "kgl_b200_enqueue_gram", "kgl_b200_last_gram_kernel_ms", "kgl_b200_enqueue_gram_tiles", "kgl_b200_gram_buffer", "kgl_b200_fetch_gram",
     "kgl_b200_enqueue_ibs_tiles", "kgl_b200_ibs_tiles_buffer", "kgl_b200_ibs_timer_reset", "kgl_b200_ibs_timer_read",
     "kgl_b200_enqueue_count_and_inbreed", "kgl_b200_flush", "kgl_b200_launch_count", "kgl_b200_last_stream_kernel_ms",
@@ -68,6 +68,15 @@ class LdPair(C.Structure):
 
 
 LD_PAIR_DTYPE = np.dtype([(name, "<f8" if ctype is C.c_double else "<u4") for name, ctype in LdPair._fields_])
+
+KGL_B200_MAX_POP = 6        # super-populations (include/kgl_b200.h); the groups of group_counts / fst with group=None
+FST_METHODS = {"hudson": 0, "weir_cockerham": 1}
+
+
+class FstOptions(C.Structure):
+    """kgl_b200_fst_options (include/kgl_b200.h), 56 bytes; zero = Hudson, the super-population labels, every locus and pair."""
+    _fields_ = [("group", C.c_void_p), ("n_groups", C.c_uint32), ("keep", C.c_void_p), ("method", C.c_uint32),
+                ("n_pairs", C.c_uint32), ("pairs", C.c_void_p), ("window_bp", C.c_uint64), ("step_bp", C.c_uint64)]
 
 
 class KglError(RuntimeError):
@@ -136,6 +145,7 @@ class KglB200:
             raise KglError(f"kgl_b200_create({device}) failed [{rc}]: {self.lib.kgl_b200_last_error(None).decode()}")
         self.h = h
         self.n_genomes = self.n_loci = 0
+        self._offsets = None
 
     def close(self):
         if getattr(self, "h", None):
@@ -179,6 +189,7 @@ class KglB200:
         self._check(self.lib.kgl_b200_upload_loci(self.h, C.c_uint64(af.shape[1]), C.c_uint32(af.shape[0]), _ptr(af), _ptr(off)),
                     "upload_loci")
         self.n_loci = int(af.shape[1])
+        self._offsets = off
 
     def set_genome_superpop(self, superpop: np.ndarray):
         sp = np.ascontiguousarray(superpop, dtype=np.uint8)
@@ -405,6 +416,59 @@ class KglB200:
         n = C.c_uint64(0)
         self._check(self.lib.kgl_b200_run_ld_prune(self.h, C.byref(opt), C.c_double(max_r2), _ptr(out), C.byref(n)), "run_ld_prune")
         return out, int(n.value)
+
+    def _groups(self, group, n_groups):
+        """(labels uint8[N] or None, G): None = the super-population labels, KGL_B200_MAX_POP groups."""
+        if group is None:
+            return None, KGL_B200_MAX_POP
+        g = np.ascontiguousarray(group, dtype=np.uint8)
+        if g.shape != (self.n_genomes,):
+            raise ValueError(f"group must be uint8[{self.n_genomes}]")
+        if n_groups is None:
+            valid = g[g != 0xFF]
+            n_groups = int(valid.max()) + 1 if valid.size else 1
+        return g, int(n_groups)
+
+    def group_counts(self, group=None, n_groups=None) -> np.ndarray:
+        """Per-group genotype counts uint32[L][G][4]: genomes of group k with code c at locus l (0xFF = in no group). group=None:
+        the super-population labels (G = 6); n_groups=None: the largest label + 1."""
+        g, G = self._groups(group, n_groups)
+        out = np.zeros((self.n_loci, G, 4), dtype=np.uint32)
+        self._check(self.lib.kgl_b200_run_group_counts(self.h, C.c_uint32(G), _ptr(g), _ptr(out)), "run_group_counts")
+        return out
+
+    def fst(self, group=None, n_groups=None, method: str = "hudson", pairs=None, keep=None, per_locus: bool = False,
+            window_bp: int = 0, step_bp: int = 0):
+        """F_ST between pairs of groups (Hudson or Weir & Cockerham, include/kgl_b200.h): a dict with pairs uint32[P][2], fst
+        float64[P] (genome-wide ratio of sums, NaN where no locus is used), with per_locus=True per_locus float64[P][L][2] =
+        (numerator, denominator), and with window_bp > 0 windows float64[P][W][3] = (sum num, sum den, loci used) and
+        window_start uint64[W] (step_bp = 0: step = window_bp). pairs=None: every pair a < b."""
+        g, G = self._groups(group, n_groups)
+        if pairs is None:
+            pr = np.array([(a, b) for a in range(G) for b in range(a + 1, G)], dtype=np.uint32).reshape(-1, 2)
+        else:
+            pr = np.ascontiguousarray(pairs, dtype=np.uint32).reshape(-1, 2)
+            if pr.shape[0] == 0:          # the C ABI reads n_pairs == 0 as "every pair", which the buffers below would not hold
+                raise ValueError("pairs is empty: pass pairs=None for every pair")
+        kp = self._keep(keep)
+        opt = FstOptions(group=None if g is None else g.ctypes.data, n_groups=G, keep=None if kp is None else kp.ctypes.data,
+                         method=FST_METHODS[method], n_pairs=0 if pairs is None else pr.shape[0],
+                         pairs=None if pairs is None else pr.ctypes.data, window_bp=int(window_bp), step_bp=int(step_bp))
+        out = np.full(pr.shape[0], np.nan, dtype=np.float64)
+        pl = np.zeros((pr.shape[0], self.n_loci, 2), dtype=np.float64) if per_locus else None
+        step = int(step_bp) or int(window_bp)
+        nw = int(self._offsets.max()) // step + 1 if window_bp and self._offsets is not None and self._offsets.size else 0
+        win = np.zeros((pr.shape[0], nw, 3), dtype=np.float64) if window_bp else None
+        n = C.c_uint64(0)
+        self._check(self.lib.kgl_b200_run_fst(self.h, C.byref(opt), _ptr(out), _ptr(pl), _ptr(win) if nw else None, C.byref(n)), "run_fst")
+        res = {"pairs": pr, "fst": out}
+        if per_locus:
+            res["per_locus"] = pl
+        if window_bp:
+            assert n.value == nw, (n.value, nw)
+            res["windows"] = win
+            res["window_start"] = np.arange(nw, dtype=np.uint64) * np.uint64(step)
+        return res
 
     def binned_genome_counts(self, lower, upper, pop: int = 0, present_only: bool = True):
         """(counts uint64[n_bins][N][4], rows uint64[n_bins]) -- CalcFWS' per-genome AlleleSummmary per AF bin."""

@@ -18,6 +18,7 @@
 #include "king.cuh"
 #include "pca.cuh"
 #include "ld.cuh"
+#include "fst.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -311,6 +312,17 @@ struct kgl_b200_ctx {
   DevBuf<uint2> d_ld_tiles;
   DevBuf<int32_t> d_ld_acc;
   DevBuf<kgl_b200_ld_pair> d_ld_pairs, d_ld_sorted;
+  // population differentiation (fst.cuh): the entry lists of the last labelling (gc_superpop: built from the super-population
+  // labels, reused until they or the matrix change), the per-group counts, and the F_ST pairs, keep mask, windows and block sums
+  DevBuf<uint2> d_gc_entries;
+  DevBuf<uint32_t> d_gc_chunk, d_gc_size;
+  bool gc_superpop = false;
+  DevBuf<uint4> d_group_counts;
+  DevBuf<uint2> d_fst_pairs, d_fst_range;
+  DevBuf<uint8_t> d_fst_keep;
+  DevBuf<double2> d_fst_terms, d_fst_blocks;
+  DevBuf<uint32_t> d_fst_used;
+  DevBuf<double> d_fst_out, d_fst_windows;
 
   // iterative estimator state
   int algo = -1, phase = 0, iteration = 0;
@@ -1784,6 +1796,48 @@ int ld_slab_pairs(kgl_b200_ctx* c, const LdTiles& T, double threshold, int prune
   return KGL_B200_OK;
 }
 
+// ---- population differentiation (fst.cuh) -------------------------------------------------------------------------------------
+// Per-group counts of every locus into d_group_counts ([L][G] uint4) for labels `group` (NULL = the super-population labels, G =
+// KGL_B200_MAX_POP); G receives the number of groups.
+int group_counts_device(kgl_b200_ctx* c, uint32_t n_groups, const uint8_t* group, uint32_t& G) {
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  if (!group) {
+    if (!c->have_superpop) return fail(c, KGL_B200_ERR_STATE, "group == NULL needs the super-population labels (kgl_b200_set_genome_superpop)");
+    n_groups = KGL_B200_MAX_POP;
+  } else {
+    if (n_groups == 0 || n_groups > kGcMaxGroups) return fail(c, KGL_B200_ERR_INVALID, "n_groups must be 1..64");
+    for (uint64_t g = 0; g < c->N; ++g)
+      if (group[g] >= n_groups && group[g] != 0xFF) return fail(c, KGL_B200_ERR_INVALID, "group label >= n_groups (0xFF = in no group)");
+  }
+  G = n_groups;
+  if (group || !c->gc_superpop) {
+    const GroupTable T = build_group_table(group ? group : c->h_superpop.data(), c->N, c->host_units, n_groups);
+    KGL_CUDA(c, c->d_gc_entries.ensure(T.entries.size()));
+    KGL_CUDA(c, c->d_gc_chunk.ensure(T.chunk_begin.size()));
+    KGL_CUDA(c, c->d_gc_size.ensure(T.size.size()));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_entries.p, T.entries.data(), T.entries.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_chunk.p, T.chunk_begin.data(), T.chunk_begin.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_size.p, T.size.data(), T.size.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // pageable host memory
+    c->gc_superpop = group == nullptr;
+  }
+  KGL_CUDA(c, c->d_group_counts.ensure((size_t)c->L * n_groups));
+  GroupCountParams P{};
+  P.packed = reinterpret_cast<const uint4*>(c->d_packed.p); P.pitch = c->units; P.n_loci = c->L;
+  P.n_tiles = (c->L + kGcRows - 1) / kGcRows; P.units = (uint32_t)c->host_units; P.n_groups = n_groups;
+  P.n_chunks = (uint32_t)((c->host_units + kGcChunkUnits - 1) / kGcChunkUnits);
+  P.entries = c->d_gc_entries.p; P.chunk_begin = c->d_gc_chunk.p; P.size = c->d_gc_size.p; P.counts = c->d_group_counts.p;
+  const size_t smem = group_counts_smem(n_groups);
+  KGL_CUDA(c, cudaFuncSetAttribute(k_group_counts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int per_sm = 0;
+  KGL_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_group_counts, kGcThreads, smem));
+  const uint64_t grid = std::min<uint64_t>(P.n_tiles, (uint64_t)c->sm_count * std::max(per_sm, 1));
+  k_group_counts<<<(unsigned)grid, kGcThreads, smem, c->stream>>>(P);
+  KGL_LAUNCH_CHECK(c);
+  return KGL_B200_OK;
+}
+
 }  // namespace
 
 // The device buffers free themselves (DevBuf) after this body, the peer regions that map d_xchg must be gone by then.
@@ -1902,7 +1956,7 @@ static int set_shape(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_loci, uint6
   c->n_multi = 0;                    // the side cells belong to the matrix: kgl_b200_upload_multi_allelic comes after it
   c->units = stream_units_padded(c->host_units); c->Npad = c->units * 64;
   c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
-  c->codes16_valid = false; c->gram_valid = false; c->codes_loci_valid = false;
+  c->codes16_valid = false; c->gram_valid = false; c->codes_loci_valid = false; c->gc_superpop = false;
   return KGL_B200_OK;
 }
 
@@ -1991,7 +2045,7 @@ int kgl_b200_set_genome_superpop(kgl_b200_ctx* c, uint64_t n_genomes, const uint
   KGL_CUDA(c, c->d_superpop.ensure(n_genomes));
   KGL_CUDA(c, cudaMemcpyAsync(c->d_superpop.p, superpop, n_genomes, cudaMemcpyHostToDevice, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  c->have_superpop = true; c->units_valid = false; c->dropped_cells_state = 0; c->prep_valid = false;
+  c->have_superpop = true; c->units_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->gc_superpop = false;
   if (!c->have_geno) c->N = n_genomes;
   return KGL_B200_OK;
 }
@@ -3118,6 +3172,83 @@ int kgl_b200_run_ld_prune(kgl_b200_ctx* c, const kgl_b200_ld_options* options, d
   uint64_t kept = 0;
   for (uint64_t l = 0; l < L; ++l) kept += keep_out[l];
   *n_kept = kept;
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_group_counts(kgl_b200_ctx* c, uint32_t n_groups, const uint8_t* group, uint32_t* counts) {
+  if (!c || !counts) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  uint32_t G = 0;
+  int rc = group_counts_device(c, n_groups, group, G); if (rc) return rc;
+  KGL_CUDA(c, cudaMemcpyAsync(counts, c->d_group_counts.p, (size_t)c->L * G * 16, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, double* fst, double* per_locus, double* windows,
+                     uint64_t* n_windows) {
+  if (!c || !options || !fst) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  const kgl_b200_fst_options& o = *options;
+  if (o.method > 1) return fail(c, KGL_B200_ERR_INVALID, "method must be 0 (Hudson) or 1 (Weir & Cockerham)");
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  const uint32_t G = o.group ? o.n_groups : KGL_B200_MAX_POP;
+  if (G == 0 || G > kGcMaxGroups) return fail(c, KGL_B200_ERR_INVALID, "n_groups must be 1..64");
+  std::vector<uint2> pairs;
+  if (o.n_pairs == 0 || !o.pairs) {
+    for (uint32_t a = 0; a < G; ++a)
+      for (uint32_t b = a + 1; b < G; ++b) pairs.push_back(make_uint2(a, b));
+  } else {
+    for (uint32_t i = 0; i < o.n_pairs; ++i) {
+      const uint32_t a = o.pairs[2 * i], b = o.pairs[2 * i + 1];
+      if (a >= b || b >= G) return fail(c, KGL_B200_ERR_INVALID, "a pair must be (a, b) with a < b < n_groups");
+      pairs.push_back(make_uint2(a, b));
+    }
+  }
+  if (pairs.empty()) return fail(c, KGL_B200_ERR_INVALID, "no pair of groups (n_groups is 1)");
+  const uint64_t L = c->L, np = pairs.size();
+  // windows w = 0 .. max offset / step over offsets [w step, w step + window): rows [lower_bound(w step), lower_bound(w step + window))
+  std::vector<uint2> range;
+  if (o.window_bp) {
+    if (!c->have_offsets || c->h_offsets.size() != L) return fail(c, KGL_B200_ERR_STATE, "F_ST windows need the locus offsets (kgl_b200_upload_loci)");
+    if (!std::is_sorted(c->h_offsets.begin(), c->h_offsets.end())) return fail(c, KGL_B200_ERR_INVALID, "F_ST windows: the locus offsets are not sorted");
+    const uint64_t step = o.step_bp ? o.step_bp : o.window_bp;
+    const uint64_t nw = (uint64_t)c->h_offsets.back() / step + 1;
+    for (uint64_t w = 0; w < nw; ++w) range.push_back(make_uint2((uint32_t)first_row_at(c, w * step), (uint32_t)first_row_at(c, w * step + o.window_bp)));
+  }
+  uint32_t G2 = 0;
+  rc = group_counts_device(c, G, o.group, G2); if (rc) return rc;
+  if (n_windows) *n_windows = range.size();            // only once the labels and the state have been accepted
+  const uint64_t n_blocks = (L + kFstBlock - 1) / kFstBlock;
+  KGL_CUDA(c, c->d_fst_pairs.ensure(np));
+  KGL_CUDA(c, c->d_fst_blocks.ensure(np * n_blocks));
+  KGL_CUDA(c, c->d_fst_used.ensure(np * n_blocks));
+  KGL_CUDA(c, c->d_fst_out.ensure(np));
+  KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_pairs.p, pairs.data(), np * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+  if (o.keep) {
+    KGL_CUDA(c, c->d_fst_keep.ensure(L));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_keep.p, o.keep, L, cudaMemcpyHostToDevice, c->stream));
+  }
+  if (per_locus) KGL_CUDA(c, c->d_fst_terms.ensure(np * L));
+  FstParams P{};
+  P.counts = c->d_group_counts.p; P.n_loci = L; P.n_blocks = n_blocks; P.n_groups = G; P.method = o.method; P.n_pairs = (uint32_t)np;
+  P.keep = o.keep ? c->d_fst_keep.p : nullptr; P.pairs = c->d_fst_pairs.p; P.terms = per_locus ? c->d_fst_terms.p : nullptr;
+  P.block_sums = c->d_fst_blocks.p; P.block_used = c->d_fst_used.p;
+  k_fst_blocks<<<dim3((unsigned)n_blocks, (unsigned)np), kFstBlock, 0, c->stream>>>(P);
+  KGL_LAUNCH_CHECK(c);
+  k_fst_total<<<blocks_for(np, 128), 128, 0, c->stream>>>(c->d_fst_blocks.p, c->d_fst_used.p, n_blocks, (uint32_t)np, c->d_fst_out.p);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, cudaMemcpyAsync(fst, c->d_fst_out.p, np * 8, cudaMemcpyDeviceToHost, c->stream));
+  if (per_locus) KGL_CUDA(c, cudaMemcpyAsync(per_locus, c->d_fst_terms.p, np * L * 16, cudaMemcpyDeviceToHost, c->stream));
+  if (!range.empty() && windows) {
+    const uint64_t nw = range.size();
+    KGL_CUDA(c, c->d_fst_range.ensure(nw));
+    KGL_CUDA(c, c->d_fst_windows.ensure(np * nw * 3));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_range.p, range.data(), nw * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+    k_fst_windows<<<blocks_for(np * nw, 128), 128, 0, c->stream>>>(P, c->d_fst_range.p, nw, c->d_fst_windows.p);
+    KGL_LAUNCH_CHECK(c);
+    KGL_CUDA(c, cudaMemcpyAsync(windows, c->d_fst_windows.p, np * nw * 24, cudaMemcpyDeviceToHost, c->stream));
+  }
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // also: the pageable pairs / keep / range copies have been read
   return KGL_B200_OK;
 }
 
