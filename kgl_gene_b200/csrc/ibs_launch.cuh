@@ -1,12 +1,30 @@
 // ibs_launch.cuh -- host-side plan and launch of k_ibs_tiles.
 #pragma once
+#include <algorithm>
+
 #include "ibs_tile.cuh"
 
 namespace kgl {
 
+constexpr uint64_t kIbsMaxTilesPerLaunch = 8192;     // 384 MB of accumulators
+
 struct IbsPlan {
   uint32_t words_per_chunk, n_chunks, grid;
 };
+
+// 32-locus words of a genome block row that k_ibs_tiles reads: rounded up to an even count (it takes two words per step; the
+// padding loci are coded 3).
+inline uint32_t ibs_words_used(uint64_t n_loci) { return (uint32_t)(((n_loci + 31) / 32 + 1) / 2 * 2); }
+
+// Segments (gridDim.y of k_ibs_missing_fix) every genome's dropped rows are cut into, so that the repair fills the GPU also
+// when few tiles are dealt to it (multi-GPU): about eight 128-thread CTAs per SM, no segment shorter than ~256 rows on average,
+// at most 64. With more than one segment the repair adds J atomically, into a plane the caller cleared.
+inline uint32_t ibs_repair_segments(uint64_t n_dropped, uint64_t n_genomes, uint32_t n_tiles, int sm_count) {
+  const uint64_t avg_rows = n_dropped / std::max<uint64_t>(1, n_genomes);
+  uint32_t segs = (uint32_t)std::max<uint64_t>(1, ((uint64_t)sm_count * 8 + n_tiles - 1) / n_tiles);
+  segs = (uint32_t)std::min<uint64_t>(segs, std::max<uint64_t>(1, avg_rows / 256));
+  return std::min<uint32_t>(segs, 64);
+}
 
 // Units = tiles x word chunks, dealt round-robin to one persistent CTA per SM. The chunk count is chosen so that every CTA
 // gets (nearly) the same number of units while a unit stays long enough (>= 256 words) to amortise its 48 adds per thread.

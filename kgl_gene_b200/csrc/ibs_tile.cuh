@@ -235,6 +235,7 @@ k_ibs_premask(const uint4* __restrict__ lo, const uint4* __restrict__ hi, uint64
 
 constexpr int kIbsFixLevels = 16;               // counter levels; 32,760 rows per genome between flushes
 constexpr int kIbsFixLow = 4;                   // levels 0..3 take 8 rows at a time; then level 3 (weight 8) moves into levels 4..15
+constexpr uint32_t kIbsFixRows = (1u << (kIbsFixLevels - 1)) - 8;    // rows a thread adds between two flushes of its counters
 
 // Sparse repair of the code-3 cells (dense-minus-sparse, DESIGN 4b). A thread owns one genome of one side of a tile and one
 // segment (blockIdx.y of gridDim.y) of that genome's dropped rows; it adds the partner unit's three 64-bit vectors (hom-alt,
@@ -265,7 +266,7 @@ k_ibs_missing_fix(const uint4* __restrict__ packed, uint32_t units, const unsign
     for (int q = 0; q < 3; ++q)
 #pragma unroll
       for (int lv = 0; lv < kIbsFixLevels; ++lv) cnt[q][lv] = 0;
-    const uint64_t k_stop = min(k_end, k + (uint64_t)((1u << (kIbsFixLevels - 1)) - 8));
+    const uint64_t k_stop = min(k_end, k + (uint64_t)kIbsFixRows);
     while (k < k_stop) {
       // eight rows at a time: the eight keys, then the eight partner units, are requested together (the walk is bound by the
       // latency of these two dependent loads, not by the counters)

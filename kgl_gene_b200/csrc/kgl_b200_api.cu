@@ -1222,8 +1222,6 @@ uint2 ibs_upper_tile(uint64_t t, uint64_t side) {
   return make_uint2((uint32_t)lo, (uint32_t)(lo + (t - start)));
 }
 
-constexpr uint64_t kIbsMaxTilesPerLaunch = 8192;     // 384 MB of accumulators
-
 // Tiles first, first + stride, ... (count of them) of the row-major upper triangle.
 TileList upper_tiles(uint64_t first, uint64_t stride, uint64_t count) { return {{TileKey::kUpper, first, stride, count}, {}}; }
 
@@ -1360,7 +1358,7 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
     KGL_CUDA(c, c->d_gram_hh.ensure(block_cells));
     KGL_CUDA(c, c->d_gram_aa.ensure(block_cells));
   }
-  const uint32_t words_used = (uint32_t)(((c->L + 31) / 32 + 1) / 2 * 2);
+  const uint32_t words_used = ibs_words_used(c->L);
   const IbsPlan pl = plan_ibs(n, words_used, c->sm_count);
   IbsParams P{};
   const bool premasked = c->ibs_mode == 2;
@@ -1391,12 +1389,7 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
   c->ibs_used_tensor = tensor;
   if (e1) KGL_CUDA(c, cudaEventRecord(e1, c->stream));
   if (c->ibs_mode == 2) {
-    // every genome's dropped rows are cut into segments so that the repair fills the GPU also when few tiles are dealt to it
-    // (multi-GPU): about eight 128-thread CTAs per SM, and no segment shorter than ~256 rows on average
-    const uint64_t avg_rows = c->n_dropped / std::max<uint64_t>(1, c->N);
-    uint32_t segs = (uint32_t)std::max<uint64_t>(1, ((uint64_t)c->sm_count * 8 + n - 1) / n);
-    segs = (uint32_t)std::min<uint64_t>(segs, std::max<uint64_t>(1, avg_rows / 256));
-    segs = std::min<uint32_t>(segs, 64);
+    const uint32_t segs = ibs_repair_segments(c->n_dropped, c->N, n, c->sm_count);
     if (segs > 1 && pl.n_chunks == 1)      // plane 2 (J) is accumulated atomically then: clear it (the whole buffer is cleared when chunked)
       KGL_CUDA(c, cudaMemset2DAsync(c->d_ibs_acc.p + 2 * kIbsTileCells, (size_t)3 * kIbsTileCells * 4, 0, (size_t)kIbsTileCells * 4, n, c->stream));
     k_ibs_missing_fix<<<dim3(n, segs), 128, 0, c->stream>>>(reinterpret_cast<const uint4*>(c->d_packed.p), (uint32_t)c->units, c->d_dropped.p,

@@ -378,21 +378,6 @@ def test_moment_tables_left_of_zero(gpu):
     assert np.max(np.abs(fast["inbred_allele_sum"] - want["inbred_allele_sum"])) < 1e-9
 
 
-@pytest.mark.parametrize("n,l,miss", [(130, 40_000, 0.012), (70, 2_400_000, 0.014)], ids=["segments", "counter-flush"])
-def test_ibs_sparse_repair_at_scale(gpu, n, l, miss):
-    """The sparse repair of code-3 cells (k_ibs_missing_fix) where it splits a genome's dropped rows into segments (few tiles,
-    many rows) and where one thread's rows exceed a counter flush (> 32,760 dropped rows per genome), against the naive
-    O(N^2 L) oracle loop."""
-    from kgl_gene_b200.flatfile import FlatPopulation
-    from kgl_gene_b200.synth import make_genomes, make_loci
-    offsets, af = make_loci(l, 91)
-    superpop, f = make_genomes(n, 91)
-    packed = O.synth_genotypes(91, n, l, af, superpop, f, missing_rate=miss)
-    pop = FlatPopulation(offsets, af, superpop, packed, n, False)
-    gpu.upload_population(pop)
-    assert np.array_equal(gpu.ibs(), O.ibs(pop))
-
-
 def test_ibs_matches_oracle(gpu):
     """Indexed code-3 cells: two-plane kernel on pre-masked planes + sparse repair (ibs_tile.cuh)."""
     from kgl_gene_b200.synth import make_population
