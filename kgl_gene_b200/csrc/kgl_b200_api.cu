@@ -6,7 +6,7 @@
 #include "stream_launch.cuh"
 #include "sparse_events.cuh"
 #include "sample_major.cuh"
-#include "terms_fast.cuh"
+#include "terms_launch.cuh"
 #include "terms_moments.cuh"
 #include "terms_moments_mma.cuh"
 #include "misc_kernels.cuh"
@@ -123,6 +123,7 @@ struct TileList {
 struct kgl_b200_ctx {
   int device = 0;
   int sm_count = 148;
+  size_t smem_optin = 227 * 1024;         // cudaDevAttrMaxSharedMemoryPerBlockOptin (232,448 B on the B200)
   uint64_t total_memory = 0;
   cudaStream_t own_stream = nullptr, stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -791,21 +792,6 @@ int multi_add(kgl_b200_ctx* c, double* target, kgl_b200_locus_results* results =
   return KGL_B200_OK;
 }
 
-struct TermLaunch { dim3 grid; uint32_t words_per_chunk; uint64_t n_chunks; };
-
-TermLaunch plan_terms(const kgl_b200_ctx* c) {
-  TermLaunch t;
-  const uint64_t gx = (c->n_gblocks + kTermWarps - 1) / kTermWarps;
-  // aim for ~4 waves of CTAs; chunks are multiples of the shared-memory tile
-  uint64_t want_chunks = std::max<uint64_t>(1, ((uint64_t)c->sm_count * 8 + gx - 1) / gx);
-  uint64_t wpc = (c->n_words + want_chunks - 1) / want_chunks;
-  wpc = std::max<uint64_t>(kTermTileWords, (wpc + kTermTileWords - 1) / kTermTileWords * kTermTileWords);
-  t.words_per_chunk = (uint32_t)wpc;
-  t.n_chunks = (c->n_words + wpc - 1) / wpc;
-  t.grid = dim3((unsigned)gx, (unsigned)t.n_chunks);
-  return t;
-}
-
 // What a k_genome_terms launch of either mode reads; its chunk outputs go to out ([tl.n_chunks][Npad][n_out]).
 TermParams term_params(const kgl_b200_ctx* c, const TermLaunch& tl, double* out, int n_out) {
   TermParams P{};
@@ -821,7 +807,7 @@ TermParams term_params(const kgl_b200_ctx* c, const TermLaunch& tl, double* out,
 int launch_grid_terms(kgl_b200_ctx* c, const double* d_grid, int n_grid, TermLaunch& tl) {
   int rc = ensure_sample_major(c);
   if (rc) return rc;
-  tl = plan_terms(c);
+  tl = plan_terms(c->n_gblocks, c->n_words, c->sm_count);
   KGL_CUDA(c, c->d_chunk_out.ensure((size_t)tl.n_chunks * c->Npad * kGridMax));
   TermParams P = term_params(c, tl, c->d_chunk_out.p, kGridMax);
   P.grid = d_grid; P.n_grid = n_grid;
@@ -843,7 +829,7 @@ int ensure_sample_codes(kgl_b200_ctx* c) {
   return KGL_B200_OK;
 }
 
-// Table-driven sweeps (terms_fast.cuh). One CTA per SM walks a contiguous range of 128-locus tiles over all genome blocks.
+// Table-driven sweeps (terms_fast.cuh), planned by plan_fast (terms_launch.cuh).
 struct FastLaunch { dim3 grid; uint32_t tiles_per_chunk, slots; uint64_t n_chunks; };
 
 template <int MODE>
@@ -851,31 +837,16 @@ int launch_fast(kgl_b200_ctx* c, FastLaunch& fl, uint64_t list_len = 0) {
   int rc = ensure_sample_major(c);
   if (rc) return rc;
   const uint64_t gblocks = list_len ? (list_len + 31) / 32 : std::min<uint64_t>(c->n_gblocks, (c->N + 31) / 32);
-  // warps per CTA: of 16..32 the count that leaves the fewest genome-block slots empty (more warps on a tie)
-  int warps = 16; double best = -1.0;
-  for (int w = 16; w <= kFastMaxWarps; ++w) {
-    const uint64_t sl = std::min<uint64_t>(8, (gblocks + w - 1) / w);
-    const uint64_t rows = (gblocks + (uint64_t)w * sl - 1) / ((uint64_t)w * sl);
-    const double filled = (double)gblocks / (double)(rows * sl * w);
-    if (filled >= best) { best = filled; warps = w; }
+  const FastPlan pl = plan_fast(MODE, gblocks, c->n_words, c->sel_row_lo, c->sel_row_hi, c->sm_count, c->smem_optin);
+  if (!pl.ok) {
+    char buf[160];
+    std::snprintf(buf, sizeof buf, "no estimator sweep plan for %llu genome blocks fits %zu bytes of shared memory per block",
+                  (unsigned long long)gblocks, c->smem_optin);
+    return fail(c, KGL_B200_ERR_CUDA, buf);
   }
-  // A handful of genome blocks (late Newton sweeps over the list of unfinished genomes, small populations) cannot fill 16
-  // warps: small CTAs instead, four of them per SM, each with a quarter of the tiles -- the sweep is then bound by the
-  // per-tile latency of a few warps, and four CTAs per SM overlap it.
-  int ctas_per_sm = 1;
-  if (gblocks <= 8) { warps = gblocks <= 4 ? 4 : 8; ctas_per_sm = 4; }
-  const uint32_t slots = (uint32_t)std::min<uint64_t>(8, (gblocks + warps - 1) / warps);
-  const uint64_t gy = (gblocks + (uint64_t)warps * slots - 1) / ((uint64_t)warps * slots);
-  // only the tiles of the selection window are swept (a contig is usually analysed in many short windows)
-  const uint64_t all_tiles = (c->n_words + kFastTileWords - 1) / kFastTileWords;
-  const uint64_t tile_begin = std::min<uint64_t>(all_tiles, c->sel_row_lo / kFastTile);
-  const uint64_t tile_end = std::max<uint64_t>(tile_begin, std::min<uint64_t>(all_tiles, c->sel_row_hi == ~0ull ? all_tiles : (c->sel_row_hi + kFastTile - 1) / kFastTile));
-  const uint64_t n_tiles = std::max<uint64_t>(1, tile_end - tile_begin);
-  const uint64_t want = std::max<uint64_t>(1, (uint64_t)c->sm_count * ctas_per_sm / gy);
-  const uint64_t tpc = std::max<uint64_t>(1, (n_tiles + want - 1) / want);
-  fl.tiles_per_chunk = (uint32_t)tpc; fl.slots = slots;
-  fl.n_chunks = (n_tiles + tpc - 1) / tpc;
-  fl.grid = dim3((unsigned)fl.n_chunks, (unsigned)gy);
+  fl.tiles_per_chunk = (uint32_t)pl.tiles_per_chunk; fl.slots = pl.slots;
+  fl.n_chunks = pl.n_chunks;
+  fl.grid = dim3((unsigned)fl.n_chunks, (unsigned)pl.gy);
   constexpr int NACC = FastAcc<MODE>::N;
   KGL_CUDA(c, c->d_chunk_out.ensure((size_t)fl.n_chunks * c->Npad * NACC));
   rc = ensure_sample_codes(c);
@@ -884,8 +855,8 @@ int launch_fast(kgl_b200_ctx* c, FastLaunch& fl, uint64_t list_len = 0) {
   P.codes = c->d_sm_codes.p;
   P.n_gblocks = gblocks; P.n_words = c->n_words; P.n_loci = c->L; P.n_genomes = c->N; P.n_genomes_padded = c->Npad;
   P.selw = c->prep[c->par].selw.p; P.af = c->d_af.p; P.superpop = c->d_superpop.p; P.n_pop = (int)c->n_pop;
-  P.unphased = c->unphased ? 1 : 0; P.tiles_per_chunk = fl.tiles_per_chunk; P.slots = slots;
-  P.tile_begin = tile_begin; P.tile_end = tile_end;
+  P.unphased = c->unphased ? 1 : 0; P.tiles_per_chunk = fl.tiles_per_chunk; P.slots = pl.slots;
+  P.tile_begin = pl.tile_begin; P.tile_end = pl.tile_end;
   P.f = c->d_f.p; P.out = c->d_chunk_out.p;
   P.list = list_len ? c->d_list.p : nullptr; P.n_list = list_len; P.n_list_dev = list_len ? c->d_list_count.p : nullptr;
   if (MODE == FAST_HALL || MODE == FAST_NEWTON) {
@@ -899,9 +870,8 @@ int launch_fast(kgl_b200_ctx* c, FastLaunch& fl, uint64_t list_len = 0) {
     }
     P.table = c->d_terms_table.p;
   }
-  const size_t smem = fast_smem_bytes(MODE, slots, warps);
-  KGL_CUDA(c, cudaFuncSetAttribute(k_terms_fast<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  k_terms_fast<MODE><<<fl.grid, warps * 32, smem, c->stream>>>(P);
+  KGL_CUDA(c, cudaFuncSetAttribute(k_terms_fast<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
+  k_terms_fast<MODE><<<fl.grid, pl.warps * 32, pl.smem, c->stream>>>(P);
   KGL_LAUNCH_CHECK(c);
   return KGL_B200_OK;
 }
@@ -910,7 +880,7 @@ int launch_fast(kgl_b200_ctx* c, FastLaunch& fl, uint64_t list_len = 0) {
 // return at once).
 int newton_exact_tail(kgl_b200_ctx* c) {
   const unsigned nb = blocks_for(c->N, 256);
-  TermLaunch tl = plan_terms(c);
+  TermLaunch tl = plan_terms(c->n_gblocks, c->n_words, c->sm_count);
   KGL_CUDA(c, c->d_slow_out.ensure((size_t)tl.n_chunks * c->Npad * 4));
   TermParams P = term_params(c, tl, c->d_slow_out.p, 4);
   P.lane_state = c->d_lane_state.p; P.n_slow = c->d_n_slow.p;
@@ -1878,6 +1848,7 @@ int kgl_b200_create(int device, kgl_b200_ctx** out) {
   auto* c = new kgl_b200_ctx();
   c->device = device;
   c->sm_count = prop.multiProcessorCount;
+  c->smem_optin = prop.sharedMemPerBlockOptin;
   c->total_memory = prop.totalGlobalMem;
   // the context stream carries the streaming kernel: highest priority, so that its CTAs are placed before the blocks of the
   // side streams (preparation, tail) when both are ready

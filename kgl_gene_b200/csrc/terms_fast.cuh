@@ -98,10 +98,6 @@ __device__ __forceinline__ double fast_rcp(double d) {
   return fma(x, e, x);
 }
 
-inline size_t fast_smem_bytes(int mode, uint32_t slots, int warps) {
-  return (size_t)kMaxPop * fast_stride(mode) * 8 + (size_t)slots * warps * 32 * fast_n_acc(mode) * 8 + kMaxPop * kFastTileWords * 2 * 4;
-}
-
 // Shared-memory address of cell j (0..15) of a code half z: base | (code * 8 E), the locus offset goes into the load's
 // immediate. One shift and one LOP3 per cell.
 template <int E, int J>
