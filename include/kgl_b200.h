@@ -343,6 +343,60 @@ int kgl_b200_run_fst(kgl_b200_ctx* ctx, const kgl_b200_fst_options* options, dou
                      double* per_locus /* nullable, [n_pairs][n_loci][2] */, double* windows /* nullable, [n_pairs][n_windows][3] */,
                      uint64_t* n_windows);
 
+/* Hardy-Weinberg equilibrium per locus and group, and variant QC (PLINK's --hardy and --hwe / --geno / --maf). The test assumes
+ * diploid calls (for Pf7 a heterozygous call is a mixed infection, not a diploid genotype). Run it per super-population: pooling
+ * differentiated populations fails HWE at nearly every common site (the Wahlund effect).
+ * For group k at locus l with the counts n0..n3 of kgl_b200_run_group_counts (code 3 is missing):
+ *     v = n0 + n1 + n2,  n_r = min(n1 + 2 n2, n1 + 2 n0) rare-allele copies,  n_c = 2 v - n_r
+ * The support is h = n_r mod 2, .., n_r - 2, n_r heterozygotes; at h there are r = (n_r - h) / 2 rare and c = (n_c - h) / 2 common
+ * homozygotes. Exact test (Wigginton, Cutler & Abecasis 2005) as this fixed sequence of IEEE double operations, round to nearest,
+ * no FMA (every integer is computed exactly and converted once; all are exact in double because v < 2^25):
+ *     mode m = floor(n_r n_c / (2 v)) in integers, plus 1 when its parity differs from n_r's;  P(m) = 1.0
+ *     downward  P(h - 2) = (P(h) * (double)(h (h - 1))) / (double)(4 (r + 1) (c + 1))
+ *     upward    P(h + 2) = (P(h) * (double)(4 r c)) / (double)((h + 2) (h + 1))
+ *     S = 1.0, then + P(m - 2), + P(m - 4), .. (the terms below the mode in the order computed), then + P(m + 2), + P(m + 4), ..
+ *     N = the same order from 0.0, adding only the terms with P(h) <= P(obs) * (1 + 2^-40) (the product rounded once), obs = n1
+ *     p = N / S;  mid-p (midp = 1, Graffelman & Moreno 2013): p = (N - 0.5 * P(obs)) / S
+ * The margin makes rounding-level near-ties count as ties. N adds a subset of S's terms in S's order and rounding is monotone, so
+ * p <= 1 without a clamp, and p == 1.0 exactly when every term qualifies. p = 1 when n_r = 0 (also with midp); NaN when v = 0.
+ * Floor: p = 0 when P(obs) underflows to 0.0 relative to the mode (PLINK reports smaller values there). A walk may stop a side
+ * early, bit for bit the same (hwe.cuh): only terms under half an ulp of both sums are skipped.
+ * Per-locus F (nullable f): F = 1 - (double)(2 v n1) / (double)(s (2 v - s)) with s = n1 + 2 n2 (one IEEE division and one
+ * subtraction); NaN when v = 0 or s is 0 or 2 v. Multi-allelic rows (kgl_b200_upload_multi_allelic) hold only codes 0 and 3 and are
+ * not biallelic genotypes: p and F are NaN there in every group.
+ * Every result is per locus, so a locus-sharded multi-GPU caller runs each shard on its own GPU and needs no exchange.
+ * Errors: those of kgl_b200_run_group_counts (KGL_B200_ERR_STATE before a genotype upload or for group == NULL without
+ * super-population labels; KGL_B200_ERR_INVALID for n_groups outside 1..64 or a bad label), and KGL_B200_ERR_INVALID for midp other
+ * than 0 / 1, a null output, or a group of 2^25 genomes or more. */
+typedef struct kgl_b200_hardy_options {      /* zero-initialise; 16 bytes */
+  const uint8_t* group;  uint32_t n_groups;  /* as kgl_b200_run_group_counts (NULL = super-population labels); pooled: all 0, 1 group */
+  uint32_t midp;                             /* 0 = p, 1 = mid-p */
+} kgl_b200_hardy_options;
+int kgl_b200_run_hardy(kgl_b200_ctx* ctx, const kgl_b200_hardy_options* options, double* p_hwe /* [n_loci][n_groups] */,
+                       double* f /* nullable, [n_loci][n_groups] */);
+/* Variant QC: keep_out uint8[n_loci] = 1 for the loci that pass every filter whose threshold is not 0, *n_kept = their number.
+ * Over ALL genomes, with the raw counts n0..n3 of kgl_b200_run_allele_count, v = n0 + n1 + n2, s = n1 + 2 n2:
+ *     call rate (N - n3) / N >= min_call_rate       (PLINK --geno x is min_call_rate = 1 - x)
+ *     MAF min(s, 2 v - s) / (2 v) >= min_maf        (v = 0 fails)
+ * each one exact IEEE division of integers; and p >= min_hwe_p (kgl_b200_run_hardy with group / n_groups / midp) in every group with
+ * v >= 1 (a group without calls does not vote). A threshold of 0 applies no filter (a zero-initialised struct filters nothing), and
+ * min_hwe_p = 0 runs no test and needs no labels. keep_out is 0 for multi-allelic rows and where the input keep is 0. It is the mask
+ * kgl_b200_pca_options.keep, kgl_b200_ld_options.keep and kgl_b200_fst_options.keep take, and kgl_b200_set_locus_filter takes it
+ * too. Only the mask crosses PCIe (n_loci bytes). Errors: those of kgl_b200_run_hardy when min_hwe_p != 0 (STATE before a genotype
+ * upload in any case), and KGL_B200_ERR_INVALID for a NaN threshold or one outside its range (min_call_rate and min_hwe_p in [0, 1],
+ * min_maf in [0, 0.5]), midp other than 0 / 1, or a null output. */
+typedef struct kgl_b200_qc_options {         /* zero-initialise; 48 bytes */
+  const uint8_t* keep;                       /* uint8[n_loci] input mask, NULL = every locus */
+  double min_call_rate;
+  double min_maf;
+  double min_hwe_p;
+  const uint8_t* group;  uint32_t n_groups;  /* the groups of the test, as kgl_b200_hardy_options */
+  uint32_t midp;
+} kgl_b200_qc_options;
+int kgl_b200_run_variant_qc(kgl_b200_ctx* ctx, const kgl_b200_qc_options* options, uint8_t* keep_out /* [n_loci] */, uint64_t* n_kept);
+/* Terms of the exact test walked by the last kgl_b200_run_hardy / kgl_b200_run_variant_qc on this context, over all cells. */
+uint64_t kgl_b200_last_hardy_terms(const kgl_b200_ctx* ctx);
+
 /* CalcFWS::updateGenomeFWSMap (kga_PfEMP/kga_analysis_PfEMP_FWS.cpp:15-101): for each of n_bins allele-frequency bins
  * [lower[b], upper[b]) of AF column `pop` (the P7FrequencyFilter pair AF >= lower and not AF >= upper,
  * kgl_variant_filter_Pf7.cpp:20-66; a locus without AF is in no bin) the AlleleSummmary of every genome over the bin's loci:

@@ -37,7 +37,7 @@ EXPORTS = [
     "kgl_b200_set_stream", "kgl_b200_synchronize", "kgl_b200_upload_genotypes", "kgl_b200_upload_loci",
     "kgl_b200_set_genome_superpop", "kgl_b200_upload_multi_allelic", "kgl_b200_run_multi_allele_count", "kgl_b200_set_unphased", "kgl_b200_select_loci", "kgl_b200_set_locus_selection",
     "kgl_b200_get_locus_selection", "kgl_b200_count_loci", "kgl_b200_set_locus_filter", "kgl_b200_synth_genotypes", "kgl_b200_download_genotypes", "kgl_b200_run_allele_count",
-    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_run_ld_pairs", "kgl_b200_run_ld_prune", "kgl_b200_run_group_counts", "kgl_b200_run_fst", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
+    "kgl_b200_run_inbreed", "kgl_b200_inbreed_used_moment_tables", "kgl_b200_run_count_and_inbreed", "kgl_b200_run_loglik_grid", "kgl_b200_run_ibs", "kgl_b200_run_king", "kgl_b200_run_king_pairs", "kgl_b200_run_pca", "kgl_b200_run_grm_product", "kgl_b200_run_ld_pairs", "kgl_b200_run_ld_prune", "kgl_b200_run_group_counts", "kgl_b200_run_fst", "kgl_b200_run_hardy", "kgl_b200_run_variant_qc", "kgl_b200_last_hardy_terms", "kgl_b200_ibs_tile_grid", "kgl_b200_enqueue_ibs_tile_list", "kgl_b200_run_ibs_tile_list", "kgl_b200_set_ibs_tensor_cores", "kgl_b200_ibs_used_tensor_cores", "kgl_b200_run_ibs_tiles",
     "kgl_b200_run_binned_genome_counts", "kgl_b200_run_hetero_homo", "kgl_b200_location_fis", "kgl_b200_run_gram", "kgl_b200_run_grm", "kgl_b200_enqueue_gram", "kgl_b200_last_gram_kernel_ms", "kgl_b200_enqueue_gram_tiles", "kgl_b200_gram_buffer", "kgl_b200_fetch_gram",
     "kgl_b200_enqueue_ibs_tiles", "kgl_b200_ibs_tiles_buffer", "kgl_b200_ibs_timer_reset", "kgl_b200_ibs_timer_read",
     "kgl_b200_enqueue_count_and_inbreed", "kgl_b200_flush", "kgl_b200_launch_count", "kgl_b200_last_stream_kernel_ms",
@@ -79,6 +79,17 @@ class FstOptions(C.Structure):
                 ("n_pairs", C.c_uint32), ("pairs", C.c_void_p), ("window_bp", C.c_uint64), ("step_bp", C.c_uint64)]
 
 
+class HardyOptions(C.Structure):
+    """kgl_b200_hardy_options (include/kgl_b200.h), 16 bytes; zero = p (not mid-p) per super-population."""
+    _fields_ = [("group", C.c_void_p), ("n_groups", C.c_uint32), ("midp", C.c_uint32)]
+
+
+class QcOptions(C.Structure):
+    """kgl_b200_qc_options (include/kgl_b200.h), 48 bytes; zero = no filter."""
+    _fields_ = [("keep", C.c_void_p), ("min_call_rate", C.c_double), ("min_maf", C.c_double), ("min_hwe_p", C.c_double),
+                ("group", C.c_void_p), ("n_groups", C.c_uint32), ("midp", C.c_uint32)]
+
+
 class KglError(RuntimeError):
     pass
 
@@ -104,6 +115,8 @@ def load_library() -> C.CDLL:
         lib.kgl_b200_last_gram_kernel_ms.restype = C.c_float
         lib.kgl_b200_last_gram_kernel_ms.argtypes = [C.c_void_p]
         lib.kgl_b200_destroy.restype = None
+        lib.kgl_b200_last_hardy_terms.restype = C.c_uint64
+        lib.kgl_b200_last_hardy_terms.argtypes = [C.c_void_p]
         lib.kgl_b200_destroy.argtypes = [C.c_void_p]
         _lib = lib
     return _lib
@@ -469,6 +482,37 @@ class KglB200:
             res["windows"] = win
             res["window_start"] = np.arange(nw, dtype=np.uint64) * np.uint64(step)
         return res
+
+    def hardy(self, group=None, n_groups=None, midp: bool = False, f: bool = False):
+        """Exact Hardy-Weinberg test per (locus, group) (include/kgl_b200.h): a dict with p float64[L][G] (mid-p with midp=True; NaN
+        where a group has no call and on multi-allelic rows) and, with f=True, f float64[L][G] = 1 - H_obs / H_exp. group=None: the
+        super-population labels (G = 6); pass zeros for one pooled group."""
+        g, G = self._groups(group, n_groups)
+        opt = HardyOptions(group=None if g is None else g.ctypes.data, n_groups=G, midp=int(bool(midp)))
+        p = np.zeros((self.n_loci, G), dtype=np.float64)
+        fo = np.zeros((self.n_loci, G), dtype=np.float64) if f else None
+        self._check(self.lib.kgl_b200_run_hardy(self.h, C.byref(opt), _ptr(p), _ptr(fo)), "run_hardy")
+        res = {"p": p}
+        if f:
+            res["f"] = fo
+        return res
+
+    def variant_qc(self, min_call_rate: float = 0.0, min_maf: float = 0.0, min_hwe_p: float = 0.0, group=None, n_groups=None,
+                   midp: bool = False, keep=None):
+        """Variant QC mask (keep uint8[L], n_kept): call rate over all genomes >= min_call_rate, MAF >= min_maf and the exact HWE
+        p >= min_hwe_p in every group with calls; 0 = no filter. The mask is meant for pca / ld_prune / fst(keep=...)."""
+        g, G = self._groups(group, n_groups) if min_hwe_p else (None, 0)
+        kp = self._keep(keep)
+        opt = QcOptions(keep=None if kp is None else kp.ctypes.data, min_call_rate=float(min_call_rate), min_maf=float(min_maf),
+                        min_hwe_p=float(min_hwe_p), group=None if g is None else g.ctypes.data, n_groups=G, midp=int(bool(midp)))
+        out = np.zeros(self.n_loci, dtype=np.uint8)
+        n = C.c_uint64(0)
+        self._check(self.lib.kgl_b200_run_variant_qc(self.h, C.byref(opt), _ptr(out), C.byref(n)), "run_variant_qc")
+        return out, int(n.value)
+
+    def last_hardy_terms(self) -> int:
+        """Terms of the exact test walked by the last hardy / variant_qc call (all cells)."""
+        return int(self.lib.kgl_b200_last_hardy_terms(self.h))
 
     def binned_genome_counts(self, lower, upper, pop: int = 0, present_only: bool = True):
         """(counts uint64[n_bins][N][4], rows uint64[n_bins]) -- CalcFWS' per-genome AlleleSummmary per AF bin."""

@@ -19,6 +19,7 @@
 #include "pca.cuh"
 #include "ld.cuh"
 #include "fst.cuh"
+#include "hwe.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 
@@ -324,6 +325,11 @@ struct kgl_b200_ctx {
   DevBuf<double2> d_fst_terms, d_fst_blocks;
   DevBuf<uint32_t> d_fst_used;
   DevBuf<double> d_fst_out, d_fst_windows;
+  // Hardy-Weinberg and variant QC (hwe.cuh): the multi-allelic row flags, the cells' sort keys, p / F per cell, the QC mask
+  DevBuf<uint8_t> d_hwe_multi, d_hwe_sort_temp, d_qc_keep, d_qc_out;
+  DevBuf<unsigned long long> d_hwe_keys, d_hwe_keys2, d_hwe_stats;   // stats: terms walked, loci kept
+  DevBuf<double> d_hwe_p, d_hwe_f;
+  uint64_t hwe_terms = 0;
 
   // iterative estimator state
   int algo = -1, phase = 0, iteration = 0;
@@ -1801,6 +1807,58 @@ int group_counts_device(kgl_b200_ctx* c, uint32_t n_groups, const uint8_t* group
   return KGL_B200_OK;
 }
 
+// ---- Hardy-Weinberg equilibrium (hwe.cuh) -----------------------------------------------------------------------------------
+// The multi-allelic row flags into d_hwe_multi; null when the matrix has none.
+int hwe_multi_flags(kgl_b200_ctx* c, const uint8_t*& flags) {
+  flags = nullptr;
+  if (c->n_multi == 0) return KGL_B200_OK;
+  KGL_CUDA(c, c->d_hwe_multi.ensure(c->L));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_hwe_multi.p, 0, c->L, c->stream));
+  k_hwe_mark_rows<<<blocks_for(c->n_multi, 256), 256, 0, c->stream>>>(c->d_multi_rows.p, c->n_multi, c->d_hwe_multi.p);
+  KGL_LAUNCH_CHECK(c);
+  flags = c->d_hwe_multi.p;
+  return KGL_B200_OK;
+}
+
+// p (and F) of every (locus, group) cell into d_hwe_p / d_hwe_f ([L][G]) for labels `group` (NULL = the super-population labels):
+// the group counts, the cells ordered by walk length, the walk. G receives the number of groups.
+int hardy_device(kgl_b200_ctx* c, const uint8_t* group, uint32_t n_groups, uint32_t midp, bool want_f, uint32_t& G) {
+  if (midp > 1) return fail(c, KGL_B200_ERR_INVALID, "midp must be 0 or 1");
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  if (c->N >= kHweMaxGenomes) {              // v < 2^25 keeps every integer of the recurrence exact in double
+    const uint8_t* lab = group ? group : c->h_superpop.data();
+    if (!group && !c->have_superpop) return fail(c, KGL_B200_ERR_STATE, "group == NULL needs the super-population labels (kgl_b200_set_genome_superpop)");
+    std::vector<uint64_t> size(256, 0);
+    for (uint64_t g = 0; g < c->N; ++g) ++size[lab[g]];
+    for (int k = 0; k < 255; ++k)
+      if (size[k] >= kHweMaxGenomes) return fail(c, KGL_B200_ERR_INVALID, "Hardy-Weinberg: a group of 2^25 genomes or more");
+  }
+  rc = group_counts_device(c, n_groups, group, G); if (rc) return rc;
+  const uint8_t* multi = nullptr;
+  rc = hwe_multi_flags(c, multi); if (rc) return rc;
+  const uint64_t cells = c->L * G;
+  KGL_CUDA(c, c->d_hwe_keys.ensure(cells));
+  KGL_CUDA(c, c->d_hwe_keys2.ensure(cells));
+  KGL_CUDA(c, c->d_hwe_p.ensure(cells));
+  if (want_f) KGL_CUDA(c, c->d_hwe_f.ensure(cells));
+  KGL_CUDA(c, c->d_hwe_stats.ensure(2));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_hwe_stats.p, 0, 16, c->stream));
+  k_hwe_keys<<<blocks_for(cells, 256), 256, 0, c->stream>>>(c->d_group_counts.p, multi, cells, G, c->d_hwe_keys.p);
+  KGL_LAUNCH_CHECK(c);
+  size_t temp_bytes = 0;
+  KGL_CUDA(c, cub::DeviceRadixSort::SortKeys(nullptr, temp_bytes, c->d_hwe_keys.p, c->d_hwe_keys2.p, cells, kHweKeyShift, kHweKeyShift + 5, c->stream));
+  KGL_CUDA(c, c->d_hwe_sort_temp.ensure(temp_bytes));
+  KGL_CUDA(c, cub::DeviceRadixSort::SortKeys(c->d_hwe_sort_temp.p, temp_bytes, c->d_hwe_keys.p, c->d_hwe_keys2.p, cells, kHweKeyShift,
+                                             kHweKeyShift + 5, c->stream));
+  HweParams P{};
+  P.counts = c->d_group_counts.p; P.order = c->d_hwe_keys2.p; P.multi = multi; P.n_cells = cells; P.n_groups = G; P.midp = midp;
+  P.p = c->d_hwe_p.p; P.f = want_f ? c->d_hwe_f.p : nullptr; P.terms = c->d_hwe_stats.p;
+  k_hwe<<<blocks_for(cells, kHweThreads), kHweThreads, 0, c->stream>>>(P);
+  KGL_LAUNCH_CHECK(c);
+  return KGL_B200_OK;
+}
+
 }  // namespace
 
 // The device buffers free themselves (DevBuf) after this body, the peer regions that map d_xchg must be gone by then.
@@ -3215,5 +3273,61 @@ int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, doubl
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // also: the pageable pairs / keep / range copies have been read
   return KGL_B200_OK;
 }
+
+int kgl_b200_run_hardy(kgl_b200_ctx* c, const kgl_b200_hardy_options* options, double* p_hwe, double* f) {
+  if (!c || !options || !p_hwe) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  uint32_t G = 0;
+  int rc = hardy_device(c, options->group, options->n_groups, options->midp, f != nullptr, G); if (rc) return rc;
+  unsigned long long terms = 0;
+  KGL_CUDA(c, cudaMemcpyAsync(p_hwe, c->d_hwe_p.p, c->L * G * 8, cudaMemcpyDeviceToHost, c->stream));
+  if (f) KGL_CUDA(c, cudaMemcpyAsync(f, c->d_hwe_f.p, c->L * G * 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(&terms, c->d_hwe_stats.p, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  c->hwe_terms = terms;
+  return KGL_B200_OK;
+}
+
+int kgl_b200_run_variant_qc(kgl_b200_ctx* c, const kgl_b200_qc_options* options, uint8_t* keep_out, uint64_t* n_kept) {
+  if (!c || !options || !keep_out || !n_kept) return fail(c, KGL_B200_ERR_INVALID, "null argument");
+  const kgl_b200_qc_options& o = *options;
+  if (!(o.min_call_rate >= 0.0 && o.min_call_rate <= 1.0)) return fail(c, KGL_B200_ERR_INVALID, "min_call_rate must be in [0, 1]");
+  if (!(o.min_maf >= 0.0 && o.min_maf <= 0.5)) return fail(c, KGL_B200_ERR_INVALID, "min_maf must be in [0, 0.5]");
+  if (!(o.min_hwe_p >= 0.0 && o.min_hwe_p <= 1.0)) return fail(c, KGL_B200_ERR_INVALID, "min_hwe_p must be in [0, 1]");
+  if (o.midp > 1) return fail(c, KGL_B200_ERR_INVALID, "midp must be 0 or 1");
+  int rc = use_device(c); if (rc) return rc;
+  rc = require_population(c, false); if (rc) return rc;
+  uint32_t G = 0;
+  if (o.min_hwe_p != 0.0) { rc = hardy_device(c, o.group, o.n_groups, o.midp, false, G); if (rc) return rc; }
+  // The pooled counts come from the raw streaming pass PCA and LD run (pca_prepare): it reads the matrix at the streaming rate, needs
+  // no label table, and leaves d_group_counts holding the groups of the test.
+  rc = default_superpop(c); if (rc) return rc;
+  rc = launch_count(c, true, true, false, false, false, nullptr, false, &c->d_pca_counts); if (rc) return rc;
+  const uint8_t* multi = nullptr;
+  rc = hwe_multi_flags(c, multi); if (rc) return rc;
+  if (o.keep) {
+    KGL_CUDA(c, c->d_qc_keep.ensure(c->L));
+    KGL_CUDA(c, cudaMemcpyAsync(c->d_qc_keep.p, o.keep, c->L, cudaMemcpyHostToDevice, c->stream));
+  }
+  KGL_CUDA(c, c->d_qc_out.ensure(c->L));
+  KGL_CUDA(c, c->d_hwe_stats.ensure(2));
+  if (o.min_hwe_p == 0.0) KGL_CUDA(c, cudaMemsetAsync(c->d_hwe_stats.p, 0, 8, c->stream));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_hwe_stats.p + 1, 0, 8, c->stream));
+  QcParams P{};
+  P.pooled = c->d_pca_counts.p; P.p = o.min_hwe_p != 0.0 ? c->d_hwe_p.p : nullptr; P.keep = o.keep ? c->d_qc_keep.p : nullptr;
+  P.multi = multi; P.n_loci = c->L; P.n_genomes = c->N; P.n_groups = G;
+  P.min_call_rate = o.min_call_rate; P.min_maf = o.min_maf; P.min_hwe_p = o.min_hwe_p;
+  P.keep_out = c->d_qc_out.p; P.n_kept = c->d_hwe_stats.p + 1;
+  k_variant_qc<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(P);
+  KGL_LAUNCH_CHECK(c);
+  unsigned long long stats[2] = {0, 0};
+  KGL_CUDA(c, cudaMemcpyAsync(keep_out, c->d_qc_out.p, c->L, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaMemcpyAsync(stats, c->d_hwe_stats.p, 16, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));     // also: the pageable keep copy has been read
+  c->hwe_terms = stats[0];
+  *n_kept = stats[1];
+  return KGL_B200_OK;
+}
+
+uint64_t kgl_b200_last_hardy_terms(const kgl_b200_ctx* c) { return c ? c->hwe_terms : 0; }
 
 }  // extern "C"
