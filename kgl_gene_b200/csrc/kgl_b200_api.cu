@@ -150,7 +150,7 @@ struct kgl_b200_ctx {
   DevBuf<uint8_t> d_sort_temp;
   DevBuf<uint2> d_dropped_cells;         // per indexed cell {row, frequency float of the genome's population} (k_dropped_cells)
   uint64_t n_dropped = 0;
-  bool dropped_indexed = false, dropped_valid = false;
+  bool dropped_indexed = false;
   int dropped_cells_state = 0;           // 0: stale; 1: rows only (no frequencies uploaded yet); 2: rows + frequencies
   std::vector<uint32_t> h_offsets;     // host copy of the locus offsets (they arrive from the host): window -> row range
   uint64_t sel_row_lo = 0, sel_row_hi = ~0ull;   // rows that can be selected (the window of the last select_loci); [0, inf): unknown
@@ -164,6 +164,14 @@ struct kgl_b200_ctx {
   DevBuf<uint8_t> d_chain_mark;
   std::vector<uint8_t> h_superpop;
   bool units_valid = false;
+  // Built from the genotype matrix on first use, reset by a new one (matrix_changed; the buffers stay for a matrix of the same shape).
+  // ibs_mode: 0: no code-3 cell; 1: in-kernel validity plane; 2: pre-masked planes + sparse repair. gram_valid: d_gram holds the last
+  // kgl_b200_enqueue_gram[_tiles] result (the IBS tensor form lends it out).
+  struct MatrixCaches {
+    bool sm_valid = false, codes_valid = false, dropped_valid = false, ibs_class_valid = false, codes16_valid = false, codes_loci_valid = false;
+    int ibs_mode = -1;
+    bool gram_valid = false;
+  } matrix_caches;
 
   // per-locus preparation
   // Outputs of k_locus_prepare, double-buffered: the preparation of pass i+1 runs on prep_stream while the tail kernel
@@ -210,7 +218,6 @@ struct kgl_b200_ctx {
   DevBuf<uint32_t> d_sm_lo, d_sm_hi;
   DevBuf<uint2> d_sm_codes;             // interleaved codes of the same cells (terms_fast.cuh)
   uint64_t n_gblocks = 0, n_words = 0;
-  bool sm_valid = false, codes_valid = false;
 
   // fused pass outputs
   DevBuf<uint32_t> d_locus_counts, d_cta_counts[2];
@@ -265,7 +272,6 @@ struct kgl_b200_ctx {
   // pairwise IBS (ibs_tile.cuh): planes of the dense kernel, tile list, accumulators, compact tile results
   DevBuf<uint32_t> d_ibs_lo, d_ibs_hi, d_sm_valid, d_ibs_acc, d_ibs_tiles_out;
   DevBuf<uint2> d_ibs_tiles;
-  int ibs_mode = -1;                 // 0: no code-3 cell; 1: in-kernel validity plane; 2: pre-masked planes + sparse repair
   TimerRing ibs_timer;
   uint64_t ibs_last_count = 0;
   TileKey ibs_tiles_key;                 // the tile list on the device
@@ -282,14 +288,11 @@ struct kgl_b200_ctx {
   DevBuf<uint32_t> d_ibs_tile_block;   // per tile: index of its block | 1 << 31 when mirrored
   uint32_t ibs_n_blocks = 0;
   DevBuf<int32_t> d_ibs_class;         // {heterozygous, hom-alt} cells per genome on the IBS planes
-  bool ibs_class_valid = false;
   bool ibs_tensor_enabled = true, ibs_used_tensor = false;
   DevBuf<uint2> d_gram_tiles;
   DevBuf<double> d_gp_chunks, d_gp;
   DevBuf<uint8_t> d_gram_out;
   uint64_t gram_tiles_ld = 0, gram_n_tiles = 0, gram_first = 0, gram_stride = 1;
-  bool codes16_valid = false;
-  bool gram_valid = false;             // d_gram holds the last kgl_b200_enqueue_gram[_tiles] result (the IBS tensor form lends it out)
   cudaEvent_t gram_e0 = nullptr, gram_e1 = nullptr;
   // KING-robust kinship (king.cuh): M = H C^T blocks, dense slab, pair list
   DevBuf<int32_t> d_king_m;
@@ -301,7 +304,6 @@ struct kgl_b200_ctx {
   DevBuf<uint8_t> d_pair_sort_temp;
   // genotype PCA (pca.cuh): loci-major codes (code 3 kept), per-locus p / d / used, the product's blocks, digits and Gram outputs
   DevBuf<uint32_t> d_codes_loci;
-  bool codes_loci_valid = false;
   DevBuf<uint8_t> d_pca_keep, d_pca_used;
   DevBuf<uint32_t> d_pca_counts;            // raw per-locus counts of PCA's own counting pass (d_locus_counts stays the caller's)
   DevBuf<double> d_pca_p, d_pca_d, d_pca_x, d_pca_y, d_pca_wv, d_pca_out;
@@ -373,7 +375,33 @@ void peer_unregister(const kgl_b200_ctx* c) {
     if (g_peer_regions[i].owner == c) g_peer_regions.erase(g_peer_regions.begin() + i); else ++i;
 }
 
+// ---- what each input invalidates: the setters call these, nothing else clears a cache, and an input that implies another calls
+// the other's function.
+void selection_changed(kgl_b200_ctx* c) { c->prep_valid = false; }      // the preparation (and the moment tables that follow it)
+void filter_changed(kgl_b200_ctx* c) { c->keep_valid = false; selection_changed(c); }
+void multi_changed(kgl_b200_ctx* c) { c->n_multi = 0; selection_changed(c); }
+void frequencies_changed(kgl_b200_ctx* c) { c->dropped_cells_state = 0; selection_changed(c); }   // the code-3 side list carries them
+void labels_changed(kgl_b200_ctx* c) { c->units_valid = false; c->gc_superpop = false; frequencies_changed(c); }
+void ibs_form_changed(kgl_b200_ctx* c) { c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0; }   // a tile list has one form's blocks
+void matrix_changed(kgl_b200_ctx* c) { c->matrix_caches = {}; ibs_form_changed(c); multi_changed(c); labels_changed(c); }
+void phase_changed(kgl_b200_ctx* c) { c->mom_valid = false; }
+
 inline unsigned blocks_for(uint64_t n, unsigned threads) { return (unsigned)((n + threads - 1) / threads); }
+
+// n elements from the host into buf (grown to hold them) on the context stream.
+template <class T>
+int upload(kgl_b200_ctx* c, DevBuf<T>& buf, const T* src, size_t n) {
+  KGL_CUDA(c, buf.ensure(n));
+  KGL_CUDA(c, cudaMemcpyAsync(buf.p, src, n * sizeof(T), cudaMemcpyHostToDevice, c->stream));
+  return KGL_B200_OK;
+}
+
+// One 64-bit counter of the device, read once the context stream has reached it.
+int read_counter(kgl_b200_ctx* c, const void* src, uint64_t& value) {
+  KGL_CUDA(c, cudaMemcpyAsync(&value, src, 8, cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
 
 // Orders the context stream after the tail of the last pass (no host synchronisation).
 int join_tail(kgl_b200_ctx* c) {
@@ -430,16 +458,16 @@ int build_unit_tables(kgl_b200_ctx* c) {
     popmask[(size_t)k * units + (g >> 6)] |= 1ull << (g & 63);
     need32[g >> 5] |= (uint8_t)(1u << k);
   }
-  KGL_CUDA(c, c->d_need32.ensure(need32.size()));
-  KGL_CUDA(c, c->d_popmask.ensure(popmask.size()));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_need32.p, need32.data(), need32.size(), cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_popmask.p, popmask.data(), popmask.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  int rc = upload(c, c->d_need32, need32.data(), need32.size()); if (rc) return rc;
+  rc = upload(c, c->d_popmask, popmask.data(), popmask.size()); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   c->units_valid = true;
   return KGL_B200_OK;
 }
 
-int require_population(kgl_b200_ctx* c, bool need_loci) {
+// Where an entry point that reads the population starts: use_device, then the checks that the population is there.
+int use_population(kgl_b200_ctx* c, bool need_loci, bool join = true) {
+  int rc = use_device(c, join); if (rc) return rc;
   if (!c->have_geno) return fail(c, KGL_B200_ERR_STATE, "no genotype matrix uploaded");
   if (need_loci) {
     if (!c->have_loci) return fail(c, KGL_B200_ERR_STATE, "no allele frequencies uploaded (kgl_b200_upload_loci)");
@@ -448,6 +476,13 @@ int require_population(kgl_b200_ctx* c, bool need_loci) {
     for (uint64_t g = 0; g < c->N; ++g)
       if (c->h_superpop[g] >= c->n_pop) return fail(c, KGL_B200_ERR_INVALID, "genome super-population index out of range");
   }
+  return KGL_B200_OK;
+}
+
+// An offset for every row of the locus table, in ascending order; `missing` and `unsorted` are the messages of the two failures.
+int require_sorted_offsets(kgl_b200_ctx* c, const char* missing, const char* unsorted) {
+  if (!c->have_offsets || c->h_offsets.size() != c->L) return fail(c, KGL_B200_ERR_STATE, missing);
+  if (!std::is_sorted(c->h_offsets.begin(), c->h_offsets.end())) return fail(c, KGL_B200_ERR_INVALID, unsorted);
   return KGL_B200_OK;
 }
 
@@ -521,7 +556,7 @@ int ensure_prepared(kgl_b200_ctx* c, bool want_w0 = false, bool want_selw = fals
 }
 
 int ensure_sample_major(kgl_b200_ctx* c) {
-  if (c->sm_valid) return KGL_B200_OK;
+  if (c->matrix_caches.sm_valid) return KGL_B200_OK;
   c->n_gblocks = c->units * 2;
   const uint64_t nw = term_words(c->L);
   c->n_words = nw;
@@ -532,7 +567,7 @@ int ensure_sample_major(kgl_b200_ctx* c) {
   k_to_sample_major<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const uint32_t*>(c->d_packed.p), c->units * 4, c->L,
                                                   c->n_gblocks, nw, c->d_sm_lo.p, c->d_sm_hi.p);
   KGL_LAUNCH_CHECK(c);
-  c->sm_valid = true;
+  c->matrix_caches.sm_valid = true;
   return KGL_B200_OK;
 }
 
@@ -573,26 +608,25 @@ int finish_dropped_index(kgl_b200_ctx* c, unsigned long long total) {
     KGL_LAUNCH_CHECK(c);
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   }
-  c->dropped_valid = true; c->dropped_cells_state = 0;
+  c->matrix_caches.dropped_valid = true; c->dropped_cells_state = 0;
   return KGL_B200_OK;
 }
 
 // The side list of code-3 cells, built once per matrix that is already resident (device-generated populations; uploads index
 // while they copy, see kgl_b200_upload_genotypes).
 int build_dropped_index(kgl_b200_ctx* c) {
-  if (c->dropped_valid) return KGL_B200_OK;
+  if (c->matrix_caches.dropped_valid) return KGL_B200_OK;
   const uint64_t n128 = c->L * c->units;
   const unsigned grid = (unsigned)std::min<uint64_t>((n128 + 255) / 256, (uint64_t)c->sm_count * 16);
   KGL_CUDA(c, c->d_dropped_counter.ensure(2));
   KGL_CUDA(c, cudaMemsetAsync(c->d_dropped_counter.p, 0, 16, c->stream));
   k_dropped_count<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const uint4*>(c->d_packed.p), n128, c->d_dropped_counter.p);
   KGL_LAUNCH_CHECK(c);
-  unsigned long long total = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_dropped_counter.p, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  uint64_t total = 0;
+  int rc = read_counter(c, c->d_dropped_counter.p, total); if (rc) return rc;
   if (total > 0 && total <= dropped_index_limit(c)) {
     KGL_CUDA(c, c->d_dropped_unsorted.ensure(total));
-    int rc = launch_dropped_index(c, 0, n128, total); if (rc) return rc;
+    rc = launch_dropped_index(c, 0, n128, total); if (rc) return rc;
   }
   return finish_dropped_index(c, total);
 }
@@ -638,7 +672,6 @@ DenseTotals dense_totals(const kgl_b200_ctx* c, const kgl_b200_ctx::PrepSet& S) 
   return DenseTotals{S.totals_fx(), 1.0 / fx, 128.0 / fx};
 }
 
-// The fused streaming pass + its tail. raw: allele_count over all loci; otherwise over the selected loci.
 // Row mask that replaces the per-population selection flags of a pass: every genome belongs to "population 0" and a row
 // counts iff bit 0 of flags16 is set (the AF-bin passes of kgl_b200_run_binned_genome_counts).
 struct MaskOverride {
@@ -646,29 +679,35 @@ struct MaskOverride {
   const uint8_t* zero_superpop;
 };
 
-// want_moments: the tail assembles the moment partials of every genome (d_partials; + the Simple closed form into d_results
-// when simple_results); otherwise it leaves the raw per-genome counts d_gcounts {set lo bits, set hi bits} and d_n3.
+// The fused streaming pass + its tail (launch_count). raw: allele_count over all loci; otherwise over the selected loci.
+// moments: the tail assembles the moment partials of every genome (d_partials; + the Simple closed form into d_results when
+// simple_results); otherwise it leaves the raw per-genome counts d_gcounts {set lo bits, set hi bits} and d_n3.
 // defer_join: the tail stays on the tail stream and the context stream is NOT ordered after it (the resident pass: the next
 // pass's streaming kernel may start while this tail runs); the next entry point joins (use_device).
 // counts: where the per-locus counts go (null = d_locus_counts, the buffer kgl_b200_fetch_locus_counts reads).
-int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_genome, bool simple_results = false, bool want_moments = false,
-                 const MaskOverride* mo = nullptr, bool defer_join = false, DevBuf<uint32_t>* counts = nullptr) {
-  DevBuf<uint32_t>& lc = counts ? *counts : c->d_locus_counts;
-  int rc = mo ? KGL_B200_OK : build_unit_tables(c);
+struct CountPass {
+  bool raw = false, locus_counts = false, genome = false, moments = false, simple_results = false, defer_join = false;
+  const MaskOverride* mask = nullptr;
+  DevBuf<uint32_t>* counts = nullptr;
+};
+
+int launch_count(kgl_b200_ctx* c, const CountPass& p) {
+  DevBuf<uint32_t>& lc = p.counts ? *p.counts : c->d_locus_counts;
+  int rc = p.mask ? KGL_B200_OK : build_unit_tables(c);
   if (rc) return rc;
   rc = build_dropped_index(c);
   if (rc) return rc;
   const StreamPlan pl = plan_stream(c->units, c->L, c->sm_count);
   if (pl.padded_rows > c->padded_rows) return fail(c, KGL_B200_ERR_STATE, "internal: stream plan needs more padded rows than allocated");
-  if (want_locus_counts) {
+  if (p.locus_counts) {
     KGL_CUDA(c, lc.ensure((size_t)c->L * 4));
     if (pl.slices > 1) KGL_CUDA(c, cudaMemsetAsync(lc.p, 0, (size_t)c->L * 16, c->stream));
   }
   const bool indexed = c->dropped_indexed || c->n_dropped == 0;
   rc = ensure_side_streams(c); if (rc) return rc;
-  if (want_genome) {
+  if (p.genome) {
     // the tail of the pass before the last one may still read the buffer this pass writes
-    if (c->tail_pending && !defer_join) { rc = join_tail(c); if (rc) return rc; }
+    if (c->tail_pending && !p.defer_join) { rc = join_tail(c); if (rc) return rc; }
     c->cbuf ^= 1;
     if (c->tail_marked[c->cbuf]) KGL_CUDA(c, cudaStreamWaitEvent(c->stream, c->tail_done[c->cbuf], 0));
     KGL_CUDA(c, c->d_cta_counts[c->cbuf].ensure((size_t)pl.n_ctas * 2 * c->Npad));
@@ -678,38 +717,38 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
     c->d_n3 = c->d_gcounts + c->Npad * 2;
     c->d_ecorr_scan = reinterpret_cast<unsigned long long*>(c->d_scratch.p + (size_t)c->Npad * 16);
     if (!indexed) KGL_CUDA(c, cudaMemsetAsync(c->d_scratch.p, 0, (size_t)c->Npad * 32, c->stream));
-    if (indexed) { rc = ensure_dropped_cells(c, want_moments); if (rc) return rc; }
+    if (indexed) { rc = ensure_dropped_cells(c, p.moments); if (rc) return rc; }
   }
   StreamParams P{};
   fill_stream_params(P, pl);
   P.packed = reinterpret_cast<const uint4*>(c->d_packed.p);
   P.units = (uint32_t)c->units; P.n_loci = (uint32_t)c->L; P.n_genomes = (uint32_t)c->N;
-  P.flags16 = mo ? mo->flags16 : (raw ? nullptr : c->prep[c->par].flags16.p);
-  P.sum64 = mo ? mo->sum64 : (raw ? nullptr : c->prep[c->par].sum64.p);
-  P.popmask32 = mo ? mo->popmask32 : reinterpret_cast<const uint32_t*>(c->d_popmask.p);     // little endian: u64 mask = {low half, high half}
-  P.need32 = mo ? mo->need32 : c->d_need32.p;
-  P.n_pop = (raw || mo) ? 1 : c->n_pop;
-  P.locus_counts = want_locus_counts ? lc.p : nullptr;
-  P.cta_counts = want_genome ? c->d_cta_counts[c->cbuf].p : nullptr;
+  P.flags16 = p.mask ? p.mask->flags16 : (p.raw ? nullptr : c->prep[c->par].flags16.p);
+  P.sum64 = p.mask ? p.mask->sum64 : (p.raw ? nullptr : c->prep[c->par].sum64.p);
+  P.popmask32 = p.mask ? p.mask->popmask32 : reinterpret_cast<const uint32_t*>(c->d_popmask.p);     // little endian: u64 mask = {low half, high half}
+  P.need32 = p.mask ? p.mask->need32 : c->d_need32.p;
+  P.n_pop = (p.raw || p.mask) ? 1 : c->n_pop;
+  P.locus_counts = p.locus_counts ? lc.p : nullptr;
+  P.cta_counts = p.genome ? c->d_cta_counts[c->cbuf].p : nullptr;
   P.n_genomes_padded = (uint32_t)c->Npad;
   stream_make_tensor_map(P, pl, c->padded_rows);          // wide populations: one 2-D TMA box per stage
   cudaEvent_t e0, e1;
   KGL_CUDA(c, c->timer.next(e0, e1));
   if (!e0) { e0 = c->ev0; e1 = c->ev1; }       // the ring is full: kgl_b200_last_stream_kernel_ms still times this launch
   KGL_CUDA(c, cudaEventRecord(e0, c->stream));
-  KGL_CUDA(c, launch_stream(P, pl, want_locus_counts, want_genome, c->stream));
+  KGL_CUDA(c, launch_stream(P, pl, p.locus_counts, p.genome, c->stream));
   ++c->launches;
   KGL_CUDA(c, cudaEventRecord(e1, c->stream));
   c->ev_valid = true;
   c->last_e0 = e0; c->last_e1 = e1;
-  if (want_locus_counts && pl.slices > 1) {
+  if (p.locus_counts && pl.slices > 1) {
     k_fix_locus_n0<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(lc.p, c->L, (uint32_t)c->N);
     KGL_LAUNCH_CHECK(c);
   }
-  if (!want_genome) return KGL_B200_OK;
-  const uint16_t* fl = mo ? mo->flags16 : (raw ? nullptr : c->prep[c->par].flags16.p);
+  if (!p.genome) return KGL_B200_OK;
+  const uint16_t* fl = p.mask ? p.mask->flags16 : (p.raw ? nullptr : c->prep[c->par].flags16.p);
   const kgl_b200_ctx::PrepSet& S = c->prep[c->par];
-  const bool prepared = !raw && !mo;
+  const bool prepared = !p.raw && !p.mask;
   const double fx = prepared ? S.fx : fx_scale_for(c->L);
   if (indexed) {
     // the tail runs on its own stream, behind this pass's streaming kernel
@@ -724,16 +763,16 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
     }
     T.n_genomes = c->N; T.flags16 = fl;
     T.unselected_blocks = prepared ? S.unselected_blocks() : nullptr;
-    T.superpop = mo ? mo->zero_superpop : c->d_superpop.p;
-    T.want_moments = want_moments ? 1 : 0; T.unphased = c->unphased ? 1 : 0;
+    T.superpop = p.mask ? p.mask->zero_superpop : c->d_superpop.p;
+    T.want_moments = p.moments ? 1 : 0; T.unphased = c->unphased ? 1 : 0;
     T.nz_rare = prepared ? S.nz_rare(c->Npad) : nullptr; T.ecorr_rare_fx = prepared ? S.ecorr_fx() : nullptr; T.fx_inv = 1.0 / fx;
     T.totals = dense_totals(c, S); T.partials = c->partials_target ? c->partials_target : c->d_partials.p;
-    T.results = simple_results ? c->d_results.p : nullptr;
+    T.results = p.simple_results ? c->d_results.p : nullptr;
     T.gcounts = c->d_gcounts; T.n3 = c->d_n3;
     k_tail<<<blocks_for(c->N, kTailGenomesPerBlock), 256, 0, c->tail_stream>>>(T);
     KGL_LAUNCH_CHECK(c);
     c->tail_pending = true;
-    if (!defer_join) return mark_tail(c, true);
+    if (!p.defer_join) return mark_tail(c, true);
     return KGL_B200_OK;              // the caller adds what else belongs on the tail stream and calls mark_tail(c, false)
   }
   // populations whose code-3 cells are too many to index: separate kernels, the matrix is scanned for the cells
@@ -742,13 +781,13 @@ int launch_count(kgl_b200_ctx* c, bool raw, bool want_locus_counts, bool want_ge
   const uint64_t n128 = c->L * c->units;
   const unsigned grid = (unsigned)std::min<uint64_t>((n128 + 255) / 256, (uint64_t)c->sm_count * 16);
   k_dropped_scan<<<grid, 256, 0, c->stream>>>(reinterpret_cast<const uint4*>(c->d_packed.p), n128, (uint32_t)c->units, fl,
-                                               mo ? mo->zero_superpop : c->d_superpop.p, c->d_af.p, c->L, c->d_n3, c->d_ecorr_scan, fx);
+                                               p.mask ? p.mask->zero_superpop : c->d_superpop.p, c->d_af.p, c->L, c->d_n3, c->d_ecorr_scan, fx);
   KGL_LAUNCH_CHECK(c);
-  if (want_moments) {
+  if (p.moments) {
     k_moment_partials<<<blocks_for(c->N, 256), 256, 0, c->stream>>>(c->d_gcounts, c->d_n3, dense_totals(c, S), c->d_ecorr_scan, S.nz_rare(c->Npad),
                                                                     S.ecorr_fx(), 1.0 / fx, c->d_superpop.p, c->N, c->unphased ? 1 : 0,
                                                                     c->partials_target ? c->partials_target : c->d_partials.p,
-                                                                    simple_results ? c->d_results.p : nullptr);
+                                                                    p.simple_results ? c->d_results.p : nullptr);
     KGL_LAUNCH_CHECK(c);
   }
   return KGL_B200_OK;
@@ -760,7 +799,8 @@ int enqueue_moments(kgl_b200_ctx* c, bool want_locus_counts, bool simple_results
   int rc = ensure_prepared(c, want_w0, want_selw);
   if (rc) return rc;
   KGL_CUDA(c, c->d_partials.ensure((size_t)c->Npad * PART_COUNT));
-  return launch_count(c, false, want_locus_counts, true, simple_results, true, nullptr, defer_join);
+  CountPass p{}; p.locus_counts = want_locus_counts; p.genome = p.moments = true; p.simple_results = simple_results; p.defer_join = defer_join;
+  return launch_count(c, p);
 }
 
 // ---- multi-allelic loci: their share of a pass, added to what the dense path left on the context stream -----------------
@@ -826,12 +866,12 @@ int launch_grid_terms(kgl_b200_ctx* c, const double* d_grid, int n_grid, TermLau
 int ensure_sample_codes(kgl_b200_ctx* c) {
   int rc = ensure_sample_major(c);
   if (rc) return rc;
-  if (c->codes_valid) return KGL_B200_OK;
+  if (c->matrix_caches.codes_valid) return KGL_B200_OK;
   const size_t n = (size_t)c->n_gblocks * c->n_words * 32;
   KGL_CUDA(c, c->d_sm_codes.ensure(n));
   k_to_sample_codes<<<blocks_for(n, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, n, c->d_sm_codes.p);
   KGL_LAUNCH_CHECK(c);
-  c->codes_valid = true;
+  c->matrix_caches.codes_valid = true;
   return KGL_B200_OK;
 }
 
@@ -965,10 +1005,9 @@ int moments_lists(kgl_b200_ctx* c, Fill fill) {
   k_mom_base<<<1, 1024, 0, st>>>(c->d_mom_totals.p, c->N, c->d_mom_base.p);
   KGL_LAUNCH_CHECK(c);
   uint64_t list_len = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&list_len, c->d_mom_base.p + c->N, 8, cudaMemcpyDeviceToHost, st));
-  KGL_CUDA(c, cudaStreamSynchronize(st));
+  int rc = read_counter(c, c->d_mom_base.p + c->N, list_len); if (rc) return rc;
   KGL_CUDA(c, c->d_mom_list.ensure_roomy(std::max<uint64_t>(1, list_len)));
-  int rc = fill(); if (rc) return rc;
+  rc = fill(); if (rc) return rc;
   k_mom_list_limits<<<blocks_for(c->N, 256), 256, 0, st>>>(c->d_mom_list.p, c->d_mom_base.p, c->d_mom_totals.p, c->d_superpop.p,
                                                            c->d_mom_pop_cmin.p, c->N, c->d_mom_limits.p);
   KGL_LAUNCH_CHECK(c);
@@ -1157,24 +1196,24 @@ int newton_sweep_moments(kgl_b200_ctx* c) {
 int ensure_ibs_planes(kgl_b200_ctx* c) {
   int rc = ensure_sample_major(c); if (rc) return rc;
   rc = build_dropped_index(c); if (rc) return rc;
-  if (c->ibs_mode >= 0) return KGL_B200_OK;
+  if (c->matrix_caches.ibs_mode >= 0) return KGL_B200_OK;
   const size_t n = (size_t)c->n_gblocks * c->n_words * 32;
   const unsigned nb = blocks_for(n / 4, 256);
   if (c->n_dropped == 0) {
-    c->ibs_mode = 0;
+    c->matrix_caches.ibs_mode = 0;
   } else if (c->dropped_indexed) {
     KGL_CUDA(c, c->d_ibs_lo.ensure(n));
     KGL_CUDA(c, c->d_ibs_hi.ensure(n));
     k_ibs_premask<<<nb, 256, 0, c->stream>>>(reinterpret_cast<const uint4*>(c->d_sm_lo.p), reinterpret_cast<const uint4*>(c->d_sm_hi.p), n / 4,
                                               reinterpret_cast<uint4*>(c->d_ibs_lo.p), reinterpret_cast<uint4*>(c->d_ibs_hi.p));
     KGL_LAUNCH_CHECK(c);
-    c->ibs_mode = 2;
+    c->matrix_caches.ibs_mode = 2;
   } else {
     KGL_CUDA(c, c->d_sm_valid.ensure(n));
     k_valid_plane<<<nb, 256, 0, c->stream>>>(reinterpret_cast<const uint4*>(c->d_sm_lo.p), reinterpret_cast<const uint4*>(c->d_sm_hi.p), n / 4,
                                               reinterpret_cast<uint4*>(c->d_sm_valid.p));
     KGL_LAUNCH_CHECK(c);
-    c->ibs_mode = 1;
+    c->matrix_caches.ibs_mode = 1;
   }
   return KGL_B200_OK;
 }
@@ -1238,7 +1277,7 @@ std::vector<uint2> tile_coords(const TileList& list, uint64_t side) {
 // reads it as 0, except the code-3 indicator of KING's M = H C^T and of PCA's code-3 run.
 int ensure_codes(kgl_b200_ctx* c) {
   int rc = ensure_sample_major(c); if (rc) return rc;
-  if (c->codes16_valid) return KGL_B200_OK;
+  if (c->matrix_caches.codes16_valid) return KGL_B200_OK;
   const uint64_t ld = gram_ld(c), k_stages = gram_k_stages(c);
   const size_t words = (size_t)ld * k_stages * 8;
   KGL_CUDA(c, c->d_codes16.ensure(words));
@@ -1246,7 +1285,7 @@ int ensure_codes(kgl_b200_ctx* c) {
   k_codes16<<<blocks_for((uint64_t)c->n_gblocks * c->n_words * 32, 256), 256, 0, c->stream>>>(c->d_sm_lo.p, c->d_sm_hi.p, c->n_gblocks,
                                                                                               c->n_words, k_stages, ld, c->d_codes16.p);
   KGL_LAUNCH_CHECK(c);
-  c->codes16_valid = true;
+  c->matrix_caches.codes16_valid = true;
   return KGL_B200_OK;
 }
 
@@ -1274,15 +1313,15 @@ int run_gram_blocks(kgl_b200_ctx* c, const uint32_t* codes, uint32_t table_a, ui
 
 // The genomes' heterozygous / hom-alt cells on the IBS planes (code 3 in neither), once per upload.
 int ensure_ibs_class(kgl_b200_ctx* c) {
-  if (c->ibs_class_valid) return KGL_B200_OK;
+  if (c->matrix_caches.ibs_class_valid) return KGL_B200_OK;
   const size_t n_rows = (size_t)std::max<uint64_t>(c->n_gblocks * 32, gram_ld(c));
   KGL_CUDA(c, c->d_ibs_class.ensure(n_rows * 2));
   KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_class.p, 0, n_rows * 2 * 4, c->stream));
   const uint32_t wpc = 4096;
   k_ibs_class_counts<<<dim3((unsigned)c->n_gblocks, (unsigned)((c->n_words + wpc - 1) / wpc)), 256, 0, c->stream>>>(
-      c->ibs_mode == 2 ? c->d_ibs_lo.p : c->d_sm_lo.p, c->ibs_mode == 2 ? c->d_ibs_hi.p : c->d_sm_hi.p, c->n_words, wpc, c->d_ibs_class.p);
+      c->matrix_caches.ibs_mode == 2 ? c->d_ibs_lo.p : c->d_sm_lo.p, c->matrix_caches.ibs_mode == 2 ? c->d_ibs_hi.p : c->d_sm_hi.p, c->n_words, wpc, c->d_ibs_class.p);
   KGL_LAUNCH_CHECK(c);
-  c->ibs_class_valid = true;
+  c->matrix_caches.ibs_class_valid = true;
   return KGL_B200_OK;
 }
 
@@ -1293,7 +1332,7 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
   KGL_CUDA(c, c->d_ibs_tiles.ensure(n));
   KGL_CUDA(c, c->d_ibs_acc.ensure((size_t)n * 3 * kIbsTileCells));
   // Tensor-core form of the dense part: populations whose code-3 cells are indexed (or absent), n_loci < 2^29
-  const bool tensor = c->ibs_tensor_enabled && c->ibs_mode != 1 && c->L < (1ull << 29);
+  const bool tensor = c->ibs_tensor_enabled && c->matrix_caches.ibs_mode != 1 && c->L < (1ull << 29);
   const bool need_blocks = tensor || want_blocks;
   if (tensor) {
     int rc = ensure_codes(c); if (rc) return rc;
@@ -1318,10 +1357,8 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
         if (it == index.end()) { it = index.emplace(k2, (uint32_t)blocks.size()).first; blocks.push_back(make_uint2(bi, bj)); }
         tile_block[t] = it->second | (mirrored ? 0x80000000u : 0u);
       }
-      KGL_CUDA(c, c->d_ibs_blocks.ensure(blocks.size()));
-      KGL_CUDA(c, c->d_ibs_tile_block.ensure(tile_block.size()));
-      KGL_CUDA(c, cudaMemcpyAsync(c->d_ibs_blocks.p, blocks.data(), blocks.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
-      KGL_CUDA(c, cudaMemcpyAsync(c->d_ibs_tile_block.p, tile_block.data(), tile_block.size() * 4, cudaMemcpyHostToDevice, c->stream));
+      int rc = upload(c, c->d_ibs_blocks, blocks.data(), blocks.size()); if (rc) return rc;
+      rc = upload(c, c->d_ibs_tile_block, tile_block.data(), tile_block.size()); if (rc) return rc;
       c->ibs_n_blocks = (uint32_t)blocks.size();
     }
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));     // the lists are pageable host memory
@@ -1329,7 +1366,7 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
   }
   if (tensor) {
     const size_t block_cells = (size_t)c->ibs_n_blocks * kGramM * kGramN;
-    c->gram_valid = false;                                  // d_gram holds the dosage blocks from here on
+    c->matrix_caches.gram_valid = false;                                  // d_gram holds the dosage blocks from here on
     KGL_CUDA(c, c->d_gram.ensure(block_cells));             // (also kgl_b200_run_gram's matrix: that call sizes it for itself)
     KGL_CUDA(c, c->d_gram_hh.ensure(block_cells));
     KGL_CUDA(c, c->d_gram_aa.ensure(block_cells));
@@ -1337,10 +1374,10 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
   const uint32_t words_used = ibs_words_used(c->L);
   const IbsPlan pl = plan_ibs(n, words_used, c->sm_count);
   IbsParams P{};
-  const bool premasked = c->ibs_mode == 2;
+  const bool premasked = c->matrix_caches.ibs_mode == 2;
   P.plane[0] = premasked ? c->d_ibs_lo.p : c->d_sm_lo.p;
   P.plane[1] = premasked ? c->d_ibs_hi.p : c->d_sm_hi.p;
-  P.plane[2] = c->ibs_mode == 1 ? c->d_sm_valid.p : nullptr;
+  P.plane[2] = c->matrix_caches.ibs_mode == 1 ? c->d_sm_valid.p : nullptr;
   P.n_words = c->n_words; P.words_used = words_used; P.tiles = c->d_ibs_tiles.p; P.n_tiles = n;
   P.words_per_chunk = pl.words_per_chunk; P.n_chunks = pl.n_chunks; P.acc = c->d_ibs_acc.p;
   if (pl.n_chunks > 1) KGL_CUDA(c, cudaMemsetAsync(c->d_ibs_acc.p, 0, (size_t)n * 3 * kIbsTileCells * 4, c->stream));
@@ -1359,12 +1396,12 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
     KGL_LAUNCH_CHECK(c);
     ++c->launches;
   } else {
-    KGL_CUDA(c, launch_ibs(P, pl, c->ibs_mode == 1, c->stream));
+    KGL_CUDA(c, launch_ibs(P, pl, c->matrix_caches.ibs_mode == 1, c->stream));
     ++c->launches;
   }
   c->ibs_used_tensor = tensor;
   if (e1) KGL_CUDA(c, cudaEventRecord(e1, c->stream));
-  if (c->ibs_mode == 2) {
+  if (c->matrix_caches.ibs_mode == 2) {
     const uint32_t segs = ibs_repair_segments(c->n_dropped, c->N, n, c->sm_count);
     if (segs > 1 && pl.n_chunks == 1)      // plane 2 (J) is accumulated atomically then: clear it (the whole buffer is cleared when chunked)
       KGL_CUDA(c, cudaMemset2DAsync(c->d_ibs_acc.p + 2 * kIbsTileCells, (size_t)3 * kIbsTileCells * 4, 0, (size_t)kIbsTileCells * 4, n, c->stream));
@@ -1377,7 +1414,7 @@ int ibs_compute_tiles(kgl_b200_ctx* c, const TileList& list, bool want_blocks = 
 
 int ibs_finalize(kgl_b200_ctx* c, uint32_t n_tiles, int mode, uint64_t row_begin, uint64_t row_end, int mirror, uint32_t* d_out) {
   k_ibs_finalize<<<blocks_for((uint64_t)n_tiles * kIbsTileCells, 256), 256, 0, c->stream>>>(
-      c->d_ibs_acc.p, c->d_ibs_tiles.p, n_tiles, c->ibs_mode, c->ibs_mode == 2 ? c->d_dropped_seg.p : nullptr, (uint32_t)c->L, mode, c->N,
+      c->d_ibs_acc.p, c->d_ibs_tiles.p, n_tiles, c->matrix_caches.ibs_mode, c->matrix_caches.ibs_mode == 2 ? c->d_dropped_seg.p : nullptr, (uint32_t)c->L, mode, c->N,
       row_begin, row_end, mirror, d_out);
   KGL_LAUNCH_CHECK(c);
   return KGL_B200_OK;
@@ -1451,7 +1488,7 @@ int king_compute_tiles(kgl_b200_ctx* c, const TileList& list, KingTiles& K) {
   }
   K = KingTiles{};
   K.acc = c->d_ibs_acc.p; K.tiles = c->d_ibs_tiles.p; K.n_tiles = (uint32_t)list.key.n;
-  K.valid_mode = c->ibs_mode; K.seg = c->ibs_mode == 2 ? c->d_dropped_seg.p : nullptr; K.n_loci = (uint32_t)c->L; K.n_genomes = c->N;
+  K.valid_mode = c->matrix_caches.ibs_mode; K.seg = c->matrix_caches.ibs_mode == 2 ? c->d_dropped_seg.p : nullptr; K.n_loci = (uint32_t)c->L; K.n_genomes = c->N;
   K.hh = c->d_gram_hh.p; K.m = c->n_dropped > 0 ? c->d_king_m.p : nullptr; K.tile_block = c->d_ibs_tile_block.p; K.counts = c->d_ibs_class.p;
   return KGL_B200_OK;
 }
@@ -1470,17 +1507,6 @@ int sort_pair_keys(kgl_b200_ctx* c, uint64_t n, int end_bit) {
   return KGL_B200_OK;
 }
 
-// The first n records of `pairs` in the order sort_pair_keys left, through `sorted` to the host.
-template <class Pair>
-int fetch_sorted_pairs(kgl_b200_ctx* c, const DevBuf<Pair>& pairs, DevBuf<Pair>& sorted, uint64_t n, Pair* out) {
-  KGL_CUDA(c, sorted.ensure(n));
-  k_gather_pairs<<<blocks_for(n, 256), 256, 0, c->stream>>>(pairs.p, c->d_pair_index2.p, n, sorted.p);
-  KGL_LAUNCH_CHECK(c);
-  KGL_CUDA(c, cudaMemcpyAsync(out, sorted.p, n * sizeof(Pair), cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  return KGL_B200_OK;
-}
-
 // Bits of the sort key (hi << 32) | lo with hi < n.
 int pair_key_bits(uint64_t n) {
   int end_bit = 32;
@@ -1488,9 +1514,45 @@ int pair_key_bits(uint64_t n) {
   return end_bit;
 }
 
+// Sort keys and append positions for n pairs, and a zeroed append cursor: what the pair kernels write.
+int pair_keys_reset(kgl_b200_ctx* c, uint64_t n) {
+  KGL_CUDA(c, c->d_pair_keys.ensure(n));
+  KGL_CUDA(c, c->d_pair_index.ensure(n));
+  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
+  KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+  return KGL_B200_OK;
+}
+
+// A pair list for the host (KING, LD), before its kernels: room for dev_cap records -- no more than capacity or than the `cells`
+// the kernels look at, and indices that fit the uint32 sort values.
+template <class Pair>
+int pairs_begin(kgl_b200_ctx* c, DevBuf<Pair>& records, uint64_t capacity, uint64_t cells, uint64_t& dev_cap) {
+  dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, cells), 0xFFFFFFFFull);
+  KGL_CUDA(c, records.ensure(dev_cap));
+  return pair_keys_reset(c, dev_cap);
+}
+
+// ... and after them: *n_pairs = the pairs found, even when more than fit, then the records through `sorted` to the host in
+// ascending key order (hi << 32) | lo, hi < n_hi, whatever the order in which the warps appended them.
+template <class Pair>
+int pairs_end(kgl_b200_ctx* c, const DevBuf<Pair>& records, DevBuf<Pair>& sorted, uint64_t dev_cap, uint64_t n_hi, const char* what,
+              Pair* out, uint64_t* n_pairs) {
+  uint64_t n = 0;
+  int rc = read_counter(c, c->d_pair_cursor.p, n); if (rc) return rc;
+  *n_pairs = n;
+  if (n > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, std::string("more ") + what + " than capacity (*n_pairs holds the total)");
+  if (n == 0) return KGL_B200_OK;
+  rc = sort_pair_keys(c, n, pair_key_bits(n_hi)); if (rc) return rc;
+  KGL_CUDA(c, sorted.ensure(n));
+  k_gather_pairs<<<blocks_for(n, 256), 256, 0, c->stream>>>(records.p, c->d_pair_index2.p, n, sorted.p);
+  KGL_LAUNCH_CHECK(c);
+  KGL_CUDA(c, cudaMemcpyAsync(out, sorted.p, n * sizeof(Pair), cudaMemcpyDeviceToHost, c->stream));
+  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  return KGL_B200_OK;
+}
+
 int king_check(kgl_b200_ctx* c) {
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (c->L >= (1ull << 29)) return fail(c, KGL_B200_ERR_INVALID, "KING: more than 2^29 loci would overflow the int32 Gram accumulators");
   return ensure_ibs_planes(c);
 }
@@ -1501,7 +1563,7 @@ int king_check(kgl_b200_ctx* c) {
 // run (stride > 1), and kgl_b200_last_gram_kernel_ms times the launch alone, without that clear.
 int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
   int rc = ensure_codes(c); if (rc) return rc;
-  c->gram_valid = false;
+  c->matrix_caches.gram_valid = false;
   const uint64_t ld = gram_ld(c);
   if (c->gram_tiles_ld != ld || c->gram_first != first || c->gram_stride != stride) {
     const std::vector<uint2> all = gram_upper_tiles(ld);
@@ -1509,8 +1571,7 @@ int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
     for (uint64_t t = first; t < all.size(); t += stride) tiles.push_back(all[t]);
     if (tiles.empty()) tiles.push_back(all[0]);              // more ranks than tiles: nothing is launched (gram_n_tiles = 0)
     c->gram_first = first; c->gram_stride = stride;
-    KGL_CUDA(c, c->d_gram_tiles.ensure(tiles.size()));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_gram_tiles.p, tiles.data(), tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+    rc = upload(c, c->d_gram_tiles, tiles.data(), tiles.size()); if (rc) return rc;
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));
     c->gram_tiles_ld = ld; c->gram_n_tiles = first < all.size() ? tiles.size() : 0;
   }
@@ -1526,7 +1587,7 @@ int gram_compute(kgl_b200_ctx* c, uint64_t first = 0, uint64_t stride = 1) {
   KGL_CUDA(c, cudaEventRecord(c->gram_e0, c->stream));
   if (c->gram_n_tiles > 0) { KGL_CUDA(c, launch_gram(P, pl, c->stream)); ++c->launches; }
   KGL_CUDA(c, cudaEventRecord(c->gram_e1, c->stream));
-  c->gram_valid = true;
+  c->matrix_caches.gram_valid = true;
   return KGL_B200_OK;
 }
 
@@ -1539,6 +1600,13 @@ int default_superpop(kgl_b200_ctx* c) {
   return KGL_B200_OK;
 }
 
+// The raw counting pass of PCA, LD and QC: per-locus counts of all loci into d_pca_counts (d_locus_counts stays the caller's).
+int raw_locus_counts(kgl_b200_ctx* c) {
+  int rc = default_superpop(c); if (rc) return rc;
+  CountPass p{}; p.raw = p.locus_counts = true; p.counts = &c->d_pca_counts;
+  return launch_count(c, p);
+}
+
 // ---- genotype PCA (pca.cuh) ---------------------------------------------------------------------------------------------
 constexpr uint64_t kPcaSlabBytes = 1ull << 30;     // int32 outputs of one slab of pass-1 loci (both runs)
 // d_pca_stats: max bits and sums of the X block, of the W | V block, and |U|
@@ -1547,25 +1615,21 @@ constexpr size_t kPcaStatX = 0, kPcaStatXSum = kPcaMaxCols, kPcaStatWV = 2 * kPc
 
 // Loci-major codes of the pass-1 runs (K = genomes), once per upload.
 int ensure_codes_loci(kgl_b200_ctx* c) {
-  if (c->codes_loci_valid) return KGL_B200_OK;
+  if (c->matrix_caches.codes_loci_valid) return KGL_B200_OK;
   const uint64_t ks = (c->N + kGramK - 1) / kGramK, words = c->padded_rows * ks * 8;
   KGL_CUDA(c, c->d_codes_loci.ensure(words));
   k_codes16_loci<<<blocks_for(words, 256), 256, 0, c->stream>>>(reinterpret_cast<const uint32_t*>(c->d_packed.p), c->units, c->padded_rows, ks,
                                                                 c->d_codes_loci.p);
   KGL_LAUNCH_CHECK(c);
-  c->codes_loci_valid = true;
+  c->matrix_caches.codes_loci_valid = true;
   return KGL_B200_OK;
 }
 
 // p_l, d_l and the used loci for the keep mask (NULL = every locus) from one raw counting pass into d_pca_counts; m = |U|. PCA
 // and LD (whose eligible loci are PCA's used set).
 int pca_prepare(kgl_b200_ctx* c, const uint8_t* keep, uint64_t& m) {
-  int rc = default_superpop(c); if (rc) return rc;
-  rc = launch_count(c, true, true, false, false, false, nullptr, false, &c->d_pca_counts); if (rc) return rc;
-  if (keep) {
-    KGL_CUDA(c, c->d_pca_keep.ensure(c->L));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_keep.p, keep, c->L, cudaMemcpyHostToDevice, c->stream));
-  }
+  int rc = raw_locus_counts(c); if (rc) return rc;
+  if (keep) { rc = upload(c, c->d_pca_keep, keep, c->L); if (rc) return rc; }
   KGL_CUDA(c, c->d_pca_p.ensure(c->L));
   KGL_CUDA(c, c->d_pca_d.ensure(c->L));
   KGL_CUDA(c, c->d_pca_used.ensure(c->L));
@@ -1574,11 +1638,7 @@ int pca_prepare(kgl_b200_ctx* c, const uint8_t* keep, uint64_t& m) {
   k_pca_loci<<<blocks_for(c->L, 256), 256, 0, c->stream>>>(c->d_pca_counts.p, keep ? c->d_pca_keep.p : nullptr, c->L, c->d_pca_p.p, c->d_pca_d.p,
                                                            c->d_pca_used.p, c->d_pca_stats.p + kPcaStatUsed);
   KGL_LAUNCH_CHECK(c);
-  unsigned long long used = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&used, c->d_pca_stats.p + kPcaStatUsed, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  m = used;
-  return KGL_B200_OK;
+  return read_counter(c, c->d_pca_stats.p + kPcaStatUsed, m);
 }
 
 // Column maxima and digits of F [k_count][cols] into d_pca_digits (B operand of k_stages), sums next to the maxima.
@@ -1617,14 +1677,12 @@ int pca_apply(kgl_b200_ctx* c, uint32_t n_in, const double* x, double* y, double
   const uint32_t n2 = (uint32_t)(ldg / kGramM * nb);
   std::vector<double> xp((size_t)N * cols, 0.0);
   for (uint64_t g = 0; g < N; ++g) std::copy(x + g * n_in, x + (g + 1) * n_in, xp.begin() + g * cols);
-  KGL_CUDA(c, c->d_pca_tiles.ensure(tiles.size()));
-  KGL_CUDA(c, c->d_pca_x.ensure(xp.size()));
   if (loci_out) KGL_CUDA(c, c->d_pca_y.ensure((size_t)L * cols));
   else KGL_CUDA(c, c->d_pca_wv.ensure((size_t)L * 2 * cols));
   KGL_CUDA(c, c->d_pca_acc.ensure(std::max<uint64_t>(runs * slab * ld1, ldg * ld2)));
   KGL_CUDA(c, c->d_pca_out.ensure((size_t)N * cols));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_tiles.p, tiles.data(), tiles.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_pca_x.p, xp.data(), xp.size() * 8, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_pca_tiles, tiles.data(), tiles.size()); if (rc) return rc;
+  rc = upload(c, c->d_pca_x, xp.data(), xp.size()); if (rc) return rc;
   unsigned long long* st = c->d_pca_stats.p;
   int32_t* acc = c->d_pca_acc.p;
 
@@ -1684,15 +1742,14 @@ struct LdPlan {
 };
 
 int ld_prepare(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double threshold, LdPlan& P, LdTiles& T) {
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   const kgl_b200_ld_options opt = options ? *options : kgl_b200_ld_options{};
   if (std::isnan(threshold)) return fail(c, KGL_B200_ERR_INVALID, "LD: the r^2 threshold is NaN");
   if (opt.window_loci == 0 && opt.window_bp == 0) return fail(c, KGL_B200_ERR_INVALID, "LD: window_loci and window_bp are both 0");
   if (c->N >= (1ull << 25)) return fail(c, KGL_B200_ERR_INVALID, "LD: n_genomes must be < 2^25 (exact int64 -> double terms)");
   if (opt.window_bp != 0) {
-    if (!c->have_offsets || c->h_offsets.size() != c->L) return fail(c, KGL_B200_ERR_STATE, "LD: window_bp needs the locus offsets (kgl_b200_upload_loci)");
-    if (!std::is_sorted(c->h_offsets.begin(), c->h_offsets.end())) return fail(c, KGL_B200_ERR_INVALID, "LD: the locus offsets are not sorted");
+    rc = require_sorted_offsets(c, "LD: window_bp needs the locus offsets (kgl_b200_upload_loci)", "LD: the locus offsets are not sorted");
+    if (rc) return rc;
   }
   const uint64_t L = c->L;
   uint64_t m = 0;
@@ -1722,12 +1779,9 @@ int ld_prepare(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double thres
   }
   P.list_begin.push_back(list.size());
   rc = ensure_codes_loci(c); if (rc) return rc;
-  KGL_CUDA(c, c->d_ld_rank.ensure(L));
-  KGL_CUDA(c, c->d_ld_tiles.ensure(list.size()));
-  KGL_CUDA(c, c->d_ld_mirror.ensure(mirror.size()));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_rank.p, rank.data(), L * 4, cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_tiles.p, list.data(), list.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_ld_mirror.p, mirror.data(), mirror.size() * 4, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_ld_rank, rank.data(), L); if (rc) return rc;
+  rc = upload(c, c->d_ld_tiles, list.data(), list.size()); if (rc) return rc;
+  rc = upload(c, c->d_ld_mirror, mirror.data(), mirror.size()); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // pageable host memory
   T = LdTiles{};
   T.counts = c->d_pca_counts.p; T.rank = c->d_ld_rank.p; T.offsets = opt.window_bp ? c->d_offsets.p : nullptr;
@@ -1766,38 +1820,39 @@ int ld_slab_pairs(kgl_b200_ctx* c, const LdTiles& T, double threshold, int prune
 }
 
 // ---- population differentiation (fst.cuh) -------------------------------------------------------------------------------------
+// The groups of a per-group call: labels `group` with n_groups of 1..64 (0xFF = in no group), or NULL for the super-population
+// labels (KGL_B200_MAX_POP groups). G receives the number of groups. labels = false checks n_groups alone (kgl_b200_run_fst checks
+// its pairs against G before the labels).
+int check_groups(kgl_b200_ctx* c, const uint8_t* group, uint32_t n_groups, uint32_t& G, bool labels = true) {
+  G = group ? n_groups : KGL_B200_MAX_POP;
+  if (G == 0 || G > kGcMaxGroups) return fail(c, KGL_B200_ERR_INVALID, "n_groups must be 1..64");
+  if (!labels) return KGL_B200_OK;
+  if (!group) return c->have_superpop ? KGL_B200_OK : fail(c, KGL_B200_ERR_STATE, "group == NULL needs the super-population labels (kgl_b200_set_genome_superpop)");
+  for (uint64_t g = 0; g < c->N; ++g)
+    if (group[g] >= G && group[g] != 0xFF) return fail(c, KGL_B200_ERR_INVALID, "group label >= n_groups (0xFF = in no group)");
+  return KGL_B200_OK;
+}
+
 // Per-group counts of every locus into d_group_counts ([L][G] uint4) for labels `group` (NULL = the super-population labels, G =
 // KGL_B200_MAX_POP); G receives the number of groups.
 int group_counts_device(kgl_b200_ctx* c, uint32_t n_groups, const uint8_t* group, uint32_t& G) {
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
-  if (!group) {
-    if (!c->have_superpop) return fail(c, KGL_B200_ERR_STATE, "group == NULL needs the super-population labels (kgl_b200_set_genome_superpop)");
-    n_groups = KGL_B200_MAX_POP;
-  } else {
-    if (n_groups == 0 || n_groups > kGcMaxGroups) return fail(c, KGL_B200_ERR_INVALID, "n_groups must be 1..64");
-    for (uint64_t g = 0; g < c->N; ++g)
-      if (group[g] >= n_groups && group[g] != 0xFF) return fail(c, KGL_B200_ERR_INVALID, "group label >= n_groups (0xFF = in no group)");
-  }
-  G = n_groups;
+  int rc = use_population(c, false); if (rc) return rc;
+  rc = check_groups(c, group, n_groups, G); if (rc) return rc;
   if (group || !c->gc_superpop) {
-    const GroupTable T = build_group_table(group ? group : c->h_superpop.data(), c->N, c->host_units, n_groups);
-    KGL_CUDA(c, c->d_gc_entries.ensure(T.entries.size()));
-    KGL_CUDA(c, c->d_gc_chunk.ensure(T.chunk_begin.size()));
-    KGL_CUDA(c, c->d_gc_size.ensure(T.size.size()));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_entries.p, T.entries.data(), T.entries.size() * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_chunk.p, T.chunk_begin.data(), T.chunk_begin.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_gc_size.p, T.size.data(), T.size.size() * 4, cudaMemcpyHostToDevice, c->stream));
+    const GroupTable T = build_group_table(group ? group : c->h_superpop.data(), c->N, c->host_units, G);
+    rc = upload(c, c->d_gc_entries, T.entries.data(), T.entries.size()); if (rc) return rc;
+    rc = upload(c, c->d_gc_chunk, T.chunk_begin.data(), T.chunk_begin.size()); if (rc) return rc;
+    rc = upload(c, c->d_gc_size, T.size.data(), T.size.size()); if (rc) return rc;
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));       // pageable host memory
     c->gc_superpop = group == nullptr;
   }
-  KGL_CUDA(c, c->d_group_counts.ensure((size_t)c->L * n_groups));
+  KGL_CUDA(c, c->d_group_counts.ensure((size_t)c->L * G));
   GroupCountParams P{};
   P.packed = reinterpret_cast<const uint4*>(c->d_packed.p); P.pitch = c->units; P.n_loci = c->L;
-  P.n_tiles = (c->L + kGcRows - 1) / kGcRows; P.units = (uint32_t)c->host_units; P.n_groups = n_groups;
+  P.n_tiles = (c->L + kGcRows - 1) / kGcRows; P.units = (uint32_t)c->host_units; P.n_groups = G;
   P.n_chunks = (uint32_t)((c->host_units + kGcChunkUnits - 1) / kGcChunkUnits);
   P.entries = c->d_gc_entries.p; P.chunk_begin = c->d_gc_chunk.p; P.size = c->d_gc_size.p; P.counts = c->d_group_counts.p;
-  const size_t smem = group_counts_smem(n_groups);
+  const size_t smem = group_counts_smem(G);
   KGL_CUDA(c, cudaFuncSetAttribute(k_group_counts, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   KGL_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_group_counts, kGcThreads, smem));
@@ -1824,11 +1879,10 @@ int hwe_multi_flags(kgl_b200_ctx* c, const uint8_t*& flags) {
 // the group counts, the cells ordered by walk length, the walk. G receives the number of groups.
 int hardy_device(kgl_b200_ctx* c, const uint8_t* group, uint32_t n_groups, uint32_t midp, bool want_f, uint32_t& G) {
   if (midp > 1) return fail(c, KGL_B200_ERR_INVALID, "midp must be 0 or 1");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (c->N >= kHweMaxGenomes) {              // v < 2^25 keeps every integer of the recurrence exact in double
+    if (!group) { rc = check_groups(c, group, n_groups, G); if (rc) return rc; }     // the super-population labels are read here
     const uint8_t* lab = group ? group : c->h_superpop.data();
-    if (!group && !c->have_superpop) return fail(c, KGL_B200_ERR_STATE, "group == NULL needs the super-population labels (kgl_b200_set_genome_superpop)");
     std::vector<uint64_t> size(256, 0);
     for (uint64_t g = 0; g < c->N; ++g) ++size[lab[g]];
     for (int k = 0; k < 255; ++k)
@@ -1971,14 +2025,12 @@ static int set_shape(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_loci, uint6
   if (row_bytes != 16 * ((n_genomes + 63) / 64)) return fail(c, KGL_B200_ERR_INVALID, "row_bytes must be 16*ceil(n_genomes/64)");
   if (n_genomes >= (1ull << 32) || n_loci >= (1ull << 32)) return fail(c, KGL_B200_ERR_INVALID, "dimension too large");
   // A matrix of a different shape starts a new population: stale loci / super-populations must be uploaded again
-  // (require_population reports what is missing at run time).
-  if (c->have_loci && c->loci_len != n_loci) { c->have_loci = false; c->prep_valid = false; }
+  // (use_population reports what is missing at run time).
+  if (c->have_loci && c->loci_len != n_loci) c->have_loci = false;
   if (c->have_superpop && c->h_superpop.size() != n_genomes) c->have_superpop = false;
   c->N = n_genomes; c->L = n_loci; c->row_bytes = row_bytes; c->host_units = row_bytes / 16;
-  c->n_multi = 0;                    // the side cells belong to the matrix: kgl_b200_upload_multi_allelic comes after it
   c->units = stream_units_padded(c->host_units); c->Npad = c->units * 64;
-  c->sm_valid = false; c->codes_valid = false; c->units_valid = false; c->dropped_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->ibs_mode = -1; c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0; c->ibs_class_valid = false;
-  c->codes16_valid = false; c->gram_valid = false; c->codes_loci_valid = false; c->gc_superpop = false;
+  matrix_changed(c);                 // also drops the side cells: kgl_b200_upload_multi_allelic comes after the matrix
   return KGL_B200_OK;
 }
 
@@ -2020,9 +2072,8 @@ int kgl_b200_upload_genotypes(kgl_b200_ctx* c, uint64_t n_genomes, uint64_t n_lo
     KGL_CUDA(c, cudaStreamWaitEvent(c->stream, c->chunk_ev[ci], 0));
     rc = launch_dropped_index(c, r0 * c->units, rows * c->units, cap); if (rc) return rc;
   }
-  unsigned long long total = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_dropped_counter.p + 1, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));      // every chunk has landed: the host buffer is free again
+  uint64_t total = 0;
+  rc = read_counter(c, c->d_dropped_counter.p + 1, total); if (rc) return rc;      // every chunk has landed: the host buffer is free again
   if (total > cap && total <= limit) {
     KGL_CUDA(c, c->d_dropped_unsorted.ensure(total));
     KGL_CUDA(c, cudaMemsetAsync(c->d_dropped_counter.p, 0, 16, c->stream));
@@ -2040,20 +2091,19 @@ int kgl_b200_upload_loci(kgl_b200_ctx* c, uint64_t n_loci, uint32_t n_pop, const
   c->have_offsets = offsets != nullptr; c->loci_len = n_loci;
   c->n_pop = n_pop;
   if (!c->have_geno) c->L = n_loci;
-  KGL_CUDA(c, c->d_af.ensure((size_t)n_pop * n_loci));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_af.p, af, (size_t)n_pop * n_loci * 4, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_af, af, (size_t)n_pop * n_loci); if (rc) return rc;
   if (offsets) {
-    KGL_CUDA(c, c->d_offsets.ensure(n_loci));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_offsets.p, offsets, n_loci * 4, cudaMemcpyHostToDevice, c->stream));
+    rc = upload(c, c->d_offsets, offsets, n_loci); if (rc) return rc;
     c->h_offsets.assign(offsets, offsets + n_loci);
   }
   c->sel_row_lo = 0; c->sel_row_hi = ~0ull;
   KGL_CUDA(c, c->d_sel.ensure(n_loci));
   KGL_CUDA(c, cudaMemsetAsync(c->d_sel.p, 0, n_loci, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  c->have_loci = true; c->prep_valid = false; c->dropped_cells_state = 0;
-  c->n_multi = 0;                    // ... and after the frequency table
-  c->keep_valid = false;
+  c->have_loci = true;
+  frequencies_changed(c);
+  multi_changed(c);                  // ... and after the frequency table
+  filter_changed(c);
   return KGL_B200_OK;
 }
 
@@ -2064,10 +2114,10 @@ int kgl_b200_set_genome_superpop(kgl_b200_ctx* c, uint64_t n_genomes, const uint
     if (superpop[g] >= KGL_B200_MAX_POP) return fail(c, KGL_B200_ERR_INVALID, "super-population index must be 0..5");
   int rc = use_device(c); if (rc) return rc;
   c->h_superpop.assign(superpop, superpop + n_genomes);
-  KGL_CUDA(c, c->d_superpop.ensure(n_genomes));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_superpop.p, superpop, n_genomes, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_superpop, superpop, n_genomes); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  c->have_superpop = true; c->units_valid = false; c->dropped_cells_state = 0; c->prep_valid = false; c->gc_superpop = false;
+  c->have_superpop = true;
+  labels_changed(c);
   if (!c->have_geno) c->N = n_genomes;
   return KGL_B200_OK;
 }
@@ -2077,21 +2127,19 @@ int kgl_b200_upload_multi_allelic(kgl_b200_ctx* c, uint64_t n_multi, const uint3
   int rc = use_device(c); if (rc) return rc;
   if (!c->have_geno || !c->have_loci || c->loci_len != c->L)
     return fail(c, KGL_B200_ERR_STATE, "upload the genotype matrix and the allele frequencies before the multi-allelic loci");
-  c->n_multi = 0; c->prep_valid = false;
+  multi_changed(c);
   if (n_multi == 0) return KGL_B200_OK;
   if (!rows || !af || !cells) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   for (uint64_t m = 0; m < n_multi; ++m)
     if (rows[m] >= c->L || (m > 0 && rows[m] <= rows[m - 1])) return fail(c, KGL_B200_ERR_INVALID, "multi-allelic rows must be ascending rows of the locus table");
-  KGL_CUDA(c, c->d_multi_rows.ensure(n_multi));
-  KGL_CUDA(c, c->d_multi_af.ensure((size_t)c->n_pop * n_multi * kMultiSlots));
-  KGL_CUDA(c, c->d_multi_cells.ensure((size_t)n_multi * c->N));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_multi_rows.p, rows, n_multi * 4, cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_multi_af.p, af, (size_t)c->n_pop * n_multi * kMultiSlots * 4, cudaMemcpyHostToDevice, c->stream));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_multi_cells.p, cells, (size_t)n_multi * c->N, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_multi_rows, rows, n_multi); if (rc) return rc;
+  rc = upload(c, c->d_multi_af, af, (size_t)c->n_pop * n_multi * kMultiSlots); if (rc) return rc;
+  rc = upload(c, c->d_multi_cells, cells, (size_t)n_multi * c->N); if (rc) return rc;
   k_multi_mask_af<<<blocks_for(n_multi * c->n_pop, 128), 128, 0, c->stream>>>(c->d_multi_rows.p, n_multi, (int)c->n_pop, c->L, c->d_af.p);
   KGL_LAUNCH_CHECK(c);
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  c->n_multi = n_multi; c->dropped_cells_state = 0;
+  c->n_multi = n_multi;
+  frequencies_changed(c);            // their rows of the frequency table now hold "no value"
   return KGL_B200_OK;
 }
 
@@ -2109,7 +2157,7 @@ int kgl_b200_run_multi_allele_count(kgl_b200_ctx* c, uint32_t* counts) {
 
 int kgl_b200_set_unphased(kgl_b200_ctx* c, int unphased) {
   if (!c) return KGL_B200_ERR_INVALID;
-  if (c->unphased != (unphased != 0)) c->mom_valid = false;
+  if (c->unphased != (unphased != 0)) phase_changed(c);
   c->unphased = unphased != 0;
   return KGL_B200_OK;
 }
@@ -2122,7 +2170,7 @@ int kgl_b200_set_locus_selection(kgl_b200_ctx* c, uint64_t n_loci, const uint8_t
   c->sel_row_lo = 0; c->sel_row_hi = ~0ull;
   KGL_CUDA(c, cudaMemcpyAsync(c->d_sel.p, selected, n_loci, cudaMemcpyHostToDevice, c->stream));
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  c->prep_valid = false;
+  selection_changed(c);
   return KGL_B200_OK;
 }
 
@@ -2197,7 +2245,8 @@ int kgl_b200_select_loci(kgl_b200_ctx* c, uint64_t lower, uint64_t upper, uint64
       KGL_LAUNCH_CHECK(c);
     }
   }
-  c->prep_valid = false; c->inputs_async = true;
+  selection_changed(c);
+  c->inputs_async = true;
   if (n_selected) {
     unsigned long long counts[kMaxPop];
     KGL_CUDA(c, cudaMemcpyAsync(counts, c->d_sel_counts.p, kMaxPop * 8, cudaMemcpyDeviceToHost, c->stream));
@@ -2211,11 +2260,10 @@ int kgl_b200_set_locus_filter(kgl_b200_ctx* c, uint64_t n_loci, const uint8_t* k
   if (!c) return KGL_B200_ERR_INVALID;
   if (!c->have_loci) return fail(c, KGL_B200_ERR_STATE, "upload_loci first");
   int rc = use_device(c); if (rc) return rc;
-  c->keep_valid = false; c->prep_valid = false;
+  filter_changed(c);
   if (!keep) return KGL_B200_OK;
   if (n_loci != c->loci_len) return fail(c, KGL_B200_ERR_INVALID, "filter length differs from n_loci");
-  KGL_CUDA(c, c->d_locus_keep.ensure(n_loci));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_locus_keep.p, keep, n_loci, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_locus_keep, keep, n_loci); if (rc) return rc;
   KGL_CUDA(c, cudaStreamSynchronize(c->stream));
   c->keep_valid = true;
   return KGL_B200_OK;
@@ -2265,8 +2313,7 @@ int kgl_b200_synth_genotypes(kgl_b200_ctx* c, uint64_t seed, uint64_t n_genomes,
   rc = set_shape(c, n_genomes, n_loci, row_bytes);
   if (rc) return rc;
   rc = alloc_matrix(c); if (rc) return rc;
-  KGL_CUDA(c, c->d_inbreeding.ensure(n_genomes));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_inbreeding.p, inbreeding, n_genomes * 8, cudaMemcpyHostToDevice, c->stream));
+  rc = upload(c, c->d_inbreeding, inbreeding, n_genomes); if (rc) return rc;
   const uint64_t total = n_loci * c->units;
   k_synth<<<blocks_for(total, 256), 256, 0, c->stream>>>(seed, n_genomes, n_loci, locus_base, c->units, c->d_af.p, c->d_superpop.p,
                                                         c->d_inbreeding.p, (uint64_t)(missing_rate * 16777216.0),
@@ -2288,11 +2335,11 @@ int kgl_b200_download_genotypes(kgl_b200_ctx* c, uint64_t n_bytes, void* packed)
 
 int kgl_b200_run_allele_count(kgl_b200_ctx* c, uint32_t* locus_counts, uint64_t* genome_counts) {
   if (!c) return KGL_B200_ERR_INVALID;
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   rc = default_superpop(c); if (rc) return rc;
   if (genome_counts) KGL_CUDA(c, c->d_genome_counts.ensure((size_t)c->N * 4));
-  rc = launch_count(c, true, locus_counts != nullptr, genome_counts != nullptr); if (rc) return rc;
+  CountPass p{}; p.raw = true; p.locus_counts = locus_counts != nullptr; p.genome = genome_counts != nullptr;
+  rc = launch_count(c, p); if (rc) return rc;
   if (locus_counts)
     KGL_CUDA(c, cudaMemcpyAsync(locus_counts, c->d_locus_counts.p, (size_t)c->L * 16, cudaMemcpyDeviceToHost, c->stream));
   if (genome_counts) {
@@ -2306,10 +2353,10 @@ int kgl_b200_run_allele_count(kgl_b200_ctx* c, uint32_t* locus_counts, uint64_t*
 
 int kgl_b200_run_hetero_homo(kgl_b200_ctx* c, int other_allele_entries, uint64_t* out) {
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   rc = default_superpop(c); if (rc) return rc;
-  rc = launch_count(c, true, false, true); if (rc) return rc;
+  CountPass p{}; p.raw = p.genome = true;
+  rc = launch_count(c, p); if (rc) return rc;
   KGL_CUDA(c, c->d_genome_counts.ensure((size_t)c->N * 7));
   k_hetero_homo<<<blocks_for(c->N, 128), 128, 0, c->stream>>>(c->d_gcounts, c->d_n3, c->n_multi ? c->d_multi_cells.p : nullptr, c->n_multi, c->N,
                                                               other_allele_entries ? 1u : 0u, c->d_genome_counts.p);
@@ -2356,8 +2403,7 @@ int kgl_b200_location_fis(uint64_t n_genomes, const uint64_t* hetero_homo, uint3
 
 int kgl_b200_enqueue_count_and_inbreed(kgl_b200_ctx* c) {
   if (!c) return KGL_B200_ERR_INVALID;
-  int rc = use_device(c, false); if (rc) return rc;      // the tail of the pass before may still be running: it is not waited for
-  rc = require_population(c, true); if (rc) return rc;
+  int rc = use_population(c, true, false); if (rc) return rc;      // the tail of the pass before may still be running: it is not waited for
   c->prep_valid = false;   // the AF vectors are an input of the pass: the per-locus preparation is part of every step
   c->peer_results = false;
   KGL_CUDA(c, c->d_results.ensure(c->Npad));
@@ -2446,8 +2492,7 @@ int kgl_b200_peer_set_timeout_ms(kgl_b200_ctx* c, uint64_t milliseconds) {
 
 int kgl_b200_enqueue_count_and_inbreed_peer(kgl_b200_ctx* c) {
   if (!c) return KGL_B200_ERR_INVALID;
-  int rc = use_device(c, false); if (rc) return rc;
-  rc = require_population(c, true); if (rc) return rc;
+  int rc = use_population(c, true, false); if (rc) return rc;
   if (c->peer_world == 0 || c->xchg_npad != c->Npad) return fail(c, KGL_B200_ERR_STATE, "kgl_b200_peer_export / kgl_b200_peer_attach first");
   c->prep_valid = false;   // the AF vectors are an input of the pass, as in kgl_b200_enqueue_count_and_inbreed
   KGL_CUDA(c, c->d_results.ensure(c->Npad));
@@ -2515,8 +2560,7 @@ int kgl_b200_run_count_and_inbreed(kgl_b200_ctx* c, uint32_t* locus_counts, kgl_
 int kgl_b200_inbreed_begin(kgl_b200_ctx* c, int algorithm, const kgl_b200_inbreed_options* options) {
   if (!c) return KGL_B200_ERR_INVALID;
   if (algorithm < KGL_B200_ALGO_SIMPLE || algorithm > KGL_B200_ALGO_LOGLIKELIHOOD) return fail(c, KGL_B200_ERR_INVALID, "unknown algorithm");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, true); if (rc) return rc;
+  int rc = use_population(c, true); if (rc) return rc;
   c->algo = algorithm; c->phase = 0; c->iteration = 0; c->peer_results = false;
   c->opt = options ? *options : kgl_b200_inbreed_options{};
   c->hall_start.clear();
@@ -2637,14 +2681,13 @@ int kgl_b200_inbreed_update(kgl_b200_ctx* c, int* finished) {
   }
   // the update kernels read the (all-reduced) moments from d_partials and the (all-reduced) iteration terms from d_iter
   KGL_CUDA(c, cudaMemsetAsync(c->d_flag.p, 0, 8, c->stream));
-  unsigned long long flag = 0;
+  uint64_t flag = 0;
   if (c->algo == KGL_B200_ALGO_HALLME) {
     ++c->iteration;
     k_hall_update<<<nb, 256, 0, c->stream>>>(c->d_partials.p, c->d_iter.p, c->N, c->d_f.p, c->d_flag.p);
     KGL_LAUNCH_CHECK(c);
     if (c->opt.hall_sweeps > 0) { *finished = (c->iteration >= c->opt.hall_sweeps) ? 1 : 0; return KGL_B200_OK; }
-    KGL_CUDA(c, cudaMemcpyAsync(&flag, c->d_flag.p, 8, cudaMemcpyDeviceToHost, c->stream));
-    KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+    rc = read_counter(c, c->d_flag.p, flag); if (rc) return rc;
     double max_delta; std::memcpy(&max_delta, &flag, 8);
     *finished = (max_delta < 1e-15 || c->iteration >= 100000) ? 1 : 0;
     return KGL_B200_OK;
@@ -2660,8 +2703,7 @@ int kgl_b200_inbreed_update(kgl_b200_ctx* c, int* finished) {
     KGL_LAUNCH_CHECK(c);
     return KGL_B200_OK;
   }
-  KGL_CUDA(c, cudaMemcpyAsync(&flag, c->d_flag.p, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  rc = read_counter(c, c->d_flag.p, flag); if (rc) return rc;
   *finished = (flag == 0 || c->iteration >= c->opt.ll_max_iterations) ? 1 : 0;
   // flag = genomes still searching. Once they are a minority the sweeps gather them through a list: the work of a sweep
   // follows the number of live genomes, not N (every rank sees the same done flags, so the same list).
@@ -2714,9 +2756,8 @@ static int run_whole_from_tables(kgl_b200_ctx* c, int* finished) {
   KGL_CUDA(c, cudaFuncSetAttribute(k_mom_run<FAST_NEWTON>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_mom_run<FAST_NEWTON><<<(unsigned)c->N, kMomRunThreads, smem, c->stream>>>(P);
   KGL_LAUNCH_CHECK(c);
-  unsigned long long remaining = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&remaining, c->d_flag.p, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+  uint64_t remaining = 0;
+  rc = read_counter(c, c->d_flag.p, remaining); if (rc) return rc;
   *finished = remaining == 0 ? 1 : 0;
   return KGL_B200_OK;
 }
@@ -2737,8 +2778,7 @@ int kgl_b200_run_inbreed(kgl_b200_ctx* c, int algorithm, const kgl_b200_inbreed_
 
 int kgl_b200_run_loglik_grid(kgl_b200_ctx* c, const double* grid, uint64_t n_grid, double* out) {
   if (!c || !grid || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, true); if (rc) return rc;
+  int rc = use_population(c, true); if (rc) return rc;
   rc = ensure_prepared(c, false, true); if (rc) return rc;
   KGL_CUDA(c, c->d_grid.ensure(kGridMax));
   // Sums the n_chunks chunk outputs at src ([n_chunks][Npad][kGridMax]) of every genome and of grid points g0 .. g0 + ng - 1 on
@@ -2775,8 +2815,7 @@ int kgl_b200_run_loglik_grid(kgl_b200_ctx* c, const double* grid, uint64_t n_gri
 
 int kgl_b200_run_ibs(kgl_b200_ctx* c, uint64_t row_begin, uint64_t row_end, uint32_t* out) {
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (row_begin >= row_end || row_end > c->N) return fail(c, KGL_B200_ERR_INVALID, "bad genome row range");
   rc = ensure_ibs_planes(c); if (rc) return rc;
   return run_pairwise(c, row_begin, row_end, 4, c->d_ibs, out, [c](const TileList& tiles, uint64_t r0, uint64_t r1, int mirror) {
@@ -2815,13 +2854,8 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
       rc = listed_tiles(c, coords + 2 * t0, n, true, slabs.back()); if (rc) return rc;
     }
   }
-  // device list: no more records than the tiles hold, and indices that fit the uint32 sort values
-  const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, n_tiles * kIbsTileCells), 0xFFFFFFFFull);
-  KGL_CUDA(c, c->d_king_pairs.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_keys.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_index.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
-  KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+  uint64_t dev_cap = 0;
+  rc = pairs_begin(c, c->d_king_pairs, capacity, n_tiles * kIbsTileCells, dev_cap); if (rc) return rc;
   KingTiles K{};
   for (const TileList& tiles : slabs) {
     rc = king_compute_tiles(c, tiles, K); if (rc) return rc;
@@ -2829,21 +2863,13 @@ int kgl_b200_run_king_pairs(kgl_b200_ctx* c, uint64_t n_coords, const uint32_t* 
                                                                                                c->d_pair_keys.p, c->d_pair_index.p, c->d_pair_cursor.p);
     KGL_LAUNCH_CHECK(c);
   }
-  unsigned long long total = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  *n_pairs = total;
-  if (total > capacity || total > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, "more related pairs than capacity (*n_pairs holds the total)");
-  if (total == 0) return KGL_B200_OK;
-  // ascending (a, b) whatever the order in which the warps appended
-  rc = sort_pair_keys(c, total, pair_key_bits(c->N)); if (rc) return rc;
-  return fetch_sorted_pairs(c, c->d_king_pairs, c->d_king_sorted, total, pairs);
+  return pairs_end(c, c->d_king_pairs, c->d_king_sorted, dev_cap, c->N, "related pairs", pairs, n_pairs);
 }
 
 int kgl_b200_set_ibs_tensor_cores(kgl_b200_ctx* c, int enable) {
   if (!c) return KGL_B200_ERR_INVALID;
   c->ibs_tensor_enabled = enable != 0;
-  c->ibs_tiles_key = TileKey{}; c->ibs_n_blocks = 0;         // the cached tile list carries no block list for the other form
+  ibs_form_changed(c);
   return KGL_B200_OK;
 }
 
@@ -2860,8 +2886,7 @@ int kgl_b200_ibs_tile_grid(kgl_b200_ctx* c, uint64_t* tiles_per_side, uint64_t* 
 
 int kgl_b200_enqueue_ibs_tiles(kgl_b200_ctx* c, uint64_t first, uint64_t stride, uint64_t count) {
   if (!c) return KGL_B200_ERR_INVALID;
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   const uint64_t side = ibs_side(c), n_upper = side * (side + 1) / 2;
   if (stride == 0 || count == 0 || count > kIbsMaxTilesPerLaunch || first + (count - 1) * stride >= n_upper)
     return fail(c, KGL_B200_ERR_INVALID, "bad tile range (count must be 1..8192 per call and stay inside the upper triangle)");
@@ -2871,8 +2896,7 @@ int kgl_b200_enqueue_ibs_tiles(kgl_b200_ctx* c, uint64_t first, uint64_t stride,
 
 int kgl_b200_enqueue_ibs_tile_list(kgl_b200_ctx* c, uint64_t count, const uint32_t* coords) {
   if (!c || !coords) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (count == 0 || count > kIbsMaxTilesPerLaunch) return fail(c, KGL_B200_ERR_INVALID, "bad tile count (1..8192 per call)");
   TileList tiles;
   rc = listed_tiles(c, coords, count, false, tiles); if (rc) return rc;
@@ -2915,8 +2939,7 @@ int kgl_b200_ibs_timer_read(kgl_b200_ctx* c, float* ms, uint32_t capacity, uint3
 int kgl_b200_enqueue_gram_tiles(kgl_b200_ctx* c, uint64_t first, uint64_t stride) {
   if (!c) return KGL_B200_ERR_INVALID;
   if (stride == 0 || first >= stride) return fail(c, KGL_B200_ERR_INVALID, "need first < stride");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (c->L >= (1ull << 29)) return fail(c, KGL_B200_ERR_INVALID, "Gram matrix: more than 2^29 loci would overflow the int32 accumulators");
   return gram_compute(c, first, stride);
 }
@@ -2925,7 +2948,7 @@ int kgl_b200_enqueue_gram(kgl_b200_ctx* c) { return kgl_b200_enqueue_gram_tiles(
 
 int kgl_b200_gram_buffer(kgl_b200_ctx* c, void** device_ptr, uint64_t* n_int32, uint64_t* ld) {
   if (!c || !device_ptr || !n_int32) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  if (!c->gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
+  if (!c->matrix_caches.gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
   *device_ptr = c->d_gram.p; *n_int32 = gram_ld(c) * gram_ld(c);
   if (ld) *ld = gram_ld(c);
   return KGL_B200_OK;
@@ -2933,7 +2956,7 @@ int kgl_b200_gram_buffer(kgl_b200_ctx* c, void** device_ptr, uint64_t* n_int32, 
 
 int kgl_b200_fetch_gram(kgl_b200_ctx* c, int32_t* out) {
   if (!c || !out) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  if (!c->gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
+  if (!c->matrix_caches.gram_valid) return fail(c, KGL_B200_ERR_STATE, "enqueue_gram first");
   int rc = use_device(c); if (rc) return rc;
   const size_t n2 = (size_t)c->N * c->N;
   KGL_CUDA(c, c->d_gram_out.ensure(n2 * 4));
@@ -2980,12 +3003,12 @@ int kgl_b200_run_grm(kgl_b200_ctx* c, uint32_t pop, double* out) {
 int kgl_b200_run_binned_genome_counts(kgl_b200_ctx* c, uint32_t pop, uint32_t n_bins, const double* lower, const double* upper,
                                       int present_only, uint64_t* genome_counts, uint64_t* bin_rows) {
   if (!c || !lower || !upper || !genome_counts || n_bins == 0) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (!c->have_loci || c->loci_len != c->L) return fail(c, KGL_B200_ERR_STATE, "AF bins need the allele frequencies (kgl_b200_upload_loci)");
   if (pop >= c->n_pop) return fail(c, KGL_B200_ERR_INVALID, "population index out of range");
   // "variants of the population" = rows carried by at least one genome: needs the per-locus counts of a raw pass
-  if (present_only) { rc = launch_count(c, true, true, false); if (rc) return rc; }
+  CountPass p{}; p.raw = p.locus_counts = true;
+  if (present_only) { rc = launch_count(c, p); if (rc) return rc; }
   if (c->n_multi && present_only) {      // which alleles of the multi-allelic loci occur
     KGL_CUDA(c, c->d_multi_counts.ensure(c->n_multi * kMultiSlots * 3));
     k_multi_allele_count<<<(unsigned)c->n_multi, 256, 0, c->stream>>>(c->d_multi_cells.p, c->N, c->d_multi_counts.p);
@@ -2995,12 +3018,10 @@ int kgl_b200_run_binned_genome_counts(kgl_b200_ctx* c, uint32_t pop, uint32_t n_
     std::vector<uint32_t> pm(c->units * 2, 0);
     for (uint64_t g = 0; g < c->N; ++g) pm[g >> 5] |= 1u << (g & 31);
     std::vector<uint8_t> need(c->units * 2, 1);
-    KGL_CUDA(c, c->d_bin_popmask32.ensure(pm.size()));
-    KGL_CUDA(c, c->d_bin_need32.ensure(need.size()));
     KGL_CUDA(c, c->d_zero_superpop.ensure(c->Npad));
     KGL_CUDA(c, c->d_bin_state.ensure(2));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_bin_popmask32.p, pm.data(), pm.size() * 4, cudaMemcpyHostToDevice, c->stream));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_bin_need32.p, need.data(), need.size(), cudaMemcpyHostToDevice, c->stream));
+    rc = upload(c, c->d_bin_popmask32, pm.data(), pm.size()); if (rc) return rc;
+    rc = upload(c, c->d_bin_need32, need.data(), need.size()); if (rc) return rc;
     KGL_CUDA(c, cudaMemsetAsync(c->d_zero_superpop.p, 0, c->Npad, c->stream));
     KGL_CUDA(c, cudaStreamSynchronize(c->stream));
     c->bin_tables_n = c->N; c->bin_tables_units = c->units;
@@ -3009,13 +3030,14 @@ int kgl_b200_run_binned_genome_counts(kgl_b200_ctx* c, uint32_t pop, uint32_t n_
   KGL_CUDA(c, c->d_bin_sum64.ensure(c->padded_rows / 64));
   KGL_CUDA(c, c->d_bin_out.ensure((size_t)n_bins * c->N * 4 + n_bins));
   const MaskOverride mo{c->d_bin_flags.p, c->d_bin_sum64.p, c->d_bin_popmask32.p, c->d_bin_need32.p, c->d_zero_superpop.p};
+  CountPass bin{}; bin.genome = true; bin.mask = &mo;
   for (uint32_t b = 0; b < n_bins; ++b) {
     KGL_CUDA(c, cudaMemsetAsync(c->d_bin_state.p, 0, 8, c->stream));
     k_bin_flags<<<blocks_for(c->padded_rows, 256), 256, 0, c->stream>>>(c->d_af.p + (size_t)pop * c->L, present_only ? c->d_locus_counts.p : nullptr,
                                                                          c->L, c->padded_rows, lower[b], upper[b], c->keep_valid ? c->d_locus_keep.p : nullptr,
                                                                          c->d_bin_flags.p, c->d_bin_sum64.p, c->d_bin_state.p + 1);
     KGL_LAUNCH_CHECK(c);
-    rc = launch_count(c, false, false, true, false, false, &mo); if (rc) return rc;
+    rc = launch_count(c, bin); if (rc) return rc;
     k_genome_counts_masked<<<blocks_for(c->N, 256), 256, 0, c->stream>>>(c->d_gcounts, c->d_n3, c->N, c->d_bin_state.p + 1,
                                                                          c->d_bin_out.p + (size_t)b * c->N * 4, c->d_bin_out.p + (size_t)n_bins * c->N * 4 + b);
     KGL_LAUNCH_CHECK(c);
@@ -3035,8 +3057,7 @@ int kgl_b200_run_binned_genome_counts(kgl_b200_ctx* c, uint32_t pop, uint32_t n_
 
 int kgl_b200_run_grm_product(kgl_b200_ctx* c, const uint8_t* keep, uint32_t n_cols, const double* x, double* y, uint64_t* n_loci_used) {
   if (!c || !x || !y) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   if (n_cols == 0 || n_cols > (uint32_t)kPcaMaxCols) return fail(c, KGL_B200_ERR_INVALID, "n_cols must be 1..48");
   if (c->L >= (1ull << 28)) return fail(c, KGL_B200_ERR_INVALID, "PCA: n_loci must be < 2^28 (int32 digit accumulators)");
   uint64_t m = 0;
@@ -3050,8 +3071,7 @@ int kgl_b200_run_grm_product(kgl_b200_ctx* c, const uint8_t* keep, uint32_t n_co
 int kgl_b200_run_pca(kgl_b200_ctx* c, const kgl_b200_pca_options* options, double* eigenvalues, double* scores, double* loadings,
                      uint64_t* n_loci_used) {
   if (!c || !eigenvalues || !scores) return fail(c, KGL_B200_ERR_INVALID, "null argument");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   const kgl_b200_pca_options opt = options ? *options : kgl_b200_pca_options{};
   const uint32_t k = opt.n_components ? opt.n_components : 10, q = opt.iterations ? opt.iterations : 10;
   const uint64_t N = c->N, L = c->L;
@@ -3118,26 +3138,13 @@ int kgl_b200_run_ld_pairs(kgl_b200_ctx* c, const kgl_b200_ld_options* options, d
   LdPlan P;
   LdTiles T{};
   int rc = ld_prepare(c, options, min_r2, P, T); if (rc) return rc;
-  // device list: no more records than the band's cells, and indices that fit the uint32 sort values
-  const uint64_t cells = (uint64_t)P.band.tiles.size() * kGramM * kGramN;
-  const uint64_t dev_cap = std::min<uint64_t>(std::min<uint64_t>(capacity, cells), 0xFFFFFFFFull);
-  KGL_CUDA(c, c->d_ld_pairs.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_keys.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_index.ensure(dev_cap));
-  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
-  KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+  uint64_t dev_cap = 0;
+  rc = pairs_begin(c, c->d_ld_pairs, capacity, (uint64_t)P.band.tiles.size() * kGramM * kGramN, dev_cap); if (rc) return rc;
   for (size_t s = 0; s + 1 < P.band.slab_begin.size(); ++s) {
     rc = ld_slab_grams(c, P, s, T); if (rc) return rc;
     rc = ld_slab_pairs(c, T, min_r2, 0, dev_cap, c->d_ld_pairs.p); if (rc) return rc;
   }
-  unsigned long long total = 0;
-  KGL_CUDA(c, cudaMemcpyAsync(&total, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
-  KGL_CUDA(c, cudaStreamSynchronize(c->stream));
-  *n_pairs = total;
-  if (total > capacity || total > dev_cap) return fail(c, KGL_B200_ERR_NOMEM, "more LD pairs than capacity (*n_pairs holds the total)");
-  if (total == 0) return KGL_B200_OK;
-  rc = sort_pair_keys(c, total, pair_key_bits(c->L)); if (rc) return rc;
-  return fetch_sorted_pairs(c, c->d_ld_pairs, c->d_ld_sorted, total, pairs);
+  return pairs_end(c, c->d_ld_pairs, c->d_ld_sorted, dev_cap, c->L, "LD pairs", pairs, n_pairs);
 }
 
 int kgl_b200_run_ld_prune(kgl_b200_ctx* c, const kgl_b200_ld_options* options, double max_r2, uint8_t* keep_out, uint64_t* n_kept) {
@@ -3147,9 +3154,6 @@ int kgl_b200_run_ld_prune(kgl_b200_ctx* c, const kgl_b200_ld_options* options, d
   int rc = ld_prepare(c, options, max_r2, P, T); if (rc) return rc;
   const uint64_t L = c->L;
   const int end_bit = pair_key_bits(L);
-  KGL_CUDA(c, c->d_pair_cursor.ensure(1));
-  KGL_CUDA(c, c->d_pair_keys.ensure(1u << 20));
-  KGL_CUDA(c, c->d_pair_index.ensure(1u << 20));
   // The greedy scan, slab by slab: pairs (i, l) with r^2 > max_r2 as keys (l << 32) | i, ascending. After slab s every pair whose
   // l lies before the next slab's first block row is known (i <= l, and the tiles ascend), so those loci are final: walk them in
   // order against the pending pairs. Loci [0, done) are final.
@@ -3169,15 +3173,12 @@ int kgl_b200_run_ld_prune(kgl_b200_ctx* c, const kgl_b200_ld_options* options, d
   const size_t n_slabs = P.band.slab_begin.size() - 1;
   for (size_t s = 0; s < n_slabs; ++s) {
     rc = ld_slab_grams(c, P, s, T); if (rc) return rc;
-    unsigned long long n = 0;
+    uint64_t n = 0;
     for (int attempt = 0; attempt < 2; ++attempt) {      // a slab with more pairs than the key buffer runs again into a larger one
-      KGL_CUDA(c, cudaMemsetAsync(c->d_pair_cursor.p, 0, 8, c->stream));
+      rc = pair_keys_reset(c, std::max<uint64_t>(n, 1u << 20)); if (rc) return rc;
       rc = ld_slab_pairs(c, T, max_r2, 1, c->d_pair_keys.cap, nullptr); if (rc) return rc;
-      KGL_CUDA(c, cudaMemcpyAsync(&n, c->d_pair_cursor.p, 8, cudaMemcpyDeviceToHost, c->stream));
-      KGL_CUDA(c, cudaStreamSynchronize(c->stream));
+      rc = read_counter(c, c->d_pair_cursor.p, n); if (rc) return rc;
       if (n <= c->d_pair_keys.cap) break;
-      KGL_CUDA(c, c->d_pair_keys.ensure(n));
-      KGL_CUDA(c, c->d_pair_index.ensure(n));
     }
     slab.resize(n);
     if (n > 0) {
@@ -3211,10 +3212,9 @@ int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, doubl
   if (!c || !options || !fst) return fail(c, KGL_B200_ERR_INVALID, "null argument");
   const kgl_b200_fst_options& o = *options;
   if (o.method > 1) return fail(c, KGL_B200_ERR_INVALID, "method must be 0 (Hudson) or 1 (Weir & Cockerham)");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
-  const uint32_t G = o.group ? o.n_groups : KGL_B200_MAX_POP;
-  if (G == 0 || G > kGcMaxGroups) return fail(c, KGL_B200_ERR_INVALID, "n_groups must be 1..64");
+  int rc = use_population(c, false); if (rc) return rc;
+  uint32_t G = 0;
+  rc = check_groups(c, o.group, o.n_groups, G, false); if (rc) return rc;
   std::vector<uint2> pairs;
   if (o.n_pairs == 0 || !o.pairs) {
     for (uint32_t a = 0; a < G; ++a)
@@ -3231,8 +3231,8 @@ int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, doubl
   // windows w = 0 .. max offset / step over offsets [w step, w step + window): rows [lower_bound(w step), lower_bound(w step + window))
   std::vector<uint2> range;
   if (o.window_bp) {
-    if (!c->have_offsets || c->h_offsets.size() != L) return fail(c, KGL_B200_ERR_STATE, "F_ST windows need the locus offsets (kgl_b200_upload_loci)");
-    if (!std::is_sorted(c->h_offsets.begin(), c->h_offsets.end())) return fail(c, KGL_B200_ERR_INVALID, "F_ST windows: the locus offsets are not sorted");
+    rc = require_sorted_offsets(c, "F_ST windows need the locus offsets (kgl_b200_upload_loci)", "F_ST windows: the locus offsets are not sorted");
+    if (rc) return rc;
     const uint64_t step = o.step_bp ? o.step_bp : o.window_bp;
     const uint64_t nw = (uint64_t)c->h_offsets.back() / step + 1;
     for (uint64_t w = 0; w < nw; ++w) range.push_back(make_uint2((uint32_t)first_row_at(c, w * step), (uint32_t)first_row_at(c, w * step + o.window_bp)));
@@ -3241,15 +3241,11 @@ int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, doubl
   rc = group_counts_device(c, G, o.group, G2); if (rc) return rc;
   if (n_windows) *n_windows = range.size();            // only once the labels and the state have been accepted
   const uint64_t n_blocks = (L + kFstBlock - 1) / kFstBlock;
-  KGL_CUDA(c, c->d_fst_pairs.ensure(np));
   KGL_CUDA(c, c->d_fst_blocks.ensure(np * n_blocks));
   KGL_CUDA(c, c->d_fst_used.ensure(np * n_blocks));
   KGL_CUDA(c, c->d_fst_out.ensure(np));
-  KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_pairs.p, pairs.data(), np * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
-  if (o.keep) {
-    KGL_CUDA(c, c->d_fst_keep.ensure(L));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_keep.p, o.keep, L, cudaMemcpyHostToDevice, c->stream));
-  }
+  rc = upload(c, c->d_fst_pairs, pairs.data(), np); if (rc) return rc;
+  if (o.keep) { rc = upload(c, c->d_fst_keep, o.keep, L); if (rc) return rc; }
   if (per_locus) KGL_CUDA(c, c->d_fst_terms.ensure(np * L));
   FstParams P{};
   P.counts = c->d_group_counts.p; P.n_loci = L; P.n_blocks = n_blocks; P.n_groups = G; P.method = o.method; P.n_pairs = (uint32_t)np;
@@ -3263,9 +3259,8 @@ int kgl_b200_run_fst(kgl_b200_ctx* c, const kgl_b200_fst_options* options, doubl
   if (per_locus) KGL_CUDA(c, cudaMemcpyAsync(per_locus, c->d_fst_terms.p, np * L * 16, cudaMemcpyDeviceToHost, c->stream));
   if (!range.empty() && windows) {
     const uint64_t nw = range.size();
-    KGL_CUDA(c, c->d_fst_range.ensure(nw));
     KGL_CUDA(c, c->d_fst_windows.ensure(np * nw * 3));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_fst_range.p, range.data(), nw * sizeof(uint2), cudaMemcpyHostToDevice, c->stream));
+    rc = upload(c, c->d_fst_range, range.data(), nw); if (rc) return rc;
     k_fst_windows<<<blocks_for(np * nw, 128), 128, 0, c->stream>>>(P, c->d_fst_range.p, nw, c->d_fst_windows.p);
     KGL_LAUNCH_CHECK(c);
     KGL_CUDA(c, cudaMemcpyAsync(windows, c->d_fst_windows.p, np * nw * 24, cudaMemcpyDeviceToHost, c->stream));
@@ -3294,20 +3289,15 @@ int kgl_b200_run_variant_qc(kgl_b200_ctx* c, const kgl_b200_qc_options* options,
   if (!(o.min_maf >= 0.0 && o.min_maf <= 0.5)) return fail(c, KGL_B200_ERR_INVALID, "min_maf must be in [0, 0.5]");
   if (!(o.min_hwe_p >= 0.0 && o.min_hwe_p <= 1.0)) return fail(c, KGL_B200_ERR_INVALID, "min_hwe_p must be in [0, 1]");
   if (o.midp > 1) return fail(c, KGL_B200_ERR_INVALID, "midp must be 0 or 1");
-  int rc = use_device(c); if (rc) return rc;
-  rc = require_population(c, false); if (rc) return rc;
+  int rc = use_population(c, false); if (rc) return rc;
   uint32_t G = 0;
   if (o.min_hwe_p != 0.0) { rc = hardy_device(c, o.group, o.n_groups, o.midp, false, G); if (rc) return rc; }
   // The pooled counts come from the raw streaming pass PCA and LD run (pca_prepare): it reads the matrix at the streaming rate, needs
   // no label table, and leaves d_group_counts holding the groups of the test.
-  rc = default_superpop(c); if (rc) return rc;
-  rc = launch_count(c, true, true, false, false, false, nullptr, false, &c->d_pca_counts); if (rc) return rc;
+  rc = raw_locus_counts(c); if (rc) return rc;
   const uint8_t* multi = nullptr;
   rc = hwe_multi_flags(c, multi); if (rc) return rc;
-  if (o.keep) {
-    KGL_CUDA(c, c->d_qc_keep.ensure(c->L));
-    KGL_CUDA(c, cudaMemcpyAsync(c->d_qc_keep.p, o.keep, c->L, cudaMemcpyHostToDevice, c->stream));
-  }
+  if (o.keep) { rc = upload(c, c->d_qc_keep, o.keep, c->L); if (rc) return rc; }
   KGL_CUDA(c, c->d_qc_out.ensure(c->L));
   KGL_CUDA(c, c->d_hwe_stats.ensure(2));
   if (o.min_hwe_p == 0.0) KGL_CUDA(c, cudaMemsetAsync(c->d_hwe_stats.p, 0, 8, c->stream));
